@@ -3,6 +3,12 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port on host cores
+    python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed
+
+--dump-outputs writes the arrays the timed step hands its caller, for the whole job's batch in env order:
+DIR/contact_forces.npy (float32 [envs, 12]) and DIR/solve_info.npy (the int32 [envs, 4] solve_info as
+float64), 80 bytes per env (2.6 MB at 8 GPUs); the CPU arm writes its contact_forces.npy alone.  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 
 A "step" is one pass of rg_mpc_build_solve over one batch of synthetic robot states: BASELINE
 config[1] -- 4096 envs per GPU, horizon 10, 4 legs, friction pyramid (weak scaling: every rank
@@ -148,8 +154,10 @@ def run_reference(args):
         c_oracle.solve_batch(mp, states.slice(0, 512), ctrl.MPC_BODY_HEIGHT, n_threads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        c_oracle.solve_batch(mp, states, ctrl.MPC_BODY_HEIGHT, n_threads=cores)
+        forces, _, _ = c_oracle.solve_batch(mp, states, ctrl.MPC_BODY_HEIGHT, n_threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        _write_outputs(args.dump_outputs, {"contact_forces": forces})
     value = n * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -264,6 +272,11 @@ def run_gpu(args):
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = rg.launch_count() - launches0
+    # the last timed step's outputs, copied now: the e2e arm below writes into the same buffers
+    dump = None
+    if args.dump_outputs:
+        dump = {"contact_forces": _gather_rows(torch, dist, forces.clone(), world),
+                "solve_info": _gather_rows(torch, dist, info.to(torch.float64), world)}
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     rank_ms = [torch.zeros(1, dtype=torch.float64, device=dev) for _ in range(world)]
@@ -398,9 +411,27 @@ def run_gpu(args):
             "solve_latency": {"solve_p50_ms": statistics.median(step_ms), "solve_max_ms": max(step_ms), "envs": n},
             "latency": latency, "control_step": control, "config4": config4, "config5": config5,
             "wall_s_timed_region": t_wall}
+    if dump is not None:
+        _write_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in dump.items()})
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def _gather_rows(torch, dist, t, world):
+    """Rank shards (equal row counts) concatenated in rank order, i.e. in global env order."""
+    if world == 1:
+        return t
+    parts = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(parts, t)
+    return torch.cat(parts)
+
+
+def _write_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def _stats_vector(torch, rg, info, forces, n):
@@ -571,7 +602,11 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
