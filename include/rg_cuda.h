@@ -61,8 +61,11 @@ enum {
   RG_STATUS_NO_STANCE = 4,       /* no foot in contact: all forces are zero by the bounds */
   RG_STATUS_NUMERIC = 8,         /* non-positive pivot met (result is the last good iterate) */
   RG_STATUS_ACTIVE_SET_ONLY = 16,/* the cold-start active-set iteration verified; no interior point ran */
-  RG_STATUS_BAD_WORKSPACE = 32   /* the workspace on the device is not the one rg_mpc_setup prepared for this horizon
+  RG_STATUS_BAD_WORKSPACE = 32,  /* the workspace on the device is not the one rg_mpc_setup prepared for this horizon
                                     (freed / overwritten without rg_mpc_release): forces are zero, nothing was solved */
+  RG_STATUS_BAD_MODEL = 64       /* this env's row of the rg_mpc_env_model fails the checks rg_mpc_setup makes (mass > 0
+                                    and finite, inertia finite and invertible, friction coefficients > 0): forces and
+                                    horizon outputs are zero, the warm-start set is reset, nothing was solved */
 };
 
 /* ---- ConvexMpc constructor arguments + the constants compiled into mpc_osqp ------------
@@ -180,6 +183,29 @@ typedef struct rg_mpc_io {
   int32_t reserved_;
 } rg_mpc_io;
 int rg_mpc_build_solve_io(const void* workspace, int n_env, const rg_mpc_io* io_host, void* stream);
+
+/* Per-env body and ground: the values each reference process passes to its own ConvexMpc(mass, inertia, ...)
+ * (mpc_controller.py:47-56) and as the `friction` argument of every compute_contact_forces call.  Float64 DEVICE
+ * arrays, env-major, 8-byte aligned; each may be NULL (= the workspace's value for every env).  They are parameters,
+ * not sensor inputs: float64 so that a model filled with the workspace's own values solves what the workspace does.
+ *   mass             [N]    kg.  The force bounds follow it with the workspace's ratios:
+ *                           fz_max_e = fz_max * (mass_e / mass), fz_min_e = fz_min * (mass_e / mass)
+ *                           (mpc_osqp's kMaxScale m g / kMinScale m g)
+ *   inertia          [N,9]  body-frame inertia, row major; inverted on the device per solve
+ *   friction_coeffs  [N,4]  one per pyramid ROW, as rg_mpc_params.friction_coeffs
+ * Weights, alpha, dt, horizon, gravity and the desired body height stay per workspace.  The kernels read the arrays
+ * on every launch (a captured control-step graph included), so new values written in place take effect at the next
+ * solve.  A row that fails the checks rg_mpc_setup makes gets RG_STATUS_BAD_MODEL; the other envs are unaffected. */
+typedef struct rg_mpc_env_model {
+  const double* mass;             /* [N]    or NULL */
+  const double* inertia;          /* [N,9]  or NULL */
+  const double* friction_coeffs;  /* [N,4]  or NULL */
+} rg_mpc_env_model;
+
+/* rg_mpc_build_solve_io with a per-env model.  model == NULL, or all three pointers NULL, is exactly
+ * rg_mpc_build_solve_io (which forwards here with NULL). */
+int rg_mpc_build_solve_model(const void* workspace, int n_env, const rg_mpc_io* io_host,
+                             const rg_mpc_env_model* model_host, void* stream);
 
 /* ---- robot model: leg chains + gait + gains ------------------------------------------------
  * Replaces the per-robot python constants the third-party stack reads through the robot
@@ -346,6 +372,15 @@ int rg_control_step_graph_create(const void* mpc_workspace, const void* robot_wo
                                  const rg_controller_state* s_host, void* stream, void** graph_out);
 int rg_control_step_graph_launch(void* graph, void* stream);
 int rg_control_step_graph_destroy(void* graph);
+
+/* The control step and its graph with a per-env model in the stance solve (rg_mpc_env_model above; NULL = the two
+ * calls before it, which forward here).  The graph bakes in the model POINTERS, not the values: writing new masses,
+ * inertias or friction coefficients into the same arrays between replays needs no re-capture. */
+int rg_control_step_model(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                          const rg_controller_state* s_host, const rg_mpc_env_model* model_host, void* stream);
+int rg_control_step_graph_create_model(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                                       const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                                       void* stream, void** graph_out);
 
 /* ---- "next" row (SURVEY.md 8f rank 1): batched HYBRID motor model ----------------------------
  * Replaces RobotMotorModel.convert_to_torque HYBRID branch (simple_motor.py:128-139):

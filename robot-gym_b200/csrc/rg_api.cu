@@ -233,6 +233,7 @@ extern "C" int rg_mpc_setup(const rg_mpc_params* p, void* workspace, size_t work
   h.cold_start_rounds = (p->max_polish_rounds > 0 && p->cold_start_rounds > 0) ? p->cold_start_rounds : 0;
   h.cold_start_max_violations = p->cold_start_max_violations > 0 ? p->cold_start_max_violations : (1 << 30);
   h.inv_mass = 1.0 / p->mass;
+  h.mass = p->mass;
   if (!inv3(p->inertia, h.inv_inertia)) { rg_set_error("inertia matrix is singular"); return RG_ERR_SINGULAR; }
   h.dt = p->dt;
   for (int i = 0; i < 6; ++i) { h.w_rho[i] = p->weights[i]; h.w_nu[i] = p->weights[6 + i]; }
@@ -300,7 +301,23 @@ extern "C" int rg_mpc_release(const void* workspace) {
   return RG_OK;
 }
 
+int rg_check_env_model(const rg_mpc_env_model* model, const char* what, const rg_mpc_env_model** out) {
+  *out = nullptr;
+  if (!model || (!model->mass && !model->inertia && !model->friction_coeffs)) return RG_OK;
+  if (((uintptr_t)model->mass | (uintptr_t)model->inertia | (uintptr_t)model->friction_coeffs) & 7u) {
+    rg_set_error("%s: env model arrays must be 8-byte aligned float64", what);
+    return RG_ERR_BAD_ARG;
+  }
+  *out = model;
+  return RG_OK;
+}
+
 extern "C" int rg_mpc_build_solve_io(const void* workspace, int n_env, const rg_mpc_io* io, void* stream) {
+  return rg_mpc_build_solve_model(workspace, n_env, io, nullptr, stream);
+}
+
+extern "C" int rg_mpc_build_solve_model(const void* workspace, int n_env, const rg_mpc_io* io,
+                                        const rg_mpc_env_model* model, void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
   if (!workspace || !io || !io->com_velocity_body || !io->base_rpy || !io->base_rpy_rate || !io->foot_contact_state ||
       !io->foot_positions_base || !io->command || !io->contact_forces) {
@@ -316,11 +333,14 @@ extern "C" int rg_mpc_build_solve_io(const void* workspace, int n_env, const rg_
     rg_set_error("rg_mpc_build_solve: foot_positions_base must be 16-byte aligned");
     return RG_ERR_BAD_ARG;
   }
+  const rg_mpc_env_model* m = nullptr;
+  int rc = rg_check_env_model(model, "rg_mpc_build_solve_model", &m);
+  if (rc != RG_OK) return rc;
   RgMpcHostInfo info;
-  int rc = rg_mpc_workspace_info(workspace, &info);
+  rc = rg_mpc_workspace_info(workspace, &info);
   if (rc != RG_OK) return rc;
   return rg_launch_mpc((const RgMpcDev*)workspace, info.horizon, n_env, *io, info.two_kernel && info.queue_capacity >= n_env,
-                       (cudaStream_t)stream);
+                       (cudaStream_t)stream, 0, m);
 }
 
 extern "C" int rg_mpc_build_solve(const void* workspace, int n_env, const float* com_velocity_body,

@@ -36,6 +36,9 @@ struct RgMpcDev {
   // env-independent tables (host-computed, read through the L1/L2-cached uniform path):
   double c2tab[RG_MAX_HORIZON * RG_MAX_HORIZON];                        // c2(j,k), row-major h x h
   double kinv_lin[3][RG_MAX_HORIZON * (RG_MAX_HORIZON + 1) / 2];        // K^-1 of the x/y/z channels, packed
+  // mass of the parameter set: a per-env model (rg_mpc_env_model) scales fz_max / fz_min by mass_e / mass.  Last, so
+  // that the offsets the model-free kernels read are the ones they were tuned with.
+  double mass;
 };
 
 // Per-workspace scratch behind the parameter block (rg_workspace_bytes(n_env, ...) sizes it for n_env envs):
@@ -98,7 +101,11 @@ struct rg_controller_state;
 // chained = 1: the caller launched a kernel that signals griddepcontrol.launch_dependents right before (the step
 // prologue) and launches one with the programmatic attribute right after (the epilogue): the first MPC kernel is then
 // launched programmatically too.  Every MPC kernel starts with griddepcontrol.wait (a no-op after a plain launch).
-int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained = 0);
+// model: a per-env model with at least one non-NULL array, or NULL (the model-free kernels).
+int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained = 0,
+                  const rg_mpc_env_model* model = nullptr);
+// NULL, or a model whose three pointers are all NULL -> NULL; RG_ERR_BAD_ARG for an array that is not 8-byte aligned
+int rg_check_env_model(const rg_mpc_env_model* model, const char* what, const rg_mpc_env_model** out);
 
 // Kernel launch with or without the programmatic-stream-serialization attribute (programmatic dependent launch: the
 // grid may become resident while its predecessor drains; it must execute griddepcontrol.wait before touching the

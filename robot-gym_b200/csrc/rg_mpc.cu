@@ -1340,15 +1340,38 @@ __device__ __forceinline__ void build_basis(unsigned& act, bool active_blk, cons
   act &= keep;
 }
 
+// Inverse of an env's 3x3 body inertia (row major) by cofactors, the formula and the rounding of the host's inv3
+// (rg_api.cu): no contracted multiply-adds, one IEEE division -- a row equal to the workspace's inertia gives the
+// workspace's inverse bit for bit.  The caller has checked |det| >= 1e-300.
+__device__ __forceinline__ void env_inv3(const double* __restrict__ m, double* o) {
+  const double c00 = __dsub_rn(__dmul_rn(m[4], m[8]), __dmul_rn(m[5], m[7]));
+  const double c01 = __dsub_rn(__dmul_rn(m[5], m[6]), __dmul_rn(m[3], m[8]));
+  const double c02 = __dsub_rn(__dmul_rn(m[3], m[7]), __dmul_rn(m[4], m[6]));
+  const double det = __dadd_rn(__dadd_rn(__dmul_rn(m[0], c00), __dmul_rn(m[1], c01)), __dmul_rn(m[2], c02));
+  const double id = 1.0 / det;
+  o[0] = __dmul_rn(c00, id);
+  o[1] = __dmul_rn(__dsub_rn(__dmul_rn(m[2], m[7]), __dmul_rn(m[1], m[8])), id);
+  o[2] = __dmul_rn(__dsub_rn(__dmul_rn(m[1], m[5]), __dmul_rn(m[2], m[4])), id);
+  o[3] = __dmul_rn(c01, id);
+  o[4] = __dmul_rn(__dsub_rn(__dmul_rn(m[0], m[8]), __dmul_rn(m[2], m[6])), id);
+  o[5] = __dmul_rn(__dsub_rn(__dmul_rn(m[2], m[3]), __dmul_rn(m[0], m[5])), id);
+  o[6] = __dmul_rn(c02, id);
+  o[7] = __dmul_rn(__dsub_rn(__dmul_rn(m[1], m[6]), __dmul_rn(m[0], m[7])), id);
+  o[8] = __dmul_rn(__dsub_rn(__dmul_rn(m[0], m[4]), __dmul_rn(m[1], m[3])), id);
+}
+
 // One env's stance QP, executed by the whole CTA.
 // LEAN = true : the verified active-set rounds only -- no interior-point state or code (the registers that frees
 //               are most of the kernel's local-memory frame).  An env whose rounds do not verify within the
 //               cold-start budget is appended to the fallback queue and gets no output from this call.
 // LEAN = false: the complete solver (cold start unless skip_cold, interior point, escalation ladder).
-template <int H, bool LEAN>
+// ENV_MODEL = true: mass, inertia and friction coefficients come from the env's row of `model` where its array is not
+//               NULL (rg_mpc_env_model).  A compile-time flag, so that the model-free instantiations -- whose schedule
+//               was tuned instruction by instruction (DESIGN.md 3.10-3.11) -- carry none of its code (DESIGN.md 3.12).
+template <int H, bool LEAN, bool ENV_MODEL>
 __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch,
                                           const int env, const bool skip_cold,
-                                          const rg_mpc_io& io) {
+                                          const rg_mpc_io& io, const rg_mpc_env_model& model) {
   using C = Cfg<H>;
   const float* __restrict__ g_com_vel = io.com_velocity_body;
   const float* __restrict__ g_rpy = io.base_rpy;
@@ -1390,11 +1413,42 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 
   // ---------------------------------------------------------------- parameters (uniform loads)
   const double dt = ws->dt, two_alpha = 2.0 * ws->alpha;
-  const double inv_mass = ws->inv_mass;
-  const double fzmax = ws->fz_max, fzmin = ws->fz_min;
+  double inv_mass = ws->inv_mass;
+  double fzmax = ws->fz_max, fzmin = ws->fz_min;
   double mu[4];
 #pragma unroll
   for (int r = 0; r < 4; ++r) mu[r] = ws->mu[r];
+  // per-env model: every thread loads the env's mass and friction row (one address across the CTA: a broadcast) --
+  // all of them use 1/m, the bounds and mu; the inertia is read by the lever-arm threads (tid < 4) only, except for
+  // the determinant every thread takes here so that the validity test is uniform over the CTA without a barrier.
+  // The bounds scale by mass_e / mass: exactly the workspace's bounds when the env's mass is the workspace's.
+  bool model_ok = true;
+  if constexpr (ENV_MODEL) {
+    if (model.mass) {
+      const double m = model.mass[env];
+      model_ok = m > 0.0 && m <= 1.79769313486231570e308;   // > 0 and finite (NaN fails both)
+      inv_mass = 1.0 / m;
+      const double scale = m / ws->mass;
+      fzmax *= scale;
+      fzmin *= scale;
+    }
+    if (model.friction_coeffs) {
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        mu[r] = model.friction_coeffs[4 * (size_t)env + r];
+        model_ok = model_ok && mu[r] > 0.0;
+      }
+    }
+    if (model.inertia) {
+      const double* __restrict__ in = model.inertia + 9 * (size_t)env;
+      double fin = 0.0;
+#pragma unroll
+      for (int i = 0; i < 9; ++i) fin += in[i] * 0.0;      // NaN unless all nine are finite
+      const double det = in[0] * (in[4] * in[8] - in[5] * in[7]) + in[1] * (in[5] * in[6] - in[3] * in[8]) +
+                         in[2] * (in[3] * in[7] - in[4] * in[6]);
+      model_ok = model_ok && fin == 0.0 && fabs(det) >= 1e-300;
+    }
+  }
   const double big_u = (mu[0] + 1.0) * fzmax;
 
   // ---------------------------------------------------------------- per-env inputs
@@ -1431,6 +1485,16 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
   const int n_stance = (int)stance_leg[0] + stance_leg[1] + stance_leg[2] + stance_leg[3];
   const bool active_blk = is_blk && ((contact_word >> (8 * leg)) & 0xffu) != 0;
 
+  if constexpr (ENV_MODEL) {
+    if (!model_ok) {     // this env's model row fails the rg_mpc_setup checks: nothing is solved
+      for (int i = tid; i < 12; i += blockDim.x) g_forces[12 * (size_t)env + i] = 0.f;
+      if (g_hforces) for (int i = tid; i < 12 * H; i += blockDim.x) g_hforces[12 * H * (size_t)env + i] = 0.f;
+      if (g_hforces64) for (int i = tid; i < 12 * H; i += blockDim.x) g_hforces64[12 * H * (size_t)env + i] = 0.0;
+      if (g_info && tid < 4) g_info[4 * (size_t)env + tid] = tid == RG_INFO_STATUS ? RG_STATUS_BAD_MODEL : 0;
+      if (g_active && is_blk) g_active[(size_t)env * C::NB + tid] = RG_ACTIVE_SET_UNKNOWN;
+      return;
+    }
+  }
   if (n_stance == 0) {   // every force pinned to zero by the bounds
     for (int i = tid; i < 12; i += blockDim.x) g_forces[12 * (size_t)env + i] = 0.f;
     if (g_hforces) for (int i = tid; i < 12 * H; i += blockDim.x) g_hforces[12 * H * (size_t)env + i] = 0.f;
@@ -1517,6 +1581,15 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
                             sy * cp, sy * sp * sr + cy * cr, sy * sp * cr - cy * sr,
                             -sp, cp * sr, cp * cr};
       // I_w^-1 = R I_b^-1 R^T
+      double ib[9];
+      if constexpr (ENV_MODEL) {
+        if (model.inertia) {
+          env_inv3(model.inertia + 9 * (size_t)env, ib);
+        } else {
+#pragma unroll
+          for (int i = 0; i < 9; ++i) ib[i] = ws->inv_inertia[i];
+        }
+      }
       double tmp[9], iw[9];
 #pragma unroll
       for (int a = 0; a < 3; ++a)
@@ -1524,7 +1597,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
         for (int b = 0; b < 3; ++b) {
           double v = 0.0;
 #pragma unroll
-          for (int c = 0; c < 3; ++c) v += rb[3 * a + c] * ws->inv_inertia[3 * c + b];
+          for (int c = 0; c < 3; ++c) v += rb[3 * a + c] * (ENV_MODEL ? ib[3 * c + b] : ws->inv_inertia[3 * c + b]);
           tmp[3 * a + b] = v;
         }
 #pragma unroll
@@ -2274,27 +2347,27 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 }
 
 // Grid of the lean kernel and of the single-kernel path: one CTA per env (blockIdx.x = env).
-template <int H, bool LEAN>
-__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
-mpc_solve_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io) {
+template <int H, bool LEAN, bool ENV_MODEL>
+__device__ __forceinline__ void solve_grid(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env,
+                                           const rg_mpc_io& io, const rg_mpc_env_model& model) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
   const int env = blockIdx.x;
 #if RG_PDL
-  RG_GRID_LAUNCH_DEPENDENTS();   // see launch_h: the fallback grid (lean) or the step epilogue (complete kernel) may be scheduled behind us
+  RG_GRID_LAUNCH_DEPENDENTS();   // see launch_kernels: the fallback grid (lean) or the step epilogue (complete kernel) may be scheduled behind us
   RG_GRID_WAIT();                // launched programmatically behind the step prologue in rg_control_step; a no-op otherwise
 #endif
   if (env >= n_env) return;
-  solve_env<H, LEAN>(sm, ws, scratch, env, false, io);
+  solve_env<H, LEAN, ENV_MODEL>(sm, ws, scratch, env, false, io, model);
 }
 
 // Second kernel of the two-kernel solve: the complete solver on the envs the lean kernel queued.  Persistent CTAs
 // stride over the list (it is empty for trot / walk batches: the launch then costs a few microseconds); the cold
 // start is skipped -- the lean kernel has just spent its budget on exactly those rounds.  The last CTA to finish
 // re-arms the queue counters for the next solve.
-template <int H>
-__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
-mpc_fallback_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io) {
+template <int H, bool ENV_MODEL>
+__device__ __forceinline__ void fallback_grid(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env,
+                                              const rg_mpc_io& io, const rg_mpc_env_model& model) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
 #if RG_PDL
@@ -2305,7 +2378,7 @@ mpc_fallback_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ 
   for (int q = blockIdx.x; q < count; q += gridDim.x) {
     const int env = scratch->queue[q];
     if (env >= 0 && env < n_env)
-      solve_env<H, false>(sm, ws, scratch, env, true, io);
+      solve_env<H, false, ENV_MODEL>(sm, ws, scratch, env, true, io, model);
     __syncthreads();   // shared memory is reused by the next env of this CTA
   }
   if (threadIdx.x == 0) {
@@ -2315,6 +2388,36 @@ mpc_fallback_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ 
       scratch->done_ctas = 0;
     }
   }
+}
+
+// The model-free kernels keep the parameter list they were tuned with (an extra kernel parameter renumbers the PTX
+// virtual registers, and ptxas then schedules the h = 10 lean kernel differently); the *_model_kernel twins take the
+// per-env model (rg_mpc_env_model, at least one array non-NULL).
+
+template <int H, bool LEAN>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_solve_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io) {
+  solve_grid<H, LEAN, false>(ws, scratch, n_env, io, rg_mpc_env_model{nullptr, nullptr, nullptr});
+}
+
+template <int H, bool LEAN>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_solve_model_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
+                       const rg_mpc_env_model model) {
+  solve_grid<H, LEAN, true>(ws, scratch, n_env, io, model);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_fallback_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io) {
+  fallback_grid<H, false>(ws, scratch, n_env, io, rg_mpc_env_model{nullptr, nullptr, nullptr});
+}
+
+template <int H>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_fallback_model_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
+                          const rg_mpc_env_model model) {
+  fallback_grid<H, true>(ws, scratch, n_env, io, model);
 }
 
 // Dynamic shared memory above 48 KB (h = 20) and the carveout are per-device function attributes: set them once
@@ -2360,40 +2463,59 @@ int sm_count() {
   return cached[dev];
 }
 
-template <int H>
-int launch_h(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained) {
+template <bool B, class A, class C>
+constexpr auto pick(A a, C c) { if constexpr (B) return c; else return a; }
+
+template <int H, bool ENV_MODEL>
+int launch_kernels(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
+                   const rg_mpc_env_model& model) {
+  const auto lean_kernel = pick<ENV_MODEL>(mpc_solve_kernel<H, true>, mpc_solve_model_kernel<H, true>);
+  const auto full_kernel = pick<ENV_MODEL>(mpc_solve_kernel<H, false>, mpc_solve_model_kernel<H, false>);
+  const auto fallback_kernel = pick<ENV_MODEL>(mpc_fallback_kernel<H>, mpc_fallback_model_kernel<H>);
   const size_t smem = sizeof(Smem<H>);
   RgMpcScratch* scratch = (RgMpcScratch*)((char*)ws + RG_MPC_SCRATCH_OFFSET);
+  auto launch = [&](auto kernel, int grid, bool programmatic) {
+    if constexpr (ENV_MODEL)
+      return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io, model);
+    else
+      return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io);
+  };
   int rc;
   const int slots = sm_count() * Cfg<H>::MIN_BLOCKS;     // CTAs resident at once
   // A batch that fits one wave gains nothing from the split (every env has an SM slot of its own from the start):
   // one launch of the complete kernel instead of two -- this is the small-N latency path.
   if (two_kernel && n_env > slots) {
     // lean active-set kernel on every env, then the complete solver on whatever it queued
-    rc = configure_kernel((const void*)mpc_solve_kernel<H, true>, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_solve_kernel lean)");
+    rc = configure_kernel((const void*)lean_kernel, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_solve_kernel lean)");
     if (rc != RG_OK) return rc;
-    rc = configure_kernel((const void*)mpc_fallback_kernel<H>, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_fallback_kernel)");
+    rc = configure_kernel((const void*)fallback_kernel, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_fallback_kernel)");
     if (rc != RG_OK) return rc;
-    rc = rg_check_cuda(rg_launch(mpc_solve_kernel<H, true>, dim3((unsigned)n_env), dim3((unsigned)Cfg<H>::NT), smem, stream,
-                                 RG_PDL && chained, ws, scratch, n_env, io), "mpc_solve_kernel (lean) launch");
+    rc = rg_check_cuda(launch(lean_kernel, n_env, RG_PDL && chained), "mpc_solve_kernel (lean) launch");
     rg_count_launch();
     if (rc != RG_OK) return rc;
     const int grid = n_env < slots ? n_env : slots;       // as many CTAs as fit at once: an empty queue costs one wave of exits
     // Programmatic dependent launch: every lean CTA signals at its start, so once the last one HAS STARTED the fallback
     // grid may take the slots the draining lean grid leaves free; its CTAs block in griddepcontrol.wait until the lean
     // grid has completed (queue visible).  The launch latency of the second kernel hides behind the first one's tail.
-    rc = rg_check_cuda(rg_launch(mpc_fallback_kernel<H>, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, RG_PDL != 0,
-                                 ws, scratch, n_env, io), "mpc_fallback_kernel launch");
+    rc = rg_check_cuda(launch(fallback_kernel, grid, RG_PDL != 0), "mpc_fallback_kernel launch");
     rg_count_launch();
     return rc;
   }
-  rc = configure_kernel((const void*)mpc_solve_kernel<H, false>, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_solve_kernel)");
+  rc = configure_kernel((const void*)full_kernel, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_solve_kernel)");
   if (rc != RG_OK) return rc;
-  rc = rg_check_cuda(rg_launch(mpc_solve_kernel<H, false>, dim3((unsigned)n_env), dim3((unsigned)Cfg<H>::NT), smem, stream,
-                               RG_PDL && chained, ws, scratch, n_env, io), "mpc_solve_kernel launch");
+  rc = rg_check_cuda(launch(full_kernel, n_env, RG_PDL && chained), "mpc_solve_kernel launch");
   rg_count_launch();
   return rc;
 }
+
+// model: NULL selects the model-free kernels
+template <int H>
+int launch_h(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
+             const rg_mpc_env_model* model) {
+  if (model) return launch_kernels<H, true>(ws, n_env, io, two_kernel, stream, chained, *model);
+  return launch_kernels<H, false>(ws, n_env, io, two_kernel, stream, chained, rg_mpc_env_model{nullptr, nullptr, nullptr});
+}
+
 
 
 // ---- debug / self-test hook (not part of the public header): factor a dense SPD matrix given in
@@ -2490,11 +2612,12 @@ extern "C" int rg_debug_riccati_solve(int horizon, const double* k1, const doubl
   }
 }
 
-int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained) {
+int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
+                  const rg_mpc_env_model* model) {
   switch (horizon) {
-    case 5: return launch_h<5>(ws, n_env, io, two_kernel, stream, chained);
-    case 10: return launch_h<10>(ws, n_env, io, two_kernel, stream, chained);
-    case 20: return launch_h<20>(ws, n_env, io, two_kernel, stream, chained);
+    case 5: return launch_h<5>(ws, n_env, io, two_kernel, stream, chained, model);
+    case 10: return launch_h<10>(ws, n_env, io, two_kernel, stream, chained, model);
+    case 20: return launch_h<20>(ws, n_env, io, two_kernel, stream, chained, model);
     default:
       rg_set_error("unsupported horizon %d (kernels are built for 5, 10, 20)", horizon);
       return RG_ERR_UNSUPPORTED;

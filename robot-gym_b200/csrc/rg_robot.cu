@@ -799,6 +799,11 @@ extern "C" int rg_hybrid_motor_torque_ex(const void* ws, int n_env, const float*
 #endif
 
 extern "C" int rg_control_step(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s, void* stream) {
+  return rg_control_step_model(mpc_ws, robot_ws, n_env, s, nullptr, stream);
+}
+
+extern "C" int rg_control_step_model(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                     const rg_mpc_env_model* model, void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
   RG_REQUIRE(mpc_ws && robot_ws && s && n_env >= 0, "rg_control_step");
   RG_REQUIRE(s->time_since_reset && s->foot_contacts && s->base_velocity_world && s->base_orientation_xyzw && s->base_rpy &&
@@ -810,11 +815,14 @@ extern "C" int rg_control_step(const void* mpc_ws, const void* robot_ws, int n_e
              s->com_velocity_body && s->contact_forces && s->motor_torques && s->action, "rg_control_step outputs");
   RG_REQUIRE(!s->applied_motor_torques || s->motor_velocities, "rg_control_step torque consumer (motor_velocities)");
   RG_REQUIRE(((uintptr_t)s->foot_positions_base & 15u) == 0, "rg_control_step foot_positions_base (16-byte alignment)");
+  const rg_mpc_env_model* m = nullptr;
+  int rc = rg_check_env_model(model, "rg_control_step_model", &m);
+  if (rc != RG_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS) step_prologue_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>((const RgRobotDev*)robot_ws, n_env, *s);
   else step_prologue_env_kernel<<<grid_for(n_env, 128), 128, 0, st>>>((const RgRobotDev*)robot_ws, n_env, *s);
   rg_count_launch();
-  int rc = rg_check_cuda(cudaGetLastError(), "step_prologue_kernel launch");
+  rc = rg_check_cuda(cudaGetLastError(), "step_prologue_kernel launch");
   if (rc != RG_OK) return rc;
   RgMpcHostInfo info;
   rc = rg_mpc_workspace_info(mpc_ws, &info);
@@ -834,7 +842,7 @@ extern "C" int rg_control_step(const void* mpc_ws, const void* robot_ws, int n_e
   io.zero_yaw = 1;
   // prologue -> solve kernel(s) -> epilogue are chained by programmatic dependent launches: each grid becomes resident
   // while its predecessor drains and waits (griddepcontrol.wait) for it to complete, so the launch latencies overlap
-  rc = rg_launch_mpc((const RgMpcDev*)mpc_ws, info.horizon, n_env, io, info.two_kernel && info.queue_capacity >= n_env, st, 1);
+  rc = rg_launch_mpc((const RgMpcDev*)mpc_ws, info.horizon, n_env, io, info.two_kernel && info.queue_capacity >= n_env, st, 1, m);
   if (rc != RG_OK) return rc;
   rc = rg_check_cuda(rg_launch(step_epilogue_kernel, dim3((unsigned)grid_for(4 * n_env, 256)), dim3(256), 0, st, true,
                                (const RgRobotDev*)robot_ws, n_env, *s), "step_epilogue_kernel launch");
@@ -854,12 +862,17 @@ struct RgStepGraph {
 
 extern "C" int rg_control_step_graph_create(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                             void* stream, void** graph_out) {
+  return rg_control_step_graph_create_model(mpc_ws, robot_ws, n_env, s, nullptr, stream, graph_out);
+}
+
+extern "C" int rg_control_step_graph_create_model(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                                  const rg_mpc_env_model* model, void* stream, void** graph_out) {
   RG_REQUIRE(mpc_ws && robot_ws && s && graph_out && n_env > 0, "rg_control_step_graph_create");
   *graph_out = nullptr;
   // one eager step on the caller's stream first: kernel attributes get configured outside the capture, and argument
   // errors surface here with their own message.  The controller state advances by this step -- the caller accounts for it
   // by creating the graph INSTEAD of a step, not before one (see rg_cuda.h).
-  int rc = rg_control_step(mpc_ws, robot_ws, n_env, s, stream);
+  int rc = rg_control_step_model(mpc_ws, robot_ws, n_env, s, model, stream);
   if (rc == RG_OK) rc = rg_check_cuda(cudaStreamSynchronize((cudaStream_t)stream), "graph warm-up step");
   if (rc != RG_OK) return rc;
   cudaStream_t cap = nullptr;
@@ -869,7 +882,7 @@ extern "C" int rg_control_step_graph_create(const void* mpc_ws, const void* robo
   RgStepGraph* g = new RgStepGraph{nullptr, nullptr, 0};
   cudaError_t e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal);
   if (e == cudaSuccess) {
-    rc = rg_control_step(mpc_ws, robot_ws, n_env, s, cap);
+    rc = rg_control_step_model(mpc_ws, robot_ws, n_env, s, model, cap);
     e = cudaStreamEndCapture(cap, &g->graph);
     if (rc != RG_OK) e = cudaErrorUnknown;
   }

@@ -91,6 +91,8 @@ class BatchedMPCController(Controller):
         self._use_graph = (n <= self.GRAPH_MAX_ENVS) if use_graph is None else bool(use_graph)
         self._graph = None
         self._graph_invalidations = 0
+        self.env_mass = self.env_inertia = self.env_friction_coeffs = None   # per-env model (set_env_model)
+        self._env_model = None
 
         # --- C-ABI workspaces (the analogue of _setup_controller, mpc_controller.py:28-66)
         c = self._constants
@@ -313,27 +315,79 @@ class BatchedMPCController(Controller):
         lib = rg.load()
         with torch.cuda.device(self.device):
             if not self._use_graph:
-                rg.check(lib.rg_control_step(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
-                                             ctypes.byref(self._state), rg.current_stream_ptr()))
+                self._eager_step(lib)
             else:
                 if changed and self._graph is not None:          # a buffer moved: the captured pointers are stale
                     self._destroy_graph()
                     self._graph_invalidations += 1
                     if self._graph_invalidations >= 3:            # a provider that hands out fresh tensors every step
                         self._use_graph = False
-                        rg.check(lib.rg_control_step(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
-                                                     ctypes.byref(self._state), rg.current_stream_ptr()))
+                        self._eager_step(lib)
                         return self.action
                 if self._graph is None:
                     # creating the graph executes this step eagerly (and synchronises once)
                     handle = ctypes.c_void_p()
-                    rg.check(lib.rg_control_step_graph_create(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
-                                                              ctypes.byref(self._state), rg.current_stream_ptr(),
-                                                              ctypes.byref(handle)))
+                    if self._env_model is None:
+                        rg.check(lib.rg_control_step_graph_create(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
+                                                                  ctypes.byref(self._state), rg.current_stream_ptr(),
+                                                                  ctypes.byref(handle)))
+                    else:
+                        rg.check(lib.rg_control_step_graph_create_model(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
+                                                                        ctypes.byref(self._state), ctypes.byref(self._env_model),
+                                                                        rg.current_stream_ptr(), ctypes.byref(handle)))
                     self._graph = handle
                 else:
                     rg.check(lib.rg_control_step_graph_launch(self._graph, rg.current_stream_ptr()))
         return self.action
+
+    def _eager_step(self, lib):
+        if self._env_model is None:
+            rg.check(lib.rg_control_step(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
+                                         ctypes.byref(self._state), rg.current_stream_ptr()))
+        else:
+            rg.check(lib.rg_control_step_model(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
+                                               ctypes.byref(self._env_model), rg.current_stream_ptr()))
+
+    # ------------------------------------------------------------------ per-env body and ground
+    def set_env_model(self, mass=None, inertia=None, friction_coeffs=None, env_ids=None):
+        """Per-env mass [N] (kg), body-frame inertia [N,9] / [N,3,3] and friction coefficients [N,4] (one per
+        pyramid row) for the stance solve -- what each reference process passes to its own ``ConvexMpc(mass,
+        inertia, ...)`` and to ``compute_contact_forces(..., friction, ...)``.  The force bounds follow the mass with
+        the workspace's ratios (fz_max / mass, fz_min / mass).  Scalars and shorter leading shapes broadcast; with
+        ``env_ids`` only those rows are written.  The first call allocates controller-owned float64 tensors
+        (``env_mass``, ``env_inertia``, ``env_friction_coeffs``) filled with the robot's constants and drops the
+        captured step graph once; later calls write into them in place, so a captured graph stays valid.
+        Raises ``ValueError`` (before anything is written) for a mass that is not > 0 and finite, an inertia that is
+        not finite or not invertible, or a friction coefficient that is not > 0.  Synchronises once."""
+        n, dev, f64 = self.num_envs, self.device, torch.float64
+        if self._env_model is None:
+            p = self.mpc_params                       # the workspace's own values: robot constants + mpc_overrides
+            self.env_mass = torch.full((n,), float(p.mass), dtype=f64, device=dev)
+            self.env_inertia = torch.tensor([float(v) for v in p.inertia], dtype=f64, device=dev).repeat(n, 1)
+            self.env_friction_coeffs = torch.tensor([float(v) for v in p.friction_coeffs], dtype=f64, device=dev).repeat(n, 1)
+            model = rg.MpcEnvModel()
+            model.mass = rg._ptr(self.env_mass, f64, (), n=n, device=dev, align=8)
+            model.inertia = rg._ptr(self.env_inertia, f64, (9,), n=n, device=dev, align=8)
+            model.friction_coeffs = rg._ptr(self.env_friction_coeffs, f64, (4,), n=n, device=dev, align=8)
+            self._env_model = model
+            self._destroy_graph()                     # the captured step was the model-free one
+        sel = slice(None) if env_ids is None else torch.as_tensor(env_ids, device=dev, dtype=torch.long)
+        rows = n if env_ids is None else int(sel.numel())
+        new = {}
+        if mass is not None:
+            new["mass"] = torch.as_tensor(mass, dtype=f64, device=dev).expand(rows)
+        if inertia is not None:
+            i = torch.as_tensor(inertia, dtype=f64, device=dev)
+            new["inertia"] = (i.reshape(*i.shape[:-2], 9) if i.dim() >= 2 and tuple(i.shape[-2:]) == (3, 3) else i).expand(rows, 9)
+        if friction_coeffs is not None:
+            new["friction_coeffs"] = torch.as_tensor(friction_coeffs, dtype=f64, device=dev).expand(rows, 4)
+        validate_env_model(**new)
+        if "mass" in new:
+            self.env_mass[sel] = new["mass"]
+        if "inertia" in new:
+            self.env_inertia[sel] = new["inertia"]
+        if "friction_coeffs" in new:
+            self.env_friction_coeffs[sel] = new["friction_coeffs"]
 
     def _destroy_graph(self):
         if self._graph is not None:
@@ -350,7 +404,7 @@ class BatchedMPCController(Controller):
 
     def unverified_count(self):
         """Number of envs (device scalar, no synchronisation) whose last stance QP did NOT end in a verified KKT
-        point (neither RG_STATUS_POLISHED nor RG_STATUS_NO_STANCE).  The reference's OSQP path returns forces only
+        point (neither RG_STATUS_POLISHED nor RG_STATUS_NO_STANCE; an env with RG_STATUS_BAD_MODEL counts).  The reference's OSQP path returns forces only
         on OSQP_SOLVED; here such an env still gets forces -- the best interior-point iterate, feasible by
         construction -- and this counter is the signal: 0 in every batch measured so far."""
         status = self.solve_info[:, rg.RG_INFO_STATUS]
@@ -373,6 +427,28 @@ class BatchedMPCController(Controller):
             ((status & rg.RG_STATUS_NUMERIC) != 0).to(torch.float64).sum(),
             self.contact_forces.abs().to(torch.float64).sum(),
         ])
+
+
+def validate_env_model(mass=None, inertia=None, friction_coeffs=None):
+    """The checks rg_mpc_setup makes on one parameter set, applied to every row of a per-env model (float64 tensors
+    on any device: mass [..], inertia [.., 9], friction_coeffs [.., 4]).  Raises ValueError naming the first failing
+    row; the kernels flag such a row with RG_STATUS_BAD_MODEL instead."""
+    def fail(what, bad):
+        idx = torch.nonzero(bad.reshape(bad.shape[0], -1).any(dim=1) if bad.dim() else bad.reshape(1)).flatten()
+        if idx.numel():
+            raise ValueError(f"env model: {what} (first bad row {int(idx[0])})")
+    if mass is not None:
+        m = mass.to(torch.float64).reshape(-1)
+        fail("mass must be > 0 and finite", ~((m > 0) & torch.isfinite(m)))
+    if inertia is not None:
+        i = inertia.to(torch.float64).reshape(-1, 9)
+        fail("inertia must be finite", ~torch.isfinite(i))
+        det = (i[:, 0] * (i[:, 4] * i[:, 8] - i[:, 5] * i[:, 7]) + i[:, 1] * (i[:, 5] * i[:, 6] - i[:, 3] * i[:, 8]) +
+               i[:, 2] * (i[:, 3] * i[:, 7] - i[:, 4] * i[:, 6]))
+        fail("inertia must be invertible (|det| >= 1e-300)", ~(det.abs() >= 1e-300))
+    if friction_coeffs is not None:
+        f = friction_coeffs.to(torch.float64).reshape(-1, 4)
+        fail("friction coefficients must be > 0", ~(f > 0))
 
 
 def shard_bounds(n_total, rank, world_size):

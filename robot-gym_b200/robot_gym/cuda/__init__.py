@@ -23,14 +23,16 @@ RG_INFO_IPM_ITERS, RG_INFO_POLISH_ROUNDS, RG_INFO_STATUS, RG_INFO_NUM_ACTIVE = 0
 RG_STATUS_POLISHED, RG_STATUS_IPM_CONVERGED, RG_STATUS_NO_STANCE, RG_STATUS_NUMERIC = 1, 2, 4, 8
 RG_STATUS_ACTIVE_SET_ONLY = 16
 RG_STATUS_BAD_WORKSPACE = 32
+RG_STATUS_BAD_MODEL = 64
 
 # every symbol include/rg_cuda.h declares (tests check the library exports all of them)
 EXPORTED_SYMBOLS = (
     "rg_mpc_default_params", "rg_workspace_bytes", "rg_mpc_setup", "rg_mpc_release", "rg_mpc_build_solve",
-    "rg_mpc_build_solve_warm", "rg_mpc_build_solve_io",
+    "rg_mpc_build_solve_warm", "rg_mpc_build_solve_io", "rg_mpc_build_solve_model",
     "rg_robot_calibrate_ik", "rg_robot_workspace_bytes", "rg_robot_setup",
     "rg_gait_step", "rg_com_velocity_update", "rg_swing_targets", "rg_leg_ik", "rg_leg_fk", "rg_state_from_sim",
     "rg_force_to_torque", "rg_pack_hybrid_action", "rg_control_step", "rg_control_step_graph_create", "rg_control_step_graph_launch", "rg_control_step_graph_destroy",
+    "rg_control_step_model", "rg_control_step_graph_create_model",
     "rg_hybrid_motor_torque", "rg_hybrid_motor_torque_ex",
     "rg_measure_fma_peak", "rg_launch_count", "rg_last_error", "rg_version",
 )
@@ -55,6 +57,12 @@ class MpcIo(Structure):
         "com_velocity_body", "base_rpy", "base_rpy_rate", "foot_contact_state", "foot_positions_base", "command",
         "com_height", "contact_forces", "horizon_forces", "solve_info", "active_set_io", "horizon_forces_f64")] + [
         ("zero_yaw", c_int32), ("reserved_", c_int32)]
+
+
+class MpcEnvModel(Structure):
+    """``rg_mpc_env_model``: per-env mass [N], inertia [N,9] and friction coefficients [N,4] (float64 device
+    pointers, each may be NULL = the workspace's value)."""
+    _fields_ = [("mass", c_void_p), ("inertia", c_void_p), ("friction_coeffs", c_void_p)]
 
 
 class LegChain(Structure):
@@ -129,6 +137,7 @@ def load(build_if_missing: bool = False):
     lib.rg_mpc_build_solve.argtypes = [c_void_p, c_int] + [c_void_p] * 10 + [c_void_p]
     lib.rg_mpc_build_solve_warm.argtypes = [c_void_p, c_int] + [c_void_p] * 11 + [c_void_p]
     lib.rg_mpc_build_solve_io.argtypes = [c_void_p, c_int, POINTER(MpcIo), c_void_p]
+    lib.rg_mpc_build_solve_model.argtypes = [c_void_p, c_int, POINTER(MpcIo), POINTER(MpcEnvModel), c_void_p]
     lib.rg_robot_calibrate_ik.argtypes = [POINTER(RobotParams), POINTER(c_double)]
     lib.rg_robot_workspace_bytes.argtypes = [POINTER(c_size_t)]
     lib.rg_robot_setup.argtypes = [POINTER(RobotParams), c_void_p, c_size_t, c_void_p]
@@ -144,6 +153,9 @@ def load(build_if_missing: bool = False):
     lib.rg_control_step_graph_create.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), c_void_p, POINTER(c_void_p)]
     lib.rg_control_step_graph_launch.argtypes = [c_void_p, c_void_p]
     lib.rg_control_step_graph_destroy.argtypes = [c_void_p]
+    lib.rg_control_step_model.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel), c_void_p]
+    lib.rg_control_step_graph_create_model.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
+                                                       c_void_p, POINTER(c_void_p)]
     lib.rg_hybrid_motor_torque.argtypes = [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.rg_hybrid_motor_torque_ex.argtypes = [c_void_p, c_int] + [c_void_p] * 6 + [c_void_p]
     lib.rg_measure_fma_peak.argtypes = [c_int, c_int, POINTER(c_double)]
@@ -270,12 +282,15 @@ def calibrate_ik(params: RobotParams, reference_motor_angles) -> None:
 def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate, foot_contact_state,
                     foot_positions_base, command, com_height=None, contact_forces=None,
                     horizon_forces=None, solve_info=None, want_horizon=False, want_info=True, active_set=None,
-                    zero_yaw=False, horizon_forces_f64=None):
+                    zero_yaw=False, horizon_forces_f64=None, env_model=None):
     """``rg_mpc_build_solve`` (``rg_mpc_build_solve_warm`` when ``active_set`` -- an ``[N, 4*horizon]`` int16 tensor
     initialised to -1, see ``new_active_set`` -- is given) on the current stream.  ``base_rpy`` is used as given:
     pass a yaw-aligned attitude (yaw = 0) to reproduce TorqueStanceLegController (the controller's fused step
     zeroes it itself) or set ``zero_yaw``.  ``horizon_forces_f64``: optional ``[N,h,12]`` float64 output (the
-    unrounded solution; goes through ``rg_mpc_build_solve_io``).  Returns (contact_forces, horizon_forces, solve_info)."""
+    unrounded solution; goes through ``rg_mpc_build_solve_io``).  ``env_model``: per-env body and ground for this
+    solve (``rg_mpc_build_solve_model``), a dict or an object with ``mass`` [N], ``inertia`` [N,9] or [N,3,3] and
+    ``friction_coeffs`` [N,4] float64 CUDA tensors, any of them None (= the workspace's value); an env whose row fails
+    the workspace checks gets zero forces and RG_STATUS_BAD_MODEL.  Returns (contact_forces, horizon_forces, solve_info)."""
     import torch
     n = base_rpy.shape[0]
     dev = base_rpy.device
@@ -296,18 +311,38 @@ def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate
             P(com_height, torch.float32, (), allow_none=True),
             P(contact_forces, torch.float32, (12,)), hf,
             P(solve_info, torch.int32, (4,), allow_none=True))
+    model = None if env_model is None else env_model_struct(env_model, n, dev)
     with torch.cuda.device(dev):
-        if zero_yaw or horizon_forces_f64 is not None:
+        if zero_yaw or horizon_forces_f64 is not None or model is not None:
             io = MpcIo(*[a if a is None or isinstance(a, int) else a.value for a in args[2:]],
                        None if active_set is None else P(active_set, torch.int16, (4 * ws.horizon,)).value,
                        None if horizon_forces_f64 is None else P(horizon_forces_f64.view(n, ws.horizon * 12), torch.float64, (ws.horizon * 12,)).value,
                        1 if zero_yaw else 0, 0)
-            check(load().rg_mpc_build_solve_io(ws.ptr, n, ctypes.byref(io), current_stream_ptr()))
+            if model is None:
+                check(load().rg_mpc_build_solve_io(ws.ptr, n, ctypes.byref(io), current_stream_ptr()))
+            else:
+                check(load().rg_mpc_build_solve_model(ws.ptr, n, ctypes.byref(io), ctypes.byref(model), current_stream_ptr()))
         elif active_set is None:
             check(load().rg_mpc_build_solve(*args, current_stream_ptr()))
         else:
             check(load().rg_mpc_build_solve_warm(*args, P(active_set, torch.int16, (4 * ws.horizon,)), current_stream_ptr()))
     return contact_forces, horizon_forces, solve_info
+
+
+def env_model_struct(env_model, n, device) -> MpcEnvModel:
+    """``MpcEnvModel`` of a dict / object with ``mass`` [N], ``inertia`` [N,9] or [N,3,3], ``friction_coeffs`` [N,4]
+    float64 CUDA tensors (any may be None or absent), after the ``_ptr`` checks.  The tensors must outlive the solve."""
+    import torch
+    get = env_model.get if isinstance(env_model, dict) else lambda k: getattr(env_model, k, None)
+    mass, inertia, mu = get("mass"), get("inertia"), get("friction_coeffs")
+    if inertia is not None and isinstance(inertia, torch.Tensor) and inertia.dim() == 3:
+        if tuple(inertia.shape[1:]) != (3, 3):
+            raise ValueError(f"expected inertia [N,9] or [N,3,3], got {tuple(inertia.shape)}")
+        inertia = inertia.view(inertia.shape[0], 9) if inertia.is_contiguous() else inertia
+    P = lambda t, tail: _ptr(t, torch.float64, tail, allow_none=True, n=n, device=device, align=8)
+    m = MpcEnvModel()
+    m.mass, m.inertia, m.friction_coeffs = P(mass, ()), P(inertia, (9,)), P(mu, (4,))
+    return m
 
 
 def new_active_set(n_env, horizon, device="cuda"):
