@@ -82,6 +82,39 @@ __host__ __device__ inline V3 leg_fk(const RgLegDev& L, const double* q, V3* jac
   return foot;
 }
 
+// Damped least squares on the exact chain, min |foot - FK(q)|, from q: the fallback of leg_ik where the Newton clean-up
+// cannot run (target out of reach or inside the abduction cylinder, or a singular straight-knee pose).  The clamped
+// closed form is the nearest reachable point only for the idealised geometry: the upper joint sits off the hip axis, so
+// turning the hip can bring a straight leg closer.  Steps (J^T J + 1e-6 I) d = J^T err, capped at 0.5 rad, as the
+// damped IK of the reference's kinematics; a step is kept only while it reduces the distance.
+__host__ __device__ __noinline__ void leg_ik_dls(const RgLegDev& L, V3 foot, double* q) {
+  double best[3] = {q[0], q[1], q[2]};
+  double best_e = 1e300;
+  for (int it = 0; it < 32; ++it) {
+    V3 jac[3];
+    const V3 err = sub(foot, leg_fk(L, q, jac));
+    const double e = dot(err, err);
+    if (!(e < best_e)) break;                          // no progress (or not finite): the best iterate stands
+    best[0] = q[0]; best[1] = q[1]; best[2] = q[2];
+    best_e = e;
+    const double lam = 1e-6;
+    const double a00 = dot(jac[0], jac[0]) + lam, a01 = dot(jac[0], jac[1]), a02 = dot(jac[0], jac[2]);
+    const double a11 = dot(jac[1], jac[1]) + lam, a12 = dot(jac[1], jac[2]), a22 = dot(jac[2], jac[2]) + lam;
+    const double g0 = dot(jac[0], err), g1 = dot(jac[1], err), g2 = dot(jac[2], err);
+    const double c00 = a11 * a22 - a12 * a12, c01 = a02 * a12 - a01 * a22, c02 = a01 * a12 - a02 * a11;
+    const double c11 = a00 * a22 - a02 * a02, c12 = a01 * a02 - a00 * a12, c22 = a00 * a11 - a01 * a01;
+    const double id = 1.0 / (a00 * c00 + a01 * c01 + a02 * c02);
+    double d0 = (c00 * g0 + c01 * g1 + c02 * g2) * id;
+    double d1 = (c01 * g0 + c11 * g1 + c12 * g2) * id;
+    double d2 = (c02 * g0 + c12 * g1 + c22 * g2) * id;
+    const double nrm = sqrt(d0 * d0 + d1 * d1 + d2 * d2);
+    if (nrm < 1e-13) break;
+    if (nrm > 0.5) { const double s = 0.5 / nrm; d0 *= s; d1 *= s; d2 *= s; }
+    q[0] = wrap_pi(q[0] + d0); q[1] = wrap_pi(q[1] + d1); q[2] = wrap_pi(q[2] + d2);
+  }
+  q[0] = best[0]; q[1] = best[1]; q[2] = best[2];
+}
+
 // Closed-form IK (derivation in DESIGN.md 4.3): hip abduction from the projection onto the plane
 // normal to the hip axis, then a planar two-link problem in the plane normal to the upper axis.
 __host__ __device__ inline void leg_ik(const RgLegDev& L, V3 foot, double* q) {
@@ -107,11 +140,11 @@ __host__ __device__ inline void leg_ik(const RgLegDev& L, V3 foot, double* q) {
     const V3 err = sub(foot, leg_fk(L, q, jac));
     const V3 c12 = cross(jac[1], jac[2]);
     const double det = dot(jac[0], c12);
-    if (fabs(det) < 1e-12) break;                      // singular pose (straight leg): keep the closed form
+    if (fabs(det) < 1e-12) { leg_ik_dls(L, foot, q); return; }                      // singular pose (straight leg)
     const double d0 = dot(err, c12) / det;
     const double d1 = dot(jac[0], cross(err, jac[2])) / det;
     const double d2 = dot(jac[0], cross(jac[1], err)) / det;
-    if (fabs(d0) + fabs(d1) + fabs(d2) > 0.1) break;   // target out of reach: the clamped closed form stands
+    if (fabs(d0) + fabs(d1) + fabs(d2) > 0.1) { leg_ik_dls(L, foot, q); return; }   // target out of reach
     q[0] = wrap_pi(q[0] + d0); q[1] = wrap_pi(q[1] + d1); q[2] = wrap_pi(q[2] + d2);
   }
 }

@@ -122,6 +122,83 @@ def make_states(n_env, description, schedule_ctrl=None, all_stance=False, nomina
     )
 
 
+OFF_NOMINAL_FAMILIES = ("tilted", "steep_pitch", "fast", "landing", "liftoff", "feet_far", "feet_coincident",
+                        "feet_colinear", "feet_high", "patterns")
+
+
+def make_off_nominal_states(n_env, family, description=None, seed=SEED):
+    """States an RL batch reaches and ``make_states`` does not: ``make_states(n_env, description, seed=seed)`` with
+    the fields of one family overridden by float32 draws from a generator seeded with (seed, family index).
+
+    tilted: roll, pitch ~U(-1,1), yaw ~U(-3,3).  steep_pitch: roll ~U(-0.3,0.3), |pitch| ~U(1.3,1.5) with a random
+    sign (cos(pitch) >= 0.07: the entries of T(rpy) reach ~14).  fast: v_body ~U(-3,3)^3, rates ~U(-6,6)^3, command
+    (vx, vy, wz) ~U(+-2, +-1, +-3) plus the robot's offsets.  landing: v_z ~U(-3,-1.5), four feet in stance.
+    liftoff: v_z ~U(1,3).  feet_far: feet + U(-0.2,0.2) per coordinate.  feet_coincident: foot 3 := foot 0,
+    foot 1 := foot 2, four feet in stance.  feet_colinear: every foot y := 0, four feet in stance (no roll
+    authority).  feet_high: every foot z ~U(-0.02,0.02) (estimated CoM height near 0).  patterns: contact pattern =
+    env index mod 16 (bit l = leg l), v_body ~U(-2,2)^3.  v_z is the body-frame z velocity; the world-frame
+    velocity and the quaternion are recomputed from the overridden body velocity and attitude.  Measured contacts
+    equal the planned ones wherever a family sets the contact pattern."""
+    if family not in OFF_NOMINAL_FAMILIES:
+        raise ValueError(f"unknown family {family!r}; expected one of {OFF_NOMINAL_FAMILIES}")
+    if description is None:
+        from robot_gym.model.robots.descriptions import GHOST
+        description = GHOST
+    ctrl = description.GetCtrlConstants()
+    st = make_states(n_env, description, seed=seed)
+    n = len(st)
+    rng = np.random.default_rng((int(seed), OFF_NOMINAL_FAMILIES.index(family)))
+    rpy = st.base_rpy.astype(np.float64)
+    v_body = st.com_velocity_body.astype(np.float64)
+    feet = st.foot_positions_base.astype(np.float64).reshape(n, 4, 3)
+    contacts = None
+    if family == "tilted":
+        rpy[:, :2] = rng.uniform(-1.0, 1.0, (n, 2))
+        rpy[:, 2] = rng.uniform(-3.0, 3.0, n)
+    elif family == "steep_pitch":
+        rpy[:, 0] = rng.uniform(-0.3, 0.3, n)
+        rpy[:, 1] = rng.uniform(1.3, 1.5, n) * rng.choice([-1.0, 1.0], n)
+    elif family == "fast":
+        v_body = rng.uniform(-3.0, 3.0, (n, 3))
+        st.base_rpy_rate = rng.uniform(-6.0, 6.0, (n, 3)).astype(np.float32)
+        cmd = rng.uniform(-1.0, 1.0, (n, 3)) * np.array([2.0, 1.0, 3.0])
+        st.command = (cmd + np.array([ctrl.VX_OFFSET, ctrl.VY_OFFSET, ctrl.WZ_OFFSET])).astype(np.float32)
+    elif family == "landing":
+        v_body[:, 2] = rng.uniform(-3.0, -1.5, n)
+        contacts = np.ones((n, 4), dtype=bool)
+    elif family == "liftoff":
+        v_body[:, 2] = rng.uniform(1.0, 3.0, n)
+    elif family == "feet_far":
+        feet = feet + rng.uniform(-0.2, 0.2, (n, 4, 3))
+    elif family == "feet_coincident":
+        feet[:, 3] = feet[:, 0]
+        feet[:, 1] = feet[:, 2]
+        contacts = np.ones((n, 4), dtype=bool)
+    elif family == "feet_colinear":
+        feet[:, :, 1] = 0.0
+        contacts = np.ones((n, 4), dtype=bool)
+    elif family == "feet_high":
+        feet[:, :, 2] = rng.uniform(-0.02, 0.02, (n, 4))
+    elif family == "patterns":
+        contacts = ((np.arange(n)[:, None] % 16) >> np.arange(4)[None, :]) & 1 != 0
+        v_body = rng.uniform(-2.0, 2.0, (n, 3))
+    if contacts is not None:
+        st.planned_contacts = contacts.astype(np.uint8)
+        st.foot_contacts = contacts.astype(np.uint8)
+    rpy32 = rpy.astype(np.float32)
+    quat = euler_to_quat_xyzw(rpy32.astype(np.float64))
+    x, y, z, w = quat.T
+    rot = np.stack([1 - 2 * (y * y + z * z), 2 * (x * y - z * w), 2 * (x * z + y * w),
+                    2 * (x * y + z * w), 1 - 2 * (x * x + z * z), 2 * (y * z - x * w),
+                    2 * (x * z - y * w), 2 * (y * z + x * w), 1 - 2 * (x * x + y * y)], axis=1).reshape(n, 3, 3)
+    st.base_rpy = rpy32
+    st.base_orientation_xyzw = quat.astype(np.float32)
+    st.com_velocity_body = v_body.astype(np.float32)
+    st.base_velocity_world = np.einsum("nij,nj->ni", rot, v_body).astype(np.float32)
+    st.foot_positions_base = np.ascontiguousarray(feet.reshape(n, 12).astype(np.float32))
+    return st
+
+
 def make_state_sequence(n_env, n_steps, description, schedule_ctrl=None, seed=SEED, control_dt_ticks=10):
     """``n_steps`` consecutive control steps for ``n_env`` envs: every step draws a fresh random
     state (no physics), while the clock advances like Simulation's: t = step_counter * 0.001 with
