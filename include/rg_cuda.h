@@ -67,6 +67,10 @@ enum {
                                     and finite, inertia finite and invertible, friction coefficients > 0): forces and
                                     horizon outputs are zero, the warm-start set is reset, nothing was solved */
 };
+/* A row of an rg_gait_env_params (below) that is not valid has no status bit: the control step holds every leg of
+ * that env in stance -- desired_leg_state = leg_state = RG_LEG_STANCE, mpc_contact_state = 1, normalized_phase = -1.0
+ * (a value a valid row never produces: t >= 0 and the phase lies in [0, 1)), no swing target, last_leg_state = STANCE
+ * -- so the env stands on the stance solve.  The other envs of the batch are not affected. */
 
 /* ---- ConvexMpc constructor arguments + the constants compiled into mpc_osqp ------------
  * Replaces: mpc_osqp.ConvexMpc(...) as constructed by TorqueStanceLegController
@@ -381,6 +385,32 @@ int rg_control_step_model(const void* mpc_workspace, const void* robot_workspace
 int rg_control_step_graph_create_model(const void* mpc_workspace, const void* robot_workspace, int n_env,
                                        const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
                                        void* stream, void** graph_out);
+
+/* Per-env OpenloopGaitGenerator arguments (mpc_controller.py:30-35): what each reference process passes to its own
+ * OpenloopGaitGenerator(stance_duration, duty_factor, initial_leg_phase, initial_leg_state).  DEVICE arrays, env-major,
+ * each [N,4] (leg order FR, FL, RR, RL) and each may be NULL (= the robot workspace's value for every env).  Read on
+ * every launch (a captured graph included), so values written in place between replays take effect at the next step,
+ * at the env's current clock.  A row is valid when, for every leg, stance_duration > 0 and finite,
+ * 0 < duty_factor <= 1, 0 <= initial_leg_phase < 1 and initial_leg_state is RG_LEG_SWING or RG_LEG_STANCE (the
+ * workspace's value standing in for a NULL array).  The kernel decides validity from the values it loads (no host check); an invalid
+ * row holds its env in stance (see the note after the status bits).  The stance duration also sets the Raibert
+ * foothold of the swing legs (hv * stance_duration / 2). */
+typedef struct rg_gait_env_params {
+  const double*  stance_duration;    /* [N,4] f64, 8-byte aligned */
+  const double*  duty_factor;        /* [N,4] f64, 8-byte aligned */
+  const double*  initial_leg_phase;  /* [N,4] f64, 8-byte aligned */
+  const int32_t* initial_leg_state;  /* [N,4] i32, 4-byte aligned */
+} rg_gait_env_params;
+
+/* The control step and its graph with a per-env model and a per-env gait (either may be NULL, or have all pointers
+ * NULL: the _model calls above forward here with gait = NULL and launch exactly the gait-free kernels).  A misaligned
+ * array returns RG_ERR_BAD_ARG before anything is launched.  As with the model, the graph bakes in the gait POINTERS. */
+int rg_control_step_env(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                        const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                        const rg_gait_env_params* gait_host, void* stream);
+int rg_control_step_graph_create_env(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                                     const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                                     const rg_gait_env_params* gait_host, void* stream, void** graph_out);
 
 /* ---- "next" row (SURVEY.md 8f rank 1): batched HYBRID motor model ----------------------------
  * Replaces RobotMotorModel.convert_to_torque HYBRID branch (simple_motor.py:128-139):

@@ -150,19 +150,71 @@ __host__ __device__ inline void leg_ik(const RgLegDev& L, V3 foot, double* q) {
 }
 
 // ------------------------------------------------------------------------------------ gait
+// One leg's OpenloopGaitGenerator arguments and what its __init__ derives from them (ratio = the share of the cycle
+// spent in the initial state, next = the state after it), from one of two sources with the same accessors:
+//  * WorkspaceGait reads the robot workspace (ratio and next precomputed by rg_robot_setup) at the point of use, so the
+//    gait-free kernels load exactly what and when they always have;
+//  * EnvGait holds one leg of a per-env gait (rg_gait_env_params), loaded once, ratio and next derived on the device
+//    as OpenloopGaitGenerator.__init__ / rg_robot_setup derive them (1 - duty is one IEEE subtraction in all three).
+struct WorkspaceGait {
+  static constexpr bool kPerEnv = false;
+  const RgRobotDev& R;
+  int leg;
+  __device__ __forceinline__ static WorkspaceGait load(const RgRobotDev& R, const rg_gait_env_params&, size_t, int leg) {
+    return WorkspaceGait{R, leg};
+  }
+  __device__ __forceinline__ bool valid() const { return true; }
+  __device__ __forceinline__ double stance() const { return R.stance_duration[leg]; }
+  __device__ __forceinline__ double duty() const { return R.duty_factor[leg]; }
+  __device__ __forceinline__ double phase0() const { return R.initial_leg_phase[leg]; }
+  __device__ __forceinline__ double ratio() const { return R.initial_state_ratio[leg]; }
+  __device__ __forceinline__ int init() const { return R.initial_leg_state[leg]; }
+  __device__ __forceinline__ int next() const { return R.next_leg_state[leg]; }
+};
+
+struct EnvGait {
+  static constexpr bool kPerEnv = true;
+  double st, du, ph, ra;
+  int in, nx;
+  // leg idx (= 4 env + leg) of a per-env gait; a NULL array stands for the workspace's value
+  __device__ __forceinline__ static EnvGait load(const RgRobotDev& R, const rg_gait_env_params& g, size_t idx, int leg) {
+    EnvGait o;
+    o.st = g.stance_duration ? g.stance_duration[idx] : R.stance_duration[leg];
+    o.du = g.duty_factor ? g.duty_factor[idx] : R.duty_factor[leg];
+    o.ph = g.initial_leg_phase ? g.initial_leg_phase[idx] : R.initial_leg_phase[leg];
+    o.in = g.initial_leg_state ? g.initial_leg_state[idx] : R.initial_leg_state[leg];
+    const bool swing_first = o.in == RG_LEG_SWING;
+    o.ra = swing_first ? __dsub_rn(1.0, o.du) : o.du;
+    o.nx = swing_first ? RG_LEG_STANCE : RG_LEG_SWING;
+    return o;
+  }
+  // the row rule of rg_gait_env_params (rg_cuda.h); NaN fails every comparison
+  __device__ __forceinline__ bool valid() const {
+    return st > 0.0 && st <= 1.7976931348623157e308 && du > 0.0 && du <= 1.0 && ph >= 0.0 && ph < 1.0 &&
+           (in == RG_LEG_SWING || in == RG_LEG_STANCE);
+  }
+  __device__ __forceinline__ double stance() const { return st; }
+  __device__ __forceinline__ double duty() const { return du; }
+  __device__ __forceinline__ double phase0() const { return ph; }
+  __device__ __forceinline__ double ratio() const { return ra; }
+  __device__ __forceinline__ int init() const { return in; }
+  __device__ __forceinline__ int next() const { return nx; }
+};
+
 // OpenloopGaitGenerator.update(t) for one leg; every operation is a separately rounded IEEE double
 // operation in CPython's order, so phases and states are bit-identical to the reference's floats.
-__device__ __forceinline__ void gait_leg(const RgRobotDev& R, int leg, double t, bool contact,
+template <class Gait>
+__device__ __forceinline__ void gait_leg(const RgRobotDev& R, const Gait& g, double t, bool contact,
                                          int& desired, int& state, double& nphase) {
-  const double period = __ddiv_rn(R.stance_duration[leg], R.duty_factor[leg]);
-  const double aug = __dadd_rn(t, __dmul_rn(R.initial_leg_phase[leg], period));
+  const double period = __ddiv_rn(g.stance(), g.duty());
+  const double aug = __dadd_rn(t, __dmul_rn(g.phase0(), period));
   const double ph = __ddiv_rn(fmod(aug, period), period);
-  const double ratio = R.initial_state_ratio[leg];
+  const double ratio = g.ratio();
   if (ph < ratio) {
-    desired = R.initial_leg_state[leg];
+    desired = g.init();
     nphase = __ddiv_rn(ph, ratio);
   } else {
-    desired = R.next_leg_state[leg];
+    desired = g.next();
     nphase = __ddiv_rn(__dsub_rn(ph, ratio), __dsub_rn(1.0, ratio));
   }
   state = desired;
@@ -179,7 +231,7 @@ __global__ void gait_kernel(const RgRobotDev* __restrict__ R, int n_env, const d
   const int env = idx >> 2, leg = idx & 3;
   int d, s;
   double np;
-  gait_leg(*R, leg, t[env], contacts[idx] != 0, d, s, np);
+  gait_leg(*R, WorkspaceGait{*R, leg}, t[env], contacts[idx] != 0, d, s, np);
   desired[idx] = d;
   state[idx] = s;
   nphase[idx] = np;
@@ -257,7 +309,8 @@ __device__ __forceinline__ double gen_parabola(double phase, double start, doubl
 
 // RaibertSwingLegController.update (latch) + get_action up to the IK call, for one leg.
 // Returns true if a swing target was produced (leg_state not in {STANCE, EARLY_CONTACT}).
-__device__ __forceinline__ bool swing_leg(const RgRobotDev& R, int leg, int desired, int state, double nphase,
+template <class Gait>
+__device__ __forceinline__ bool swing_leg(const RgRobotDev& R, int leg, const Gait& gait, int desired, int state, double nphase,
                                           const float* foot_pos /* this leg, 3 */, const double* v_body,
                                           double yaw_dot, const float* cmd, int32_t& last_state,
                                           float* latch /* this leg, 3 */, double* target_out) {
@@ -277,7 +330,7 @@ __device__ __forceinline__ bool swing_leg(const RgRobotDev& R, int leg, int desi
   for (int a = 0; a < 3; ++a) {
     const double hv = cv[a] + yaw_dot * tw[a];
     const double thv = ds[a] + dtw * tw[a];
-    end[a] = (hv * R.stance_duration[leg] / 2.0 - R.swing_kp[a] * (thv - hv)) - hgt[a] + hip[a];
+    end[a] = (hv * gait.stance() / 2.0 - R.swing_kp[a] * (thv - hv)) - hgt[a] + hip[a];
   }
   // _gen_swing_foot_trajectory
   double phase;
@@ -302,7 +355,7 @@ __global__ void swing_kernel(const RgRobotDev* __restrict__ R, int n_env, const 
   const double vb[3] = {v_body[3 * (size_t)env], v_body[3 * (size_t)env + 1], v_body[3 * (size_t)env + 2]};
   int32_t ls = last_state[idx];
   double tg[3];
-  const bool has = swing_leg(*R, leg, desired[idx], state[idx], nphase[idx], feet + 3 * (size_t)idx, vb,
+  const bool has = swing_leg(*R, leg, WorkspaceGait{*R, leg}, desired[idx], state[idx], nphase[idx], feet + 3 * (size_t)idx, vb,
                              (double)rpy_rate[3 * (size_t)env + 2], cmd + 3 * (size_t)env, ls, latch + 3 * (size_t)idx, tg);
   last_state[idx] = ls;
   if (has) for (int a = 0; a < 3; ++a) target[3 * (size_t)idx + a] = (float)tg[a];
@@ -433,7 +486,13 @@ __global__ void pack_kernel(const RgRobotDev* __restrict__ R, int n_env, const i
 // adjacent lanes; the estimator's three axes are updated by the lanes of legs 0-2 and handed round with shuffles (a
 // single thread per env did the four legs and three axes one after the other: 4x the dependent chain at N = 1 and a
 // quarter of the threads at large N).  Epilogue: J^T force -> torque + pack, one thread per leg.
-__global__ void step_prologue_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
+// Gait = EnvGait: the gait of each env comes from `gp` (rg_gait_env_params) instead of the workspace.  The gait-free
+// kernels instantiate the bodies with WorkspaceGait and keep their own parameter list (an extra kernel parameter, even an
+// unused one, moves ptxas's register assignment: DESIGN.md §3.12), so they compile to the code they had before the
+// per-env gait existed (DESIGN.md §3.14).
+template <class Gait>
+__device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__ R, int n_env, const rg_controller_state& s,
+                                                  const rg_gait_env_params& gp) {
   RG_GRID_LAUNCH_DEPENDENTS();   // the solve kernel is launched programmatically behind this grid (rg_control_step)
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int env = (int)(idx >> 2), leg = (int)(idx & 3);
@@ -464,14 +523,21 @@ __global__ void step_prologue_kernel(const RgRobotDev* __restrict__ R, int n_env
   const double yaw_dot = (double)s.base_rpy_rate[3 * (size_t)env + 2];
   int d, st;
   double np;
-  gait_leg(*R, leg, t, s.foot_contacts[idx] != 0, d, st, np);
+  const Gait g = Gait::load(*R, gp, idx, leg);
+  // a row is valid when its four legs are: the four lanes of the env vote (all four are past the `ok` return)
+  if (!Gait::kPerEnv || __all_sync(0xfu << lane0, g.valid())) {
+    gait_leg(*R, g, t, s.foot_contacts[idx] != 0, d, st, np);
+  } else {
+    d = st = RG_LEG_STANCE;
+    np = -1.0;
+  }
   s.desired_leg_state[idx] = d;
   s.leg_state[idx] = st;
   s.normalized_phase[idx] = np;
   s.mpc_contact_state[idx] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
   int32_t ls = s.last_leg_state[idx];
   double tg[3];
-  const bool has = swing_leg(*R, leg, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
+  const bool has = swing_leg(*R, leg, g, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
                              s.command + 3 * (size_t)env, ls, s.phase_switch_foot_local_position + 3 * idx, tg);
   s.last_leg_state[idx] = ls;
   if (has) {
@@ -490,7 +556,9 @@ __global__ void step_prologue_kernel(const RgRobotDev* __restrict__ R, int n_env
 // The same prologue with one thread per env (the four legs unrolled): fewer, fatter threads -- the faster mapping for
 // large batches, where the kernel is bound by its FP64 instruction count and per-leg lanes diverge (swing legs run the IK,
 // stance legs idle).  Bit-identical results: both call the same per-leg / per-axis routines.
-__global__ void step_prologue_env_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
+template <class Gait>
+__device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__ R, int n_env, const rg_controller_state& s,
+                                                  const rg_gait_env_params& gp) {
   RG_GRID_LAUNCH_DEPENDENTS();   // the solve kernel is launched programmatically behind this grid (rg_control_step)
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= n_env) return;
@@ -504,18 +572,28 @@ __global__ void step_prologue_env_kernel(const RgRobotDev* __restrict__ R, int n
   const double vbr[3] = {(double)vbf[0], (double)vbf[1], (double)vbf[2]};
   const double t = s.time_since_reset[env];
   const double yaw_dot = (double)s.base_rpy_rate[3 * (size_t)env + 2];
+  // the row's validity first (a pass over its four legs: holding the four legs' values live costs registers)
+  bool valid = true;
+  if (Gait::kPerEnv)
+    for (int leg = 0; leg < 4; ++leg) valid = valid && Gait::load(*R, gp, 4 * (size_t)env + leg, leg).valid();
   for (int leg = 0; leg < 4; ++leg) {
     const size_t idx = 4 * (size_t)env + leg;
     int d, st;
     double np;
-    gait_leg(*R, leg, t, s.foot_contacts[idx] != 0, d, st, np);
+    const Gait g = Gait::load(*R, gp, idx, leg);
+    if (valid) {
+      gait_leg(*R, g, t, s.foot_contacts[idx] != 0, d, st, np);
+    } else {
+      d = st = RG_LEG_STANCE;
+      np = -1.0;
+    }
     s.desired_leg_state[idx] = d;
     s.leg_state[idx] = st;
     s.normalized_phase[idx] = np;
     s.mpc_contact_state[idx] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
     int32_t ls = s.last_leg_state[idx];
     double tg[3];
-    const bool has = swing_leg(*R, leg, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
+    const bool has = swing_leg(*R, leg, g, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
                                s.command + 3 * (size_t)env, ls, s.phase_switch_foot_local_position + 3 * idx, tg);
     s.last_leg_state[idx] = ls;
     if (has) {
@@ -530,6 +608,26 @@ __global__ void step_prologue_env_kernel(const RgRobotDev* __restrict__ R, int n
       s.swing_joint_valid[idx] = 1;
     }
   }
+}
+
+__global__ void step_prologue_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
+  step_prologue_leg<WorkspaceGait>(R, n_env, s, rg_gait_env_params{});
+}
+
+__global__ void step_prologue_env_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
+  step_prologue_env<WorkspaceGait>(R, n_env, s, rg_gait_env_params{});
+}
+
+// Per-env gait (rg_control_step_env): each (env, leg) loads its own 28 B of gait arguments, coalesced in the per-leg
+// mapping.  An invalid row holds its env in stance (rg_cuda.h).
+__global__ void step_prologue_gait_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
+                                          rg_gait_env_params gp) {
+  step_prologue_leg<EnvGait>(R, n_env, s, gp);
+}
+
+__global__ void step_prologue_env_gait_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
+                                              rg_gait_env_params gp) {
+  step_prologue_env<EnvGait>(R, n_env, s, gp);
 }
 
 __global__ void step_epilogue_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
@@ -837,6 +935,27 @@ extern "C" int rg_control_step(const void* mpc_ws, const void* robot_ws, int n_e
 
 extern "C" int rg_control_step_model(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                      const rg_mpc_env_model* model, void* stream) {
+  return rg_control_step_env(mpc_ws, robot_ws, n_env, s, model, nullptr, stream);
+}
+
+// NULL, or a gait whose four pointers are all NULL -> NULL (the gait-free prologues); RG_ERR_BAD_ARG for a misaligned array
+static int rg_check_env_gait(const rg_gait_env_params* gait, const char* what, const rg_gait_env_params** out) {
+  *out = nullptr;
+  if (!gait || (!gait->stance_duration && !gait->duty_factor && !gait->initial_leg_phase && !gait->initial_leg_state)) return RG_OK;
+  if (((uintptr_t)gait->stance_duration | (uintptr_t)gait->duty_factor | (uintptr_t)gait->initial_leg_phase) & 7u) {
+    rg_set_error("%s: gait arrays stance_duration, duty_factor and initial_leg_phase must be 8-byte aligned float64", what);
+    return RG_ERR_BAD_ARG;
+  }
+  if ((uintptr_t)gait->initial_leg_state & 3u) {
+    rg_set_error("%s: gait array initial_leg_state must be 4-byte aligned int32", what);
+    return RG_ERR_BAD_ARG;
+  }
+  *out = gait;
+  return RG_OK;
+}
+
+extern "C" int rg_control_step_env(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                   const rg_mpc_env_model* model, const rg_gait_env_params* gait, void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
   RG_REQUIRE(mpc_ws && robot_ws && s && n_env >= 0, "rg_control_step");
   RG_REQUIRE(s->time_since_reset && s->foot_contacts && s->base_velocity_world && s->base_orientation_xyzw && s->base_rpy &&
@@ -849,11 +968,20 @@ extern "C" int rg_control_step_model(const void* mpc_ws, const void* robot_ws, i
   RG_REQUIRE(!s->applied_motor_torques || s->motor_velocities, "rg_control_step torque consumer (motor_velocities)");
   RG_REQUIRE(((uintptr_t)s->foot_positions_base & 15u) == 0, "rg_control_step foot_positions_base (16-byte alignment)");
   const rg_mpc_env_model* m = nullptr;
-  int rc = rg_check_env_model(model, "rg_control_step_model", &m);
+  int rc = rg_check_env_model(model, "rg_control_step_env", &m);
+  if (rc != RG_OK) return rc;
+  const rg_gait_env_params* g = nullptr;
+  rc = rg_check_env_gait(gait, "rg_control_step_env", &g);
   if (rc != RG_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS) step_prologue_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>((const RgRobotDev*)robot_ws, n_env, *s);
-  else step_prologue_env_kernel<<<grid_for(n_env, 128), 128, 0, st>>>((const RgRobotDev*)robot_ws, n_env, *s);
+  const RgRobotDev* R = (const RgRobotDev*)robot_ws;
+  if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS) {
+    if (g) step_prologue_gait_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, *g);
+    else step_prologue_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s);
+  } else {
+    if (g) step_prologue_env_gait_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s, *g);
+    else step_prologue_env_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s);
+  }
   rg_count_launch();
   rc = rg_check_cuda(cudaGetLastError(), "step_prologue_kernel launch");
   if (rc != RG_OK) return rc;
@@ -900,12 +1028,18 @@ extern "C" int rg_control_step_graph_create(const void* mpc_ws, const void* robo
 
 extern "C" int rg_control_step_graph_create_model(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                                   const rg_mpc_env_model* model, void* stream, void** graph_out) {
+  return rg_control_step_graph_create_env(mpc_ws, robot_ws, n_env, s, model, nullptr, stream, graph_out);
+}
+
+extern "C" int rg_control_step_graph_create_env(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                                const rg_mpc_env_model* model, const rg_gait_env_params* gait, void* stream,
+                                                void** graph_out) {
   RG_REQUIRE(mpc_ws && robot_ws && s && graph_out && n_env > 0, "rg_control_step_graph_create");
   *graph_out = nullptr;
   // one eager step on the caller's stream first: kernel attributes get configured outside the capture, and argument
   // errors surface here with their own message.  The controller state advances by this step -- the caller accounts for it
   // by creating the graph INSTEAD of a step, not before one (see rg_cuda.h).
-  int rc = rg_control_step_model(mpc_ws, robot_ws, n_env, s, model, stream);
+  int rc = rg_control_step_env(mpc_ws, robot_ws, n_env, s, model, gait, stream);
   if (rc == RG_OK) rc = rg_check_cuda(cudaStreamSynchronize((cudaStream_t)stream), "graph warm-up step");
   if (rc != RG_OK) return rc;
   cudaStream_t cap = nullptr;
@@ -915,7 +1049,7 @@ extern "C" int rg_control_step_graph_create_model(const void* mpc_ws, const void
   RgStepGraph* g = new RgStepGraph{nullptr, nullptr, 0};
   cudaError_t e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal);
   if (e == cudaSuccess) {
-    rc = rg_control_step_model(mpc_ws, robot_ws, n_env, s, model, cap);
+    rc = rg_control_step_env(mpc_ws, robot_ws, n_env, s, model, gait, cap);
     e = cudaStreamEndCapture(cap, &g->graph);
     if (rc != RG_OK) e = cudaErrorUnknown;
   }

@@ -93,6 +93,9 @@ class BatchedMPCController(Controller):
         self._graph_invalidations = 0
         self.env_mass = self.env_inertia = self.env_friction_coeffs = None   # per-env model (set_env_model)
         self._env_model = None
+        # per-env gait (set_env_gait)
+        self.env_stance_duration = self.env_duty_factor = self.env_initial_leg_phase = self.env_initial_leg_state = None
+        self._env_gait = None
 
         # --- C-ABI workspaces (the analogue of _setup_controller, mpc_controller.py:28-66)
         c = self._constants
@@ -190,8 +193,9 @@ class BatchedMPCController(Controller):
 
     def reset(self, env_ids=None):
         """LocomotionController.reset (mpc_controller.py:108-109): reset_time = clock(); gait, estimator,
-        swing (latch = current feet, joint-angle store cleared) and stance state are re-armed.
-        ``env_ids`` (LongTensor) restricts the reset to a subset of envs."""
+        swing (latch = current feet, joint-angle store cleared) and stance state are re-armed.  The leg states
+        start from INIT_LEG_STATE, or with a per-env gait (``set_env_gait``) from each env's own
+        ``env_initial_leg_state`` row.  ``env_ids`` (LongTensor) restricts the reset to a subset of envs."""
         sel = slice(None) if env_ids is None else env_ids
         if self._adapter is not None:
             self._adapter.refresh()
@@ -207,7 +211,10 @@ class BatchedMPCController(Controller):
         self.swing_joint_valid[sel] = 0
         if self.mpc_active_set is not None:
             self.mpc_active_set[sel] = -1   # RG_ACTIVE_SET_UNKNOWN
-        init_state = torch.tensor([int(s) for s in self._constants.INIT_LEG_STATE], dtype=torch.int32, device=self.device)
+        if self._env_gait is None:
+            init_state = torch.tensor([int(s) for s in self._constants.INIT_LEG_STATE], dtype=torch.int32, device=self.device)
+        else:                               # OpenloopGaitGenerator.reset with each env's own initial_leg_state
+            init_state = self.env_initial_leg_state[sel]
         self.desired_leg_state[sel] = init_state
         self.leg_state[sel] = init_state
         self.normalized_phase[sel] = 0
@@ -327,26 +334,33 @@ class BatchedMPCController(Controller):
                 if self._graph is None:
                     # creating the graph executes this step eagerly (and synchronises once)
                     handle = ctypes.c_void_p()
-                    if self._env_model is None:
+                    if self._env_model is None and self._env_gait is None:
                         rg.check(lib.rg_control_step_graph_create(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
                                                                   ctypes.byref(self._state), rg.current_stream_ptr(),
                                                                   ctypes.byref(handle)))
                     else:
-                        rg.check(lib.rg_control_step_graph_create_model(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
-                                                                        ctypes.byref(self._state), ctypes.byref(self._env_model),
-                                                                        rg.current_stream_ptr(), ctypes.byref(handle)))
+                        rg.check(lib.rg_control_step_graph_create_env(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
+                                                                      ctypes.byref(self._state), self._env_model_ref(),
+                                                                      self._env_gait_ref(), rg.current_stream_ptr(),
+                                                                      ctypes.byref(handle)))
                     self._graph = handle
                 else:
                     rg.check(lib.rg_control_step_graph_launch(self._graph, rg.current_stream_ptr()))
         return self.action
 
     def _eager_step(self, lib):
-        if self._env_model is None:
+        if self._env_model is None and self._env_gait is None:
             rg.check(lib.rg_control_step(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
                                          ctypes.byref(self._state), rg.current_stream_ptr()))
         else:
-            rg.check(lib.rg_control_step_model(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
-                                               ctypes.byref(self._env_model), rg.current_stream_ptr()))
+            rg.check(lib.rg_control_step_env(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
+                                             self._env_model_ref(), self._env_gait_ref(), rg.current_stream_ptr()))
+
+    def _env_model_ref(self):
+        return None if self._env_model is None else ctypes.byref(self._env_model)
+
+    def _env_gait_ref(self):
+        return None if self._env_gait is None else ctypes.byref(self._env_gait)
 
     # ------------------------------------------------------------------ per-env body and ground
     def set_env_model(self, mass=None, inertia=None, friction_coeffs=None, env_ids=None):
@@ -388,6 +402,64 @@ class BatchedMPCController(Controller):
             self.env_inertia[sel] = new["inertia"]
         if "friction_coeffs" in new:
             self.env_friction_coeffs[sel] = new["friction_coeffs"]
+
+    # ------------------------------------------------------------------ per-env gait
+    def set_env_gait(self, stance_duration=None, duty_factor=None, initial_leg_phase=None, initial_leg_state=None,
+                     schedule=None, env_ids=None):
+        """Per-env ``OpenloopGaitGenerator(stance_duration, duty_factor, initial_leg_phase, initial_leg_state)``
+        arguments, each [N,4] (leg order FR, FL, RR, RL) -- what each reference process passes to its own gait
+        generator (mpc_controller.py:30-35).  ``schedule`` (a name of ``descriptions.GAIT_SCHEDULES``: trot, pace,
+        bound, walk, stand) supplies all four instead.  Scalars and [4] rows broadcast; with ``env_ids`` only those rows
+        are written.  The stance duration also sets the Raibert foothold of the swing legs.
+
+        The first call allocates controller-owned tensors (``env_stance_duration``, ``env_duty_factor``,
+        ``env_initial_leg_phase`` float64 and ``env_initial_leg_state`` int32, [N,4]) filled with the robot's gait
+        constants and drops the captured step graph once; later calls write into them in place, so a captured graph
+        stays valid.  Raises ``ValueError`` before anything is written for a stance duration that is not > 0 and
+        finite, a duty factor outside (0, 1], a phase outside [0, 1) or a state other than SWING / STANCE.
+
+        The new timing applies from the next step, at each env's current clock (``time_since_reset``): this call
+        does not reset.  A task that wants the envs to start a fresh cycle calls ``reset(env_ids)`` after it, which
+        re-arms their leg states from the new ``initial_leg_state`` rows.  Synchronises once."""
+        from robot_gym.model.robots.descriptions import GAIT_SCHEDULES
+        n, dev, f64, i32 = self.num_envs, self.device, torch.float64, torch.int32
+        given = dict(stance_duration=stance_duration, duty_factor=duty_factor, initial_leg_phase=initial_leg_phase,
+                     initial_leg_state=initial_leg_state)
+        if schedule is not None:
+            if any(v is not None for v in given.values()):
+                raise ValueError("set_env_gait: pass either schedule= or the gait arrays, not both")
+            if schedule not in GAIT_SCHEDULES:
+                raise ValueError(f"unknown gait schedule {schedule!r}; expected one of {tuple(GAIT_SCHEDULES)}")
+            given = _gait_rows(GAIT_SCHEDULES[schedule])
+        sel = slice(None) if env_ids is None else torch.as_tensor(env_ids, device=dev, dtype=torch.long)
+        rows = n if env_ids is None else int(sel.numel())
+        new = {}
+        for key, value in given.items():
+            if value is None:
+                continue
+            if key == "initial_leg_state":
+                t = torch.as_tensor(value if isinstance(value, torch.Tensor) else np.asarray(value), device=dev)
+                if t.is_floating_point() and not torch.equal(t, t.round()):
+                    raise ValueError("env gait: initial_leg_state must hold integer leg states")
+                new[key] = t.to(i32).expand(rows, 4)
+            else:
+                new[key] = torch.as_tensor(value, dtype=f64, device=dev).expand(rows, 4)
+        validate_env_gait(**new)
+        if self._env_gait is None:
+            c = _gait_rows(self._constants)            # the robot workspace's own gait (robot_params_from_description)
+            self.env_stance_duration = torch.tensor(c["stance_duration"], dtype=f64, device=dev).repeat(n, 1)
+            self.env_duty_factor = torch.tensor(c["duty_factor"], dtype=f64, device=dev).repeat(n, 1)
+            self.env_initial_leg_phase = torch.tensor(c["initial_leg_phase"], dtype=f64, device=dev).repeat(n, 1)
+            self.env_initial_leg_state = torch.tensor(c["initial_leg_state"], dtype=i32, device=dev).repeat(n, 1)
+            gait = rg.GaitEnvParams()
+            gait.stance_duration = rg._ptr(self.env_stance_duration, f64, (4,), n=n, device=dev, align=8)
+            gait.duty_factor = rg._ptr(self.env_duty_factor, f64, (4,), n=n, device=dev, align=8)
+            gait.initial_leg_phase = rg._ptr(self.env_initial_leg_phase, f64, (4,), n=n, device=dev, align=8)
+            gait.initial_leg_state = rg._ptr(self.env_initial_leg_state, i32, (4,), n=n, device=dev, align=4)
+            self._env_gait = gait
+            self._destroy_graph()                     # the captured step was the gait-free one
+        for key, value in new.items():
+            getattr(self, "env_" + key)[sel] = value
 
     def _destroy_graph(self):
         if self._graph is not None:
@@ -449,6 +521,37 @@ def validate_env_model(mass=None, inertia=None, friction_coeffs=None):
     if friction_coeffs is not None:
         f = friction_coeffs.to(torch.float64).reshape(-1, 4)
         fail("friction coefficients must be > 0", ~(f > 0))
+
+
+def _gait_rows(ctrl):
+    """The four OpenloopGaitGenerator arguments of a ctrl-constants module or a GAIT_SCHEDULES entry, as [4] lists."""
+    get = ctrl.get if isinstance(ctrl, dict) else lambda k: getattr(ctrl, k)
+    return dict(stance_duration=[float(v) for v in get("STANCE_DURATION_SECONDS")],
+                duty_factor=[float(v) for v in get("DUTY_FACTOR")],
+                initial_leg_phase=[float(v) for v in get("INIT_PHASE_FULL_CYCLE")],
+                initial_leg_state=[int(v) for v in get("INIT_LEG_STATE")])
+
+
+def validate_env_gait(stance_duration=None, duty_factor=None, initial_leg_phase=None, initial_leg_state=None):
+    """The row rule of rg_gait_env_params (include/rg_cuda.h) on [.., 4] tensors on any device: stance_duration > 0
+    and finite, 0 < duty_factor <= 1, 0 <= initial_leg_phase < 1, initial_leg_state SWING (0) or STANCE (1).
+    Raises ValueError naming the first failing row; the control step holds such an env in stance instead."""
+    def fail(what, bad):
+        idx = torch.nonzero(bad.reshape(-1, 4).any(dim=1)).flatten()
+        if idx.numel():
+            raise ValueError(f"env gait: {what} (first bad row {int(idx[0])})")
+    if stance_duration is not None:
+        s = stance_duration.to(torch.float64)
+        fail("stance_duration must be > 0 and finite", ~((s > 0) & torch.isfinite(s)))
+    if duty_factor is not None:
+        d = duty_factor.to(torch.float64)
+        fail("duty_factor must lie in (0, 1]", ~((d > 0) & (d <= 1)))
+    if initial_leg_phase is not None:
+        p = initial_leg_phase.to(torch.float64)
+        fail("initial_leg_phase must lie in [0, 1)", ~((p >= 0) & (p < 1)))
+    if initial_leg_state is not None:
+        st = initial_leg_state
+        fail("initial_leg_state must be SWING (0) or STANCE (1)", ~((st == int(LegState.SWING)) | (st == int(LegState.STANCE))))
 
 
 def shard_bounds(n_total, rank, world_size):

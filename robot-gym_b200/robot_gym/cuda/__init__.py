@@ -32,7 +32,7 @@ EXPORTED_SYMBOLS = (
     "rg_robot_calibrate_ik", "rg_robot_workspace_bytes", "rg_robot_setup",
     "rg_gait_step", "rg_com_velocity_update", "rg_swing_targets", "rg_leg_ik", "rg_leg_fk", "rg_state_from_sim",
     "rg_force_to_torque", "rg_pack_hybrid_action", "rg_control_step", "rg_control_step_graph_create", "rg_control_step_graph_launch", "rg_control_step_graph_destroy",
-    "rg_control_step_model", "rg_control_step_graph_create_model",
+    "rg_control_step_model", "rg_control_step_graph_create_model", "rg_control_step_env", "rg_control_step_graph_create_env",
     "rg_hybrid_motor_torque", "rg_hybrid_motor_torque_ex",
     "rg_measure_fma_peak", "rg_launch_count", "rg_last_error", "rg_version",
 )
@@ -63,6 +63,13 @@ class MpcEnvModel(Structure):
     """``rg_mpc_env_model``: per-env mass [N], inertia [N,9] and friction coefficients [N,4] (float64 device
     pointers, each may be NULL = the workspace's value)."""
     _fields_ = [("mass", c_void_p), ("inertia", c_void_p), ("friction_coeffs", c_void_p)]
+
+
+class GaitEnvParams(Structure):
+    """``rg_gait_env_params``: per-env stance_duration, duty_factor, initial_leg_phase (float64 [N,4]) and
+    initial_leg_state (int32 [N,4]) device pointers, each may be NULL = the robot workspace's value."""
+    _fields_ = [("stance_duration", c_void_p), ("duty_factor", c_void_p), ("initial_leg_phase", c_void_p),
+                ("initial_leg_state", c_void_p)]
 
 
 class LegChain(Structure):
@@ -156,6 +163,10 @@ def load(build_if_missing: bool = False):
     lib.rg_control_step_model.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel), c_void_p]
     lib.rg_control_step_graph_create_model.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
                                                        c_void_p, POINTER(c_void_p)]
+    lib.rg_control_step_env.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
+                                        POINTER(GaitEnvParams), c_void_p]
+    lib.rg_control_step_graph_create_env.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
+                                                     POINTER(GaitEnvParams), c_void_p, POINTER(c_void_p)]
     lib.rg_hybrid_motor_torque.argtypes = [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.rg_hybrid_motor_torque_ex.argtypes = [c_void_p, c_int] + [c_void_p] * 6 + [c_void_p]
     lib.rg_measure_fma_peak.argtypes = [c_int, c_int, POINTER(c_double)]

@@ -43,12 +43,14 @@ class SyntheticStates:
 
 
 def desired_stance(time_s, stance_duration, duty_factor, init_phase, init_state):
-    """Vectorised planned-stance flags of the open-loop gait at time ``time_s`` [N] -> [N,4] bool."""
+    """Vectorised planned-stance flags of the open-loop gait at time ``time_s`` [N] -> [N,4] bool.  Each gait
+    argument is one [4] row for every env or [N,4] rows, one per env."""
+    rows = lambda a: a if a.ndim == 2 else a[None, :]
     t = np.asarray(time_s, dtype=np.float64)[:, None]
-    stance = np.asarray(stance_duration, dtype=np.float64)[None, :]
-    duty = np.asarray(duty_factor, dtype=np.float64)[None, :]
-    phase0 = np.asarray(init_phase, dtype=np.float64)[None, :]
-    init = np.asarray([int(s) for s in init_state])[None, :]
+    stance = rows(np.asarray(stance_duration, dtype=np.float64))
+    duty = rows(np.asarray(duty_factor, dtype=np.float64))
+    phase0 = rows(np.asarray(init_phase, dtype=np.float64))
+    init = np.asarray(init_state).astype(np.int64) if np.ndim(init_state) == 2 else np.asarray([int(s) for s in init_state])[None, :]
     period = stance / duty
     ph = np.fmod(t + phase0 * period, period) / period
     ratio = np.where(init == 0, 1.0 - duty, duty)
@@ -199,11 +201,17 @@ def make_off_nominal_states(n_env, family, description=None, seed=SEED):
     return st
 
 
-def make_state_sequence(n_env, n_steps, description, schedule_ctrl=None, seed=SEED, control_dt_ticks=10):
+def make_state_sequence(n_env, n_steps, description, schedule_ctrl=None, seed=SEED, control_dt_ticks=10, env_gait=None):
     """``n_steps`` consecutive control steps for ``n_env`` envs: every step draws a fresh random
     state (no physics), while the clock advances like Simulation's: t = step_counter * 0.001 with
-    ACTION_REPEAT = 10 ticks per control step (core/sim_constants.py:7,11) from a per-env start."""
+    ACTION_REPEAT = 10 ticks per control step (core/sim_constants.py:7,11) from a per-env start.
+    ``env_gait``: per-env gait rows for the planned (and so the measured) contacts, a dict with any of
+    ``stance_duration``, ``duty_factor``, ``initial_leg_phase``, ``initial_leg_state`` as [N,4] arrays (a missing
+    key takes the schedule's row); the random draws do not depend on it."""
     ctrl = schedule_ctrl or description.GetCtrlConstants()
+    g = env_gait or {}
+    gait = (g.get("stance_duration", ctrl.STANCE_DURATION_SECONDS), g.get("duty_factor", ctrl.DUTY_FACTOR),
+            g.get("initial_leg_phase", ctrl.INIT_PHASE_FULL_CYCLE), g.get("initial_leg_state", ctrl.INIT_LEG_STATE))
     rng = np.random.default_rng(seed + 1)
     start = rng.integers(0, 500, int(n_env))
     seq = []
@@ -211,8 +219,7 @@ def make_state_sequence(n_env, n_steps, description, schedule_ctrl=None, seed=SE
         st = make_states(n_env, description, schedule_ctrl=ctrl, seed=seed + 17 * (k + 1))
         tick = start + control_dt_ticks * k
         st.time_since_reset = (tick * 0.001).astype(np.float64)
-        planned = desired_stance(st.time_since_reset - start * 0.001, ctrl.STANCE_DURATION_SECONDS, ctrl.DUTY_FACTOR,
-                                 ctrl.INIT_PHASE_FULL_CYCLE, ctrl.INIT_LEG_STATE)
+        planned = desired_stance(st.time_since_reset - start * 0.001, *gait)
         flip = np.random.default_rng(seed + 31 * (k + 1)).uniform(0, 1, planned.shape) < 0.08
         st.planned_contacts = planned.astype(np.uint8)
         st.foot_contacts = np.logical_xor(planned, flip).astype(np.uint8)
