@@ -134,7 +134,8 @@ int rg_mpc_release(const void* workspace);
  *                                   yaw-aligned attitude (yaw = 0); rg_control_step zeroes it itself, a direct caller
  *                                   of this entry point (or of robot_gym.cuda.mpc_build_solve) must do so too
  *   base_rpy_rate      [N,3]  f32   Robot.GetBaseRollPitchYawRate (robot.py:205-213)
- *   foot_contact_state [N,4]  u8    1 = planned stance (held over the horizon); 4-byte aligned
+ *   foot_contact_state [N,4]  u8    1 = planned stance (held over the horizon; see rg_mpc_build_solve_schedule for
+ *                                   a per-step plan); 4-byte aligned
  *   foot_positions_base[N,12] f32   Robot.GetFootPositionsInBaseFrame (robot.py:389-397); 16-byte aligned
  *   command            [N,3]  f32   desired (vx, vy, wz) incl. per-robot offsets
  *   com_height         [N]    f32   or NULL -> EstimateCoMHeightSimple from the stance feet
@@ -210,6 +211,22 @@ typedef struct rg_mpc_env_model {
  * rg_mpc_build_solve_io (which forwards here with NULL). */
 int rg_mpc_build_solve_model(const void* workspace, int n_env, const rg_mpc_io* io_host,
                              const rg_mpc_env_model* model_host, void* stream);
+
+/* Contact schedule: the planned stance of every leg at every step of the MPC horizon (Di Carlo et al. 2018), instead of
+ * one contact row held over the whole horizon.  A [N,h,4] uint8 DEVICE array, env-major, 4-byte aligned; row k is the
+ * 4-byte planned-stance word of horizon step k in the format of foot_contact_state (nonzero = stance).
+ *  - Block (k, leg) of the QP is a stance block iff its byte is nonzero; otherwise its forces are pinned to zero, as a
+ *    swing leg's are without a schedule.
+ *  - io->foot_contact_state is not read and may be NULL.
+ *  - The com height (only when io->com_height is NULL) is the mean z of the stance feet of row 0, or of the first row
+ *    that has a stance foot when row 0 has none.  The lever arms are the feet's current positions at every step.
+ *  - An all-zero schedule gives zero forces and RG_STATUS_NO_STANCE | RG_STATUS_POLISHED, and resets the warm start.
+ *  - A schedule whose rows all equal one contact row gives bit-identical forces, solve_info and warm-start words to the
+ *    call without a schedule.
+ * rg_mpc_build_solve_schedule with contact_schedule == NULL is exactly rg_mpc_build_solve_model; model may be NULL
+ * (the workspace's body and ground).  A misaligned schedule returns RG_ERR_BAD_ARG before anything is launched. */
+int rg_mpc_build_solve_schedule(const void* workspace, int n_env, const rg_mpc_io* io_host,
+                                const rg_mpc_env_model* model_host, const uint8_t* contact_schedule, void* stream);
 
 /* ---- robot model: leg chains + gait + gains ------------------------------------------------
  * Replaces the per-robot python constants the third-party stack reads through the robot
@@ -411,6 +428,22 @@ int rg_control_step_env(const void* mpc_workspace, const void* robot_workspace, 
 int rg_control_step_graph_create_env(const void* mpc_workspace, const void* robot_workspace, int n_env,
                                      const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
                                      const rg_gait_env_params* gait_host, void* stream, void** graph_out);
+
+/* The control step with the stance solve planned over the gait's contact schedule (rg_mpc_build_solve_schedule).  The
+ * prologue writes contact_schedule_out ([N,h,4] uint8 DEVICE array, 4-byte aligned, h = the MPC workspace's horizon)
+ * and the solve reads it.  Row k is desired_leg_state == RG_LEG_STANCE of the env's OpenloopGaitGenerator (the
+ * workspace's, or the env's row of `gait`) evaluated at t_k = t + k * dt, dt the MPC workspace's planning step, with
+ * the separately rounded arithmetic of the gait update and no contact detection; row 0 therefore equals
+ * mpc_contact_state.  An env whose gait row is not valid gets all-stance rows.  contact_schedule_out == NULL is exactly
+ * rg_control_step_env / rg_control_step_graph_create_env.  A misaligned schedule returns RG_ERR_BAD_ARG before anything
+ * is launched; the graph bakes in its pointer. */
+int rg_control_step_plan(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                         const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                         const rg_gait_env_params* gait_host, uint8_t* contact_schedule_out, void* stream);
+int rg_control_step_graph_create_plan(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                                      const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                                      const rg_gait_env_params* gait_host, uint8_t* contact_schedule_out, void* stream,
+                                      void** graph_out);
 
 /* ---- "next" row (SURVEY.md 8f rank 1): batched HYBRID motor model ----------------------------
  * Replaces RobotMotorModel.convert_to_torque HYBRID branch (simple_motor.py:128-139):

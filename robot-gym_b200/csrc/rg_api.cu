@@ -290,6 +290,7 @@ extern "C" int rg_mpc_setup(const rg_mpc_params* p, void* workspace, size_t work
   info.horizon = p->horizon;
   info.queue_capacity = sc.capacity;
   info.two_kernel = (p->two_kernel_solve != 0 && h.cold_start_rounds > 0) ? 1 : 0;
+  info.dt = p->dt;
   std::lock_guard<std::mutex> lock(g_ws_mutex);
   g_ws_info[workspace] = info;
   return RG_OK;
@@ -318,15 +319,25 @@ extern "C" int rg_mpc_build_solve_io(const void* workspace, int n_env, const rg_
 
 extern "C" int rg_mpc_build_solve_model(const void* workspace, int n_env, const rg_mpc_io* io,
                                         const rg_mpc_env_model* model, void* stream) {
+  return rg_mpc_build_solve_schedule(workspace, n_env, io, model, nullptr, stream);
+}
+
+extern "C" int rg_mpc_build_solve_schedule(const void* workspace, int n_env, const rg_mpc_io* io,
+                                           const rg_mpc_env_model* model, const uint8_t* contact_schedule, void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
-  if (!workspace || !io || !io->com_velocity_body || !io->base_rpy || !io->base_rpy_rate || !io->foot_contact_state ||
-      !io->foot_positions_base || !io->command || !io->contact_forces) {
+  // with a schedule the contact row is not read (it may be NULL)
+  if (!workspace || !io || !io->com_velocity_body || !io->base_rpy || !io->base_rpy_rate ||
+      (!io->foot_contact_state && !contact_schedule) || !io->foot_positions_base || !io->command || !io->contact_forces) {
     rg_set_error("rg_mpc_build_solve: NULL argument");
     return RG_ERR_BAD_ARG;
   }
   if (n_env < 0) { rg_set_error("rg_mpc_build_solve: n_env < 0"); return RG_ERR_BAD_ARG; }
-  if (((uintptr_t)io->foot_contact_state & 3u) != 0) {   // the kernel reads the four contact flags of an env as one 32-bit word
+  if (!contact_schedule && ((uintptr_t)io->foot_contact_state & 3u) != 0) {   // the kernel reads the four contact flags of an env as one 32-bit word
     rg_set_error("rg_mpc_build_solve: foot_contact_state must be 4-byte aligned");
+    return RG_ERR_BAD_ARG;
+  }
+  if (((uintptr_t)contact_schedule & 3u) != 0) {   // ... and each row of a schedule likewise
+    rg_set_error("rg_mpc_build_solve_schedule: contact_schedule must be 4-byte aligned");
     return RG_ERR_BAD_ARG;
   }
   if (((uintptr_t)io->foot_positions_base & 15u) != 0) {  // ... and the twelve foot coordinates with three 128-bit loads
@@ -340,7 +351,7 @@ extern "C" int rg_mpc_build_solve_model(const void* workspace, int n_env, const 
   rc = rg_mpc_workspace_info(workspace, &info);
   if (rc != RG_OK) return rc;
   return rg_launch_mpc((const RgMpcDev*)workspace, info.horizon, n_env, *io, info.two_kernel && info.queue_capacity >= n_env,
-                       (cudaStream_t)stream, 0, m);
+                       (cudaStream_t)stream, 0, m, contact_schedule);
 }
 
 extern "C" int rg_mpc_build_solve(const void* workspace, int n_env, const float* com_velocity_body,

@@ -102,8 +102,10 @@ struct rg_controller_state;
 // prologue) and launches one with the programmatic attribute right after (the epilogue): the first MPC kernel is then
 // launched programmatically too.  Every MPC kernel starts with griddepcontrol.wait (a no-op after a plain launch).
 // model: a per-env model with at least one non-NULL array, or NULL (the model-free kernels).
+// plan: a [N,h,4] contact schedule (rg_mpc_build_solve_schedule) or NULL; non-NULL launches the schedule kernels, with
+// `model` or, when it is NULL, the workspace's body and ground.
 int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained = 0,
-                  const rg_mpc_env_model* model = nullptr);
+                  const rg_mpc_env_model* model = nullptr, const uint8_t* plan = nullptr);
 // NULL, or a model whose three pointers are all NULL -> NULL; RG_ERR_BAD_ARG for an array that is not 8-byte aligned
 int rg_check_env_model(const rg_mpc_env_model* model, const char* what, const rg_mpc_env_model** out);
 
@@ -124,5 +126,6 @@ inline cudaError_t rg_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
 #define RG_GRID_WAIT() asm volatile("griddepcontrol.wait;" ::: "memory")
 #define RG_GRID_LAUNCH_DEPENDENTS() asm volatile("griddepcontrol.launch_dependents;")
 // host-side record of a workspace prepared by rg_mpc_setup (no device access on the launch path)
-struct RgMpcHostInfo { int horizon; int queue_capacity; int two_kernel; };
+// dt: the planning step, which the control step's prologue needs to evaluate the gait across the horizon
+struct RgMpcHostInfo { int horizon; int queue_capacity; int two_kernel; double dt; };
 int rg_mpc_workspace_info(const void* workspace, RgMpcHostInfo* info);

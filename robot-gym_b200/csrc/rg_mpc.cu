@@ -1360,6 +1360,11 @@ __device__ __forceinline__ void env_inv3(const double* __restrict__ m, double* o
   o[8] = __dmul_rn(__dsub_rn(__dmul_rn(m[0], m[4]), __dmul_rn(m[1], m[3])), id);
 }
 
+// number of stance legs (nonzero bytes) in a 4-byte contact word
+__device__ __forceinline__ int stance_count(const unsigned w) {
+  return (int)((w & 0xffu) != 0) + (int)((w & 0xff00u) != 0) + (int)((w & 0xff0000u) != 0) + (int)((w & 0xff000000u) != 0);
+}
+
 // One env's stance QP, executed by the whole CTA.
 // LEAN = true : the verified active-set rounds only -- no interior-point state or code (the registers that frees
 //               are most of the kernel's local-memory frame).  An env whose rounds do not verify within the
@@ -1368,10 +1373,14 @@ __device__ __forceinline__ void env_inv3(const double* __restrict__ m, double* o
 // ENV_MODEL = true: mass, inertia and friction coefficients come from the env's row of `model` where its array is not
 //               NULL (rg_mpc_env_model).  A compile-time flag, so that the model-free instantiations -- whose schedule
 //               was tuned instruction by instruction (DESIGN.md 3.10-3.11) -- carry none of its code (DESIGN.md 3.12).
-template <int H, bool LEAN, bool ENV_MODEL>
+// PLAN = true : the stance of block (t, leg) comes from byte `leg` of row t of the env's contact schedule `plan`
+//               ([N,h,4], rg_mpc_build_solve_schedule) instead of one contact word held over the horizon; the com
+//               height is taken over the stance feet of row 0, or of the first row that has one (DESIGN.md 3.15).
+template <int H, bool LEAN, bool ENV_MODEL, bool PLAN = false>
 __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch,
                                           const int env, const bool skip_cold,
-                                          const rg_mpc_io& io, const rg_mpc_env_model& model) {
+                                          const rg_mpc_io& io, const rg_mpc_env_model& model,
+                                          const uint8_t* __restrict__ plan = nullptr) {
   using C = Cfg<H>;
   const float* __restrict__ g_com_vel = io.com_velocity_body;
   const float* __restrict__ g_rpy = io.base_rpy;
@@ -1400,6 +1409,12 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 #endif
   const int t_blk = tid >> 2, leg = tid & 3;
   const bool is_blk = tid < C::NB;
+#ifdef RG_DEBUG_POISON_SMEM
+  // debug builds: overwrite this CTA's shared memory with a byte pattern before the env is solved, so that a read of
+  // a value left by the previous env on the SM shows up as a result that depends on the pattern
+  for (size_t i = tid; i < sizeof(Smem<H>); i += blockDim.x) reinterpret_cast<unsigned char*>(&sm)[i] = (unsigned char)(RG_DEBUG_POISON_SMEM);
+  __syncthreads();
+#endif
 
   // the host record of this workspace may be stale (memory reused without rg_mpc_release): never index the
   // tables with the wrong horizon
@@ -1453,7 +1468,22 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 
   // ---------------------------------------------------------------- per-env inputs
   // every load is issued here, before anything depends on one of them: one DRAM latency, not four
-  const unsigned contact_word = *reinterpret_cast<const unsigned*>(g_contacts + 4 * (size_t)env);
+  // PLAN: every thread reads the env's h row words (one address across the CTA: broadcasts) for the schedule-wide
+  // quantities -- the number of stance blocks and the first non-empty row -- and its own block's row word
+  unsigned contact_word = 0u, row_word = 0u;
+  int plan_blocks = 0;
+  if constexpr (PLAN) {
+    const unsigned* __restrict__ rows = reinterpret_cast<const unsigned*>(plan + 4 * (size_t)H * env);
+#pragma unroll
+    for (int k = 0; k < H; ++k) {
+      const unsigned w = rows[k];
+      if (contact_word == 0u) contact_word = w;
+      plan_blocks += stance_count(w);
+    }
+    if (is_blk) row_word = rows[t_blk];
+  } else {
+    contact_word = *reinterpret_cast<const unsigned*>(g_contacts + 4 * (size_t)env);
+  }
   // The attitude, the feet, the rates and the command are consumed by threads of warp 0 only (setup_warp below): the
   // other warps do not load them.  The twelve foot coordinates of an env are 48 contiguous, 16-byte aligned bytes:
   // three 128-bit loads.
@@ -1483,7 +1513,9 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
   const bool stance_leg[4] = {(contact_word & 0xffu) != 0, (contact_word & 0xff00u) != 0,
                               (contact_word & 0xff0000u) != 0, (contact_word & 0xff000000u) != 0};
   const int n_stance = (int)stance_leg[0] + stance_leg[1] + stance_leg[2] + stance_leg[3];
-  const bool active_blk = is_blk && ((contact_word >> (8 * leg)) & 0xffu) != 0;
+  // stance legs of this block's own horizon step (= n_stance without a schedule)
+  const int n_step = PLAN ? stance_count(row_word) : n_stance;
+  const bool active_blk = is_blk && (((PLAN ? row_word : contact_word) >> (8 * leg)) & 0xffu) != 0;
 
   if constexpr (ENV_MODEL) {
     if (!model_ok) {     // this env's model row fails the rg_mpc_setup checks: nothing is solved
@@ -1495,7 +1527,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       return;
     }
   }
-  if (n_stance == 0) {   // every force pinned to zero by the bounds
+  if (PLAN ? plan_blocks == 0 : n_stance == 0) {   // every force pinned to zero by the bounds
     for (int i = tid; i < 12; i += blockDim.x) g_forces[12 * (size_t)env + i] = 0.f;
     if (g_hforces) for (int i = tid; i < 12 * H; i += blockDim.x) g_hforces[12 * H * (size_t)env + i] = 0.f;
     if (g_hforces64) for (int i = tid; i < 12 * H; i += blockDim.x) g_hforces64[12 * H * (size_t)env + i] = 0.0;
@@ -1734,7 +1766,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
   // (the lean instantiation declares the interior-point state with one element and never touches it)
   double u[3] = {0.0, 0.0, 0.0}, s[LEAN ? 1 : 10], lam[LEAN ? 1 : 10];
   // strictly feasible start: every stance foot carries its share of the weight
-  const double fz0 = fmin(0.5 * (fzmin + fzmax), fmax(2.0 * fzmin, ws->gravity / (inv_mass * n_stance)));
+  const double fz0 = fmin(0.5 * (fzmin + fzmax), fmax(2.0 * fzmin, ws->gravity / (inv_mass * n_step)));
   u[2] = active_blk ? fz0 : 0.0;
   double qmax = active_blk ? fmax(fabs(q[0]), fmax(fabs(q[1]), fabs(q[2]))) : 0.0;
   {
@@ -1756,7 +1788,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       lam[r] = active_blk ? RG_IPM_LAM0 * qscale / s[r] : 1.0;   // inactive threads carry harmless 1/1 pairs
     }
   }
-  const double m_total = 10.0 * H * n_stance;
+  const double m_total = PLAN ? 10.0 * plan_blocks : 10.0 * H * n_stance;
   const int max_iters = ws->max_ipm_iters;
   const int max_polish = ws->max_polish_rounds;
   double tol = ws->ipm_tol;
@@ -1963,7 +1995,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       // warm start: the verified active set of this block from the previous solve of the same env
       // (consecutive control steps see almost the same problem); wrong guesses are repaired by the rounds
       act = active_blk ? warm_act : 0u;
-    } else if (RG_COLD_GUESS_LAST && active_blk && t_blk >= H - (n_stance == 4 ? RG_COLD_GUESS_LAST_4 : RG_COLD_GUESS_LAST)) {
+    } else if (RG_COLD_GUESS_LAST && active_blk && t_blk >= H - (n_step == 4 ? RG_COLD_GUESS_LAST_4 : RG_COLD_GUESS_LAST)) {
       // a force in the last step(s) of the horizon barely moves any tracked state, so the regulariser
       // drives it to zero: fz >= fz_min is active there in practically every problem (bit 9)
       act = 1u << 9;
@@ -2347,9 +2379,10 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 }
 
 // Grid of the lean kernel and of the single-kernel path: one CTA per env (blockIdx.x = env).
-template <int H, bool LEAN, bool ENV_MODEL>
+template <int H, bool LEAN, bool ENV_MODEL, bool PLAN = false>
 __device__ __forceinline__ void solve_grid(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env,
-                                           const rg_mpc_io& io, const rg_mpc_env_model& model) {
+                                           const rg_mpc_io& io, const rg_mpc_env_model& model,
+                                           const uint8_t* __restrict__ plan = nullptr) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
   const int env = blockIdx.x;
@@ -2358,16 +2391,17 @@ __device__ __forceinline__ void solve_grid(const RgMpcDev* __restrict__ ws, RgMp
   RG_GRID_WAIT();                // launched programmatically behind the step prologue in rg_control_step; a no-op otherwise
 #endif
   if (env >= n_env) return;
-  solve_env<H, LEAN, ENV_MODEL>(sm, ws, scratch, env, false, io, model);
+  solve_env<H, LEAN, ENV_MODEL, PLAN>(sm, ws, scratch, env, false, io, model, plan);
 }
 
 // Second kernel of the two-kernel solve: the complete solver on the envs the lean kernel queued.  Persistent CTAs
 // stride over the list (it is empty for trot / walk batches: the launch then costs a few microseconds); the cold
 // start is skipped -- the lean kernel has just spent its budget on exactly those rounds.  The last CTA to finish
 // re-arms the queue counters for the next solve.
-template <int H, bool ENV_MODEL>
+template <int H, bool ENV_MODEL, bool PLAN = false>
 __device__ __forceinline__ void fallback_grid(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env,
-                                              const rg_mpc_io& io, const rg_mpc_env_model& model) {
+                                              const rg_mpc_io& io, const rg_mpc_env_model& model,
+                                              const uint8_t* __restrict__ plan = nullptr) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
 #if RG_PDL
@@ -2378,7 +2412,7 @@ __device__ __forceinline__ void fallback_grid(const RgMpcDev* __restrict__ ws, R
   for (int q = blockIdx.x; q < count; q += gridDim.x) {
     const int env = scratch->queue[q];
     if (env >= 0 && env < n_env)
-      solve_env<H, false, ENV_MODEL>(sm, ws, scratch, env, true, io, model);
+      solve_env<H, false, ENV_MODEL, PLAN>(sm, ws, scratch, env, true, io, model, plan);
     __syncthreads();   // shared memory is reused by the next env of this CTA
   }
   if (threadIdx.x == 0) {
@@ -2418,6 +2452,22 @@ __global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
 mpc_fallback_model_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
                           const rg_mpc_env_model model) {
   fallback_grid<H, true>(ws, scratch, n_env, io, model);
+}
+
+// Contact-schedule twins (rg_mpc_build_solve_schedule): always with the per-env model, whose NULL arrays stand for the
+// workspace's values, so one instantiation per (H, LEAN) serves a schedule with or without a model.
+template <int H, bool LEAN>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_solve_plan_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
+                      const rg_mpc_env_model model, const uint8_t* __restrict__ plan) {
+  solve_grid<H, LEAN, true, true>(ws, scratch, n_env, io, model, plan);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_fallback_plan_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
+                         const rg_mpc_env_model model, const uint8_t* __restrict__ plan) {
+  fallback_grid<H, true, true>(ws, scratch, n_env, io, model, plan);
 }
 
 // Dynamic shared memory above 48 KB (h = 20) and the carveout are per-device function attributes: set them once
@@ -2466,16 +2516,22 @@ int sm_count() {
 template <bool B, class A, class C>
 constexpr auto pick(A a, C c) { if constexpr (B) return c; else return a; }
 
-template <int H, bool ENV_MODEL>
+template <int H, bool ENV_MODEL, bool PLAN = false>
 int launch_kernels(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
-                   const rg_mpc_env_model& model) {
-  const auto lean_kernel = pick<ENV_MODEL>(mpc_solve_kernel<H, true>, mpc_solve_model_kernel<H, true>);
-  const auto full_kernel = pick<ENV_MODEL>(mpc_solve_kernel<H, false>, mpc_solve_model_kernel<H, false>);
-  const auto fallback_kernel = pick<ENV_MODEL>(mpc_fallback_kernel<H>, mpc_fallback_model_kernel<H>);
+                   const rg_mpc_env_model& model, const uint8_t* plan = nullptr) {
+  static_assert(!PLAN || ENV_MODEL, "the schedule kernels are instantiated with the per-env model only");
+  const auto lean_kernel = pick<PLAN>(pick<ENV_MODEL>(mpc_solve_kernel<H, true>, mpc_solve_model_kernel<H, true>),
+                                      mpc_solve_plan_kernel<H, true>);
+  const auto full_kernel = pick<PLAN>(pick<ENV_MODEL>(mpc_solve_kernel<H, false>, mpc_solve_model_kernel<H, false>),
+                                      mpc_solve_plan_kernel<H, false>);
+  const auto fallback_kernel = pick<PLAN>(pick<ENV_MODEL>(mpc_fallback_kernel<H>, mpc_fallback_model_kernel<H>),
+                                          mpc_fallback_plan_kernel<H>);
   const size_t smem = sizeof(Smem<H>);
   RgMpcScratch* scratch = (RgMpcScratch*)((char*)ws + RG_MPC_SCRATCH_OFFSET);
   auto launch = [&](auto kernel, int grid, bool programmatic) {
-    if constexpr (ENV_MODEL)
+    if constexpr (PLAN)
+      return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io, model, plan);
+    else if constexpr (ENV_MODEL)
       return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io, model);
     else
       return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io);
@@ -2508,10 +2564,13 @@ int launch_kernels(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_k
   return rc;
 }
 
-// model: NULL selects the model-free kernels
+// model: NULL selects the model-free kernels; plan: non-NULL selects the schedule kernels (NULL model = the workspace's)
 template <int H>
 int launch_h(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
-             const rg_mpc_env_model* model) {
+             const rg_mpc_env_model* model, const uint8_t* plan) {
+  if (plan)
+    return launch_kernels<H, true, true>(ws, n_env, io, two_kernel, stream, chained,
+                                         model ? *model : rg_mpc_env_model{nullptr, nullptr, nullptr}, plan);
   if (model) return launch_kernels<H, true>(ws, n_env, io, two_kernel, stream, chained, *model);
   return launch_kernels<H, false>(ws, n_env, io, two_kernel, stream, chained, rg_mpc_env_model{nullptr, nullptr, nullptr});
 }
@@ -2613,11 +2672,11 @@ extern "C" int rg_debug_riccati_solve(int horizon, const double* k1, const doubl
 }
 
 int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
-                  const rg_mpc_env_model* model) {
+                  const rg_mpc_env_model* model, const uint8_t* plan) {
   switch (horizon) {
-    case 5: return launch_h<5>(ws, n_env, io, two_kernel, stream, chained, model);
-    case 10: return launch_h<10>(ws, n_env, io, two_kernel, stream, chained, model);
-    case 20: return launch_h<20>(ws, n_env, io, two_kernel, stream, chained, model);
+    case 5: return launch_h<5>(ws, n_env, io, two_kernel, stream, chained, model, plan);
+    case 10: return launch_h<10>(ws, n_env, io, two_kernel, stream, chained, model, plan);
+    case 20: return launch_h<20>(ws, n_env, io, two_kernel, stream, chained, model, plan);
     default:
       rg_set_error("unsupported horizon %d (kernels are built for 5, 10, 20)", horizon);
       return RG_ERR_UNSUPPORTED;

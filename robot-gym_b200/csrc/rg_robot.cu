@@ -223,6 +223,24 @@ __device__ __forceinline__ void gait_leg(const RgRobotDev& R, const Gait& g, dou
   if (state == RG_LEG_STANCE && !contact) state = RG_LEG_LOSE_CONTACT;
 }
 
+// The desired state alone at time t (OpenloopGaitGenerator.update without the contact detection), in the same
+// separately rounded arithmetic as gait_leg: the contact schedule of rg_control_step_plan.
+template <class Gait>
+__device__ __forceinline__ int gait_desired(const Gait& g, double t) {
+  const double period = __ddiv_rn(g.stance(), g.duty());
+  const double aug = __dadd_rn(t, __dmul_rn(g.phase0(), period));
+  const double ph = __ddiv_rn(fmod(aug, period), period);
+  return ph < g.ratio() ? g.init() : g.next();
+}
+
+// Rows 1 .. h-1 of one leg's contact schedule: desired stance at t_k = t + k dt (row 0 is the step's own contact flag).
+// A gait row that is not valid holds the env in stance over the whole horizon.
+template <class Gait>
+__device__ __forceinline__ void plan_leg(const Gait& g, bool row_ok, double t, int h, double dt, uint8_t* __restrict__ col) {
+  for (int k = 1; k < h; ++k)
+    col[4 * k] = row_ok ? (gait_desired(g, __dadd_rn(t, __dmul_rn((double)k, dt))) == RG_LEG_STANCE) : 1;
+}
+
 __global__ void gait_kernel(const RgRobotDev* __restrict__ R, int n_env, const double* __restrict__ t,
                             const uint8_t* __restrict__ contacts, int32_t* __restrict__ desired,
                             int32_t* __restrict__ state, double* __restrict__ nphase) {
@@ -490,9 +508,11 @@ __global__ void pack_kernel(const RgRobotDev* __restrict__ R, int n_env, const i
 // kernels instantiate the bodies with WorkspaceGait and keep their own parameter list (an extra kernel parameter, even an
 // unused one, moves ptxas's register assignment: DESIGN.md §3.12), so they compile to the code they had before the
 // per-env gait existed (DESIGN.md §3.14).
-template <class Gait>
+// PLAN = true (Gait = EnvGait): the prologue also writes the env's contact schedule `plan` ([N,h,4], rg_control_step_plan).
+template <class Gait, bool PLAN = false>
 __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__ R, int n_env, const rg_controller_state& s,
-                                                  const rg_gait_env_params& gp) {
+                                                  const rg_gait_env_params& gp, uint8_t* __restrict__ plan = nullptr,
+                                                  int h = 0, double dt = 0.0) {
   RG_GRID_LAUNCH_DEPENDENTS();   // the solve kernel is launched programmatically behind this grid (rg_control_step)
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int env = (int)(idx >> 2), leg = (int)(idx & 3);
@@ -525,7 +545,8 @@ __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__
   double np;
   const Gait g = Gait::load(*R, gp, idx, leg);
   // a row is valid when its four legs are: the four lanes of the env vote (all four are past the `ok` return)
-  if (!Gait::kPerEnv || __all_sync(0xfu << lane0, g.valid())) {
+  const bool row_ok = !Gait::kPerEnv || __all_sync(0xfu << lane0, g.valid());
+  if (row_ok) {
     gait_leg(*R, g, t, s.foot_contacts[idx] != 0, d, st, np);
   } else {
     d = st = RG_LEG_STANCE;
@@ -535,6 +556,11 @@ __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__
   s.leg_state[idx] = st;
   s.normalized_phase[idx] = np;
   s.mpc_contact_state[idx] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
+  if constexpr (PLAN) {
+    uint8_t* col = plan + 4 * (size_t)h * env + leg;
+    col[0] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
+    plan_leg(g, row_ok, t, h, dt, col);
+  }
   int32_t ls = s.last_leg_state[idx];
   double tg[3];
   const bool has = swing_leg(*R, leg, g, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
@@ -556,9 +582,10 @@ __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__
 // The same prologue with one thread per env (the four legs unrolled): fewer, fatter threads -- the faster mapping for
 // large batches, where the kernel is bound by its FP64 instruction count and per-leg lanes diverge (swing legs run the IK,
 // stance legs idle).  Bit-identical results: both call the same per-leg / per-axis routines.
-template <class Gait>
+template <class Gait, bool PLAN = false>
 __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__ R, int n_env, const rg_controller_state& s,
-                                                  const rg_gait_env_params& gp) {
+                                                  const rg_gait_env_params& gp, uint8_t* __restrict__ plan = nullptr,
+                                                  int h = 0, double dt = 0.0) {
   RG_GRID_LAUNCH_DEPENDENTS();   // the solve kernel is launched programmatically behind this grid (rg_control_step)
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= n_env) return;
@@ -576,6 +603,7 @@ __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__
   bool valid = true;
   if (Gait::kPerEnv)
     for (int leg = 0; leg < 4; ++leg) valid = valid && Gait::load(*R, gp, 4 * (size_t)env + leg, leg).valid();
+  unsigned row0 = 0u;   // PLAN: the env's planned-stance word of horizon step 0
   for (int leg = 0; leg < 4; ++leg) {
     const size_t idx = 4 * (size_t)env + leg;
     int d, st;
@@ -591,6 +619,7 @@ __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__
     s.leg_state[idx] = st;
     s.normalized_phase[idx] = np;
     s.mpc_contact_state[idx] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
+    if constexpr (PLAN) row0 |= (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1u << (8 * leg) : 0u;
     int32_t ls = s.last_leg_state[idx];
     double tg[3];
     const bool has = swing_leg(*R, leg, g, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
@@ -606,6 +635,20 @@ __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__
         s.swing_joint_angles[3 * idx + j] = (float)((q[j] - R->motor_offset[m]) * R->motor_direction[m]);
       }
       s.swing_joint_valid[idx] = 1;
+    }
+  }
+  if constexpr (PLAN) {   // one 4-byte store per row: the row's four leg bytes assembled in a register
+    unsigned* rows = reinterpret_cast<unsigned*>(plan + 4 * (size_t)h * env);
+    rows[0] = row0;
+    for (int k = 1; k < h; ++k) {
+      const double tk = __dadd_rn(t, __dmul_rn((double)k, dt));
+      unsigned w = 0x01010101u;
+      if (valid) {
+        w = 0u;
+        for (int leg = 0; leg < 4; ++leg)
+          if (gait_desired(Gait::load(*R, gp, 4 * (size_t)env + leg, leg), tk) == RG_LEG_STANCE) w |= 1u << (8 * leg);
+      }
+      rows[k] = w;
     }
   }
 }
@@ -628,6 +671,17 @@ __global__ void step_prologue_gait_kernel(const RgRobotDev* __restrict__ R, int 
 __global__ void step_prologue_env_gait_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
                                               rg_gait_env_params gp) {
   step_prologue_env<EnvGait>(R, n_env, s, gp);
+}
+
+// Contact-schedule twins (rg_control_step_plan): always with EnvGait, whose NULL arrays stand for the workspace's gait.
+__global__ void step_prologue_plan_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
+                                          rg_gait_env_params gp, uint8_t* __restrict__ plan, int h, double dt) {
+  step_prologue_leg<EnvGait, true>(R, n_env, s, gp, plan, h, dt);
+}
+
+__global__ void step_prologue_env_plan_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
+                                              rg_gait_env_params gp, uint8_t* __restrict__ plan, int h, double dt) {
+  step_prologue_env<EnvGait, true>(R, n_env, s, gp, plan, h, dt);
 }
 
 __global__ void step_epilogue_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
@@ -956,6 +1010,12 @@ static int rg_check_env_gait(const rg_gait_env_params* gait, const char* what, c
 
 extern "C" int rg_control_step_env(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                    const rg_mpc_env_model* model, const rg_gait_env_params* gait, void* stream) {
+  return rg_control_step_plan(mpc_ws, robot_ws, n_env, s, model, gait, nullptr, stream);
+}
+
+extern "C" int rg_control_step_plan(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                    const rg_mpc_env_model* model, const rg_gait_env_params* gait, uint8_t* plan,
+                                    void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
   RG_REQUIRE(mpc_ws && robot_ws && s && n_env >= 0, "rg_control_step");
   RG_REQUIRE(s->time_since_reset && s->foot_contacts && s->base_velocity_world && s->base_orientation_xyzw && s->base_rpy &&
@@ -973,9 +1033,22 @@ extern "C" int rg_control_step_env(const void* mpc_ws, const void* robot_ws, int
   const rg_gait_env_params* g = nullptr;
   rc = rg_check_env_gait(gait, "rg_control_step_env", &g);
   if (rc != RG_OK) return rc;
+  if ((uintptr_t)plan & 3u) {
+    rg_set_error("rg_control_step_plan: contact_schedule_out must be 4-byte aligned");
+    return RG_ERR_BAD_ARG;
+  }
   cudaStream_t st = (cudaStream_t)stream;
   const RgRobotDev* R = (const RgRobotDev*)robot_ws;
-  if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS) {
+  RgMpcHostInfo info;
+  if (plan) {   // the prologue needs the horizon and dt: look the workspace up before the first launch
+    rc = rg_mpc_workspace_info(mpc_ws, &info);
+    if (rc != RG_OK) return rc;
+    const rg_gait_env_params gp = g ? *g : rg_gait_env_params{nullptr, nullptr, nullptr, nullptr};
+    if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS)
+      step_prologue_plan_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, info.horizon, info.dt);
+    else
+      step_prologue_env_plan_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, info.horizon, info.dt);
+  } else if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS) {
     if (g) step_prologue_gait_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, *g);
     else step_prologue_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s);
   } else {
@@ -985,9 +1058,10 @@ extern "C" int rg_control_step_env(const void* mpc_ws, const void* robot_ws, int
   rg_count_launch();
   rc = rg_check_cuda(cudaGetLastError(), "step_prologue_kernel launch");
   if (rc != RG_OK) return rc;
-  RgMpcHostInfo info;
-  rc = rg_mpc_workspace_info(mpc_ws, &info);
-  if (rc != RG_OK) return rc;
+  if (!plan) {
+    rc = rg_mpc_workspace_info(mpc_ws, &info);
+    if (rc != RG_OK) return rc;
+  }
   // TorqueStanceLegController.get_action zeroes the yaw before the solve ("yaw aligned world frame")
   rg_mpc_io io;
   memset(&io, 0, sizeof(io));
@@ -1003,7 +1077,7 @@ extern "C" int rg_control_step_env(const void* mpc_ws, const void* robot_ws, int
   io.zero_yaw = 1;
   // prologue -> solve kernel(s) -> epilogue are chained by programmatic dependent launches: each grid becomes resident
   // while its predecessor drains and waits (griddepcontrol.wait) for it to complete, so the launch latencies overlap
-  rc = rg_launch_mpc((const RgMpcDev*)mpc_ws, info.horizon, n_env, io, info.two_kernel && info.queue_capacity >= n_env, st, 1, m);
+  rc = rg_launch_mpc((const RgMpcDev*)mpc_ws, info.horizon, n_env, io, info.two_kernel && info.queue_capacity >= n_env, st, 1, m, plan);
   if (rc != RG_OK) return rc;
   rc = rg_check_cuda(rg_launch(step_epilogue_kernel, dim3((unsigned)grid_for(4 * n_env, 256)), dim3(256), 0, st, true,
                                (const RgRobotDev*)robot_ws, n_env, *s), "step_epilogue_kernel launch");
@@ -1034,12 +1108,18 @@ extern "C" int rg_control_step_graph_create_model(const void* mpc_ws, const void
 extern "C" int rg_control_step_graph_create_env(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                                 const rg_mpc_env_model* model, const rg_gait_env_params* gait, void* stream,
                                                 void** graph_out) {
+  return rg_control_step_graph_create_plan(mpc_ws, robot_ws, n_env, s, model, gait, nullptr, stream, graph_out);
+}
+
+extern "C" int rg_control_step_graph_create_plan(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                                 const rg_mpc_env_model* model, const rg_gait_env_params* gait, uint8_t* plan,
+                                                 void* stream, void** graph_out) {
   RG_REQUIRE(mpc_ws && robot_ws && s && graph_out && n_env > 0, "rg_control_step_graph_create");
   *graph_out = nullptr;
   // one eager step on the caller's stream first: kernel attributes get configured outside the capture, and argument
   // errors surface here with their own message.  The controller state advances by this step -- the caller accounts for it
   // by creating the graph INSTEAD of a step, not before one (see rg_cuda.h).
-  int rc = rg_control_step_env(mpc_ws, robot_ws, n_env, s, model, gait, stream);
+  int rc = rg_control_step_plan(mpc_ws, robot_ws, n_env, s, model, gait, plan, stream);
   if (rc == RG_OK) rc = rg_check_cuda(cudaStreamSynchronize((cudaStream_t)stream), "graph warm-up step");
   if (rc != RG_OK) return rc;
   cudaStream_t cap = nullptr;
@@ -1049,7 +1129,7 @@ extern "C" int rg_control_step_graph_create_env(const void* mpc_ws, const void* 
   RgStepGraph* g = new RgStepGraph{nullptr, nullptr, 0};
   cudaError_t e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal);
   if (e == cudaSuccess) {
-    rc = rg_control_step_env(mpc_ws, robot_ws, n_env, s, model, gait, cap);
+    rc = rg_control_step_plan(mpc_ws, robot_ws, n_env, s, model, gait, plan, cap);
     e = cudaStreamEndCapture(cap, &g->graph);
     if (rc != RG_OK) e = cudaErrorUnknown;
   }

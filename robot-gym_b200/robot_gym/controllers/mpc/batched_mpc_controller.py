@@ -65,12 +65,15 @@ class BatchedMPCController(Controller):
     GRAPH_MAX_ENVS = 2048          # below this a control step is launch-bound: replay it as one CUDA graph
 
     def __init__(self, robot, get_time_since_reset, horizon=10, mpc_overrides=None, squeeze_single=True,
-                 warm_start=True, use_graph=None):
+                 warm_start=True, use_graph=None, contact_plan=False):
         """``robot``: batched state provider with the getter names of robot.py (see
         ``SyntheticRobotBatch``); ``get_time_since_reset``: callable returning a float or an
         ``[N]`` float64 tensor (Simulation.GetTimeSinceReset, core/simulation.py:141-142).
         ``warm_start``: seed each stance QP with the active set the same env verified one control step
-        earlier (``rg_mpc_build_solve_warm``); the optimum is unique, so the forces do not depend on it."""
+        earlier (``rg_mpc_build_solve_warm``); the optimum is unique, so the forces do not depend on it.
+        ``contact_plan``: plan the stance QP over each env's gait schedule -- the desired stance of every leg at every
+        horizon step (``rg_control_step_plan``) -- instead of holding the current contact row over the horizon.  The
+        schedule the step solved against is ``mpc_contact_schedule`` ([N, horizon, 4] uint8, row 0 = ``mpc_contact_state``)."""
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedMPCController needs a CUDA device (no CPU fallback)")
         rg.load()
@@ -137,6 +140,7 @@ class BatchedMPCController(Controller):
         self.motor_torques = z((n, 12), f32)
         self.solve_info = z((n, 4), i32)
         self.mpc_active_set = rg.new_active_set(n, self.horizon, dev) if warm_start else None
+        self.mpc_contact_schedule = z((n, self.horizon, 4), u8) if contact_plan else None
         self.action = z((n, 60), f32)
         self.reset_time = z((n,), f64)
         self.time_since_reset = z((n,), f64)
@@ -334,7 +338,12 @@ class BatchedMPCController(Controller):
                 if self._graph is None:
                     # creating the graph executes this step eagerly (and synchronises once)
                     handle = ctypes.c_void_p()
-                    if self._env_model is None and self._env_gait is None:
+                    if self.mpc_contact_schedule is not None:
+                        rg.check(lib.rg_control_step_graph_create_plan(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
+                                                                       ctypes.byref(self._state), self._env_model_ref(),
+                                                                       self._env_gait_ref(), self._schedule_ptr(),
+                                                                       rg.current_stream_ptr(), ctypes.byref(handle)))
+                    elif self._env_model is None and self._env_gait is None:
                         rg.check(lib.rg_control_step_graph_create(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
                                                                   ctypes.byref(self._state), rg.current_stream_ptr(),
                                                                   ctypes.byref(handle)))
@@ -349,12 +358,19 @@ class BatchedMPCController(Controller):
         return self.action
 
     def _eager_step(self, lib):
-        if self._env_model is None and self._env_gait is None:
+        if self.mpc_contact_schedule is not None:
+            rg.check(lib.rg_control_step_plan(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
+                                              self._env_model_ref(), self._env_gait_ref(), self._schedule_ptr(),
+                                              rg.current_stream_ptr()))
+        elif self._env_model is None and self._env_gait is None:
             rg.check(lib.rg_control_step(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
                                          ctypes.byref(self._state), rg.current_stream_ptr()))
         else:
             rg.check(lib.rg_control_step_env(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
                                              self._env_model_ref(), self._env_gait_ref(), rg.current_stream_ptr()))
+
+    def _schedule_ptr(self):
+        return rg._ptr(self.mpc_contact_schedule, torch.uint8, (self.horizon, 4), n=self.num_envs, device=self.device, align=4)
 
     def _env_model_ref(self):
         return None if self._env_model is None else ctypes.byref(self._env_model)

@@ -33,6 +33,7 @@ EXPORTED_SYMBOLS = (
     "rg_gait_step", "rg_com_velocity_update", "rg_swing_targets", "rg_leg_ik", "rg_leg_fk", "rg_state_from_sim",
     "rg_force_to_torque", "rg_pack_hybrid_action", "rg_control_step", "rg_control_step_graph_create", "rg_control_step_graph_launch", "rg_control_step_graph_destroy",
     "rg_control_step_model", "rg_control_step_graph_create_model", "rg_control_step_env", "rg_control_step_graph_create_env",
+    "rg_mpc_build_solve_schedule", "rg_control_step_plan", "rg_control_step_graph_create_plan",
     "rg_hybrid_motor_torque", "rg_hybrid_motor_torque_ex",
     "rg_measure_fma_peak", "rg_launch_count", "rg_last_error", "rg_version",
 )
@@ -167,6 +168,11 @@ def load(build_if_missing: bool = False):
                                         POINTER(GaitEnvParams), c_void_p]
     lib.rg_control_step_graph_create_env.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
                                                      POINTER(GaitEnvParams), c_void_p, POINTER(c_void_p)]
+    lib.rg_mpc_build_solve_schedule.argtypes = [c_void_p, c_int, POINTER(MpcIo), POINTER(MpcEnvModel), c_void_p, c_void_p]
+    lib.rg_control_step_plan.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
+                                         POINTER(GaitEnvParams), c_void_p, c_void_p]
+    lib.rg_control_step_graph_create_plan.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
+                                                      POINTER(GaitEnvParams), c_void_p, c_void_p, POINTER(c_void_p)]
     lib.rg_hybrid_motor_torque.argtypes = [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.rg_hybrid_motor_torque_ex.argtypes = [c_void_p, c_int] + [c_void_p] * 6 + [c_void_p]
     lib.rg_measure_fma_peak.argtypes = [c_int, c_int, POINTER(c_double)]
@@ -293,7 +299,7 @@ def calibrate_ik(params: RobotParams, reference_motor_angles) -> None:
 def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate, foot_contact_state,
                     foot_positions_base, command, com_height=None, contact_forces=None,
                     horizon_forces=None, solve_info=None, want_horizon=False, want_info=True, active_set=None,
-                    zero_yaw=False, horizon_forces_f64=None, env_model=None):
+                    zero_yaw=False, horizon_forces_f64=None, env_model=None, contact_schedule=None):
     """``rg_mpc_build_solve`` (``rg_mpc_build_solve_warm`` when ``active_set`` -- an ``[N, 4*horizon]`` int16 tensor
     initialised to -1, see ``new_active_set`` -- is given) on the current stream.  ``base_rpy`` is used as given:
     pass a yaw-aligned attitude (yaw = 0) to reproduce TorqueStanceLegController (the controller's fused step
@@ -301,7 +307,9 @@ def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate
     unrounded solution; goes through ``rg_mpc_build_solve_io``).  ``env_model``: per-env body and ground for this
     solve (``rg_mpc_build_solve_model``), a dict or an object with ``mass`` [N], ``inertia`` [N,9] or [N,3,3] and
     ``friction_coeffs`` [N,4] float64 CUDA tensors, any of them None (= the workspace's value); an env whose row fails
-    the workspace checks gets zero forces and RG_STATUS_BAD_MODEL.  Returns (contact_forces, horizon_forces, solve_info)."""
+    the workspace checks gets zero forces and RG_STATUS_BAD_MODEL.  ``contact_schedule``: the planned stance of every
+    leg at every horizon step, an ``[N,h,4]`` uint8 or bool CUDA tensor (nonzero = stance; ``rg_mpc_build_solve_schedule``);
+    ``foot_contact_state`` is then not read and may be None.  Returns (contact_forces, horizon_forces, solve_info)."""
     import torch
     n = base_rpy.shape[0]
     dev = base_rpy.device
@@ -317,19 +325,29 @@ def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate
     hf = None if horizon_forces is None else P(horizon_forces.view(n, ws.horizon * 12), torch.float32, (ws.horizon * 12,))
     args = (ws.ptr, n,
             P(com_velocity_body, torch.float32, (3,)), P(base_rpy, torch.float32, (3,)),
-            P(base_rpy_rate, torch.float32, (3,)), P(foot_contact_state, torch.uint8, (4,), align=4),
+            P(base_rpy_rate, torch.float32, (3,)),
+            P(foot_contact_state, torch.uint8, (4,), align=4, allow_none=contact_schedule is not None),
             P(foot_positions_base.view(n, 12), torch.float32, (12,), align=16), P(command, torch.float32, (3,)),
             P(com_height, torch.float32, (), allow_none=True),
             P(contact_forces, torch.float32, (12,)), hf,
             P(solve_info, torch.int32, (4,), allow_none=True))
     model = None if env_model is None else env_model_struct(env_model, n, dev)
+    schedule = None
+    if contact_schedule is not None:
+        if isinstance(contact_schedule, torch.Tensor) and contact_schedule.dtype == torch.bool:
+            contact_schedule = contact_schedule.view(torch.uint8)
+        schedule = P(contact_schedule, torch.uint8, (ws.horizon, 4), align=4)
     with torch.cuda.device(dev):
-        if zero_yaw or horizon_forces_f64 is not None or model is not None:
+        if zero_yaw or horizon_forces_f64 is not None or model is not None or schedule is not None:
             io = MpcIo(*[a if a is None or isinstance(a, int) else a.value for a in args[2:]],
                        None if active_set is None else P(active_set, torch.int16, (4 * ws.horizon,)).value,
                        None if horizon_forces_f64 is None else P(horizon_forces_f64.view(n, ws.horizon * 12), torch.float64, (ws.horizon * 12,)).value,
                        1 if zero_yaw else 0, 0)
-            if model is None:
+            if schedule is not None:
+                check(load().rg_mpc_build_solve_schedule(ws.ptr, n, ctypes.byref(io),
+                                                         None if model is None else ctypes.byref(model), schedule,
+                                                         current_stream_ptr()))
+            elif model is None:
                 check(load().rg_mpc_build_solve_io(ws.ptr, n, ctypes.byref(io), current_stream_ptr()))
             else:
                 check(load().rg_mpc_build_solve_model(ws.ptr, n, ctypes.byref(io), ctypes.byref(model), current_stream_ptr()))

@@ -58,6 +58,16 @@ def desired_stance(time_s, stance_duration, duty_factor, init_phase, init_state)
     return np.where(in_init, init == 1, init != 1)
 
 
+def planned_contact_schedule(time_s, dt, horizon, stance_duration, duty_factor, init_phase, init_state):
+    """Contact schedule of the open-loop gait over an MPC horizon: ``[N, horizon, 4]`` uint8, row k the planned stance
+    at ``t + k * dt`` (each product and sum rounded separately, as the control step's prologue evaluates it).  The
+    gait arguments are as for ``desired_stance``."""
+    t = np.asarray(time_s, dtype=np.float64)
+    rows = [desired_stance(t + float(k) * float(dt), stance_duration, duty_factor, init_phase, init_state)
+            for k in range(int(horizon))]
+    return np.stack(rows, axis=1).astype(np.uint8)
+
+
 def euler_to_quat_xyzw(rpy):
     r, p, y = rpy[:, 0] * 0.5, rpy[:, 1] * 0.5, rpy[:, 2] * 0.5
     cr, sr, cp, sp, cy, sy = np.cos(r), np.sin(r), np.cos(p), np.sin(p), np.cos(y), np.sin(y)
