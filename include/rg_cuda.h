@@ -219,7 +219,8 @@ int rg_mpc_build_solve_model(const void* workspace, int n_env, const rg_mpc_io* 
  *    swing leg's are without a schedule.
  *  - io->foot_contact_state is not read and may be NULL.
  *  - The com height (only when io->com_height is NULL) is the mean z of the stance feet of row 0, or of the first row
- *    that has a stance foot when row 0 has none.  The lever arms are the feet's current positions at every step.
+ *    that has a stance foot when row 0 has none.  The lever arms are the feet's current positions at every step (see
+ *    rg_mpc_build_solve_footholds for per-step footholds).
  *  - An all-zero schedule gives zero forces and RG_STATUS_NO_STANCE | RG_STATUS_POLISHED, and resets the warm start.
  *  - A schedule whose rows all equal one contact row gives bit-identical forces, solve_info and warm-start words to the
  *    call without a schedule.
@@ -227,6 +228,25 @@ int rg_mpc_build_solve_model(const void* workspace, int n_env, const rg_mpc_io* 
  * (the workspace's body and ground).  A misaligned schedule returns RG_ERR_BAD_ARG before anything is launched. */
 int rg_mpc_build_solve_schedule(const void* workspace, int n_env, const rg_mpc_io* io_host,
                                 const rg_mpc_env_model* model_host, const uint8_t* contact_schedule, void* stream);
+
+/* Foothold plan: the position of every foot at every step of the MPC horizon, so that the QP's lever arms follow the
+ * feet through the plan (Di Carlo et al. 2018: one B per step from the predicted footholds) instead of holding the
+ * current feet.  A [N,h,12] float32 DEVICE array, env-major, 16-byte aligned; row k holds the four feet (FR, FL, RR, RL;
+ * x, y, z) at horizon step k, in the frame and convention of foot_positions_base (the base frame of the current step,
+ * rotated by the solve's Rx Ry Rz of the yaw-zeroed attitude, as the current feet are).
+ *  - Block (k, leg) takes row k's foot `leg` as its lever arm.  Entries of swing blocks (schedule byte 0) are not read:
+ *    any value there, NaN included, changes nothing.
+ *  - io->foot_positions_base is not read and may be NULL.  The com height (only when io->com_height is NULL) is the mean
+ *    z of the stance feet of row r* of the plan, r* being the schedule row rg_mpc_build_solve_schedule takes it from
+ *    (row 0, or the first row with a stance foot).
+ *  - A plan whose rows all equal foot_positions_base gives bit-identical forces, solve_info and warm-start words to
+ *    rg_mpc_build_solve_schedule.
+ * A plan requires a contact schedule.  rg_mpc_build_solve_footholds with foothold_plan == NULL is exactly
+ * rg_mpc_build_solve_schedule; a non-NULL plan with a NULL schedule, or a misaligned plan, returns RG_ERR_BAD_ARG before
+ * anything is launched. */
+int rg_mpc_build_solve_footholds(const void* workspace, int n_env, const rg_mpc_io* io_host,
+                                 const rg_mpc_env_model* model_host, const uint8_t* contact_schedule,
+                                 const float* foothold_plan, void* stream);
 
 /* ---- robot model: leg chains + gait + gains ------------------------------------------------
  * Replaces the per-robot python constants the third-party stack reads through the robot
@@ -444,6 +464,30 @@ int rg_control_step_graph_create_plan(const void* mpc_workspace, const void* rob
                                       const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
                                       const rg_gait_env_params* gait_host, uint8_t* contact_schedule_out, void* stream,
                                       void** graph_out);
+
+/* The planned control step with predicted footholds (rg_mpc_build_solve_footholds).  The prologue writes
+ * foothold_plan_out ([N,h,12] float32 DEVICE array, 16-byte aligned) next to contact_schedule_out, and the solve reads
+ * both.  Per leg, with p its current foot (foot_positions_base) and v = (command[0], command[1], 0), in double and
+ * stored as float32:
+ *     anchor = p, k_a = 0
+ *     for k in 0 .. h-1:
+ *         if k >= 1 and schedule[k] is stance and schedule[k-1] is swing:   touchdown inside the horizon
+ *             anchor = the Raibert foothold of the swing controller, k_a = k
+ *         foothold[k] = anchor - (k - k_a) * dt * v                          the body walks over a planted foot
+ * The Raibert foothold is exactly the end point of the leg's swing trajectory (the float32-rounded velocity estimate, yaw
+ * rate, command, the env's stance duration, the hip offset and desired_height - foot_clearance).  The yaw rate is not
+ * integrated into the footholds, as the QP's model holds the yaw in B.  An env whose gait row is not valid gets held
+ * rows (foothold[k] = p).  foothold_plan_out == NULL is exactly rg_control_step_plan /
+ * rg_control_step_graph_create_plan; a non-NULL plan with a NULL contact_schedule_out, or a misaligned plan, returns
+ * RG_ERR_BAD_ARG before anything is launched; the graph bakes in its pointer. */
+int rg_control_step_footholds(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                              const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                              const rg_gait_env_params* gait_host, uint8_t* contact_schedule_out,
+                              float* foothold_plan_out, void* stream);
+int rg_control_step_graph_create_footholds(const void* mpc_workspace, const void* robot_workspace, int n_env,
+                                           const rg_controller_state* s_host, const rg_mpc_env_model* model_host,
+                                           const rg_gait_env_params* gait_host, uint8_t* contact_schedule_out,
+                                           float* foothold_plan_out, void* stream, void** graph_out);
 
 /* ---- "next" row (SURVEY.md 8f rank 1): batched HYBRID motor model ----------------------------
  * Replaces RobotMotorModel.convert_to_torque HYBRID branch (simple_motor.py:128-139):

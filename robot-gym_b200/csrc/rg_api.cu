@@ -324,10 +324,21 @@ extern "C" int rg_mpc_build_solve_model(const void* workspace, int n_env, const 
 
 extern "C" int rg_mpc_build_solve_schedule(const void* workspace, int n_env, const rg_mpc_io* io,
                                            const rg_mpc_env_model* model, const uint8_t* contact_schedule, void* stream) {
+  return rg_mpc_build_solve_footholds(workspace, n_env, io, model, contact_schedule, nullptr, stream);
+}
+
+extern "C" int rg_mpc_build_solve_footholds(const void* workspace, int n_env, const rg_mpc_io* io,
+                                            const rg_mpc_env_model* model, const uint8_t* contact_schedule,
+                                            const float* foothold_plan, void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
-  // with a schedule the contact row is not read (it may be NULL)
+  if (foothold_plan && !contact_schedule) {
+    rg_set_error("rg_mpc_build_solve_footholds: a foothold plan needs a contact schedule");
+    return RG_ERR_BAD_ARG;
+  }
+  // with a schedule the contact row is not read (it may be NULL), with a foothold plan the current feet are not
   if (!workspace || !io || !io->com_velocity_body || !io->base_rpy || !io->base_rpy_rate ||
-      (!io->foot_contact_state && !contact_schedule) || !io->foot_positions_base || !io->command || !io->contact_forces) {
+      (!io->foot_contact_state && !contact_schedule) || (!io->foot_positions_base && !foothold_plan) || !io->command ||
+      !io->contact_forces) {
     rg_set_error("rg_mpc_build_solve: NULL argument");
     return RG_ERR_BAD_ARG;
   }
@@ -340,8 +351,12 @@ extern "C" int rg_mpc_build_solve_schedule(const void* workspace, int n_env, con
     rg_set_error("rg_mpc_build_solve_schedule: contact_schedule must be 4-byte aligned");
     return RG_ERR_BAD_ARG;
   }
-  if (((uintptr_t)io->foot_positions_base & 15u) != 0) {  // ... and the twelve foot coordinates with three 128-bit loads
+  if (!foothold_plan && ((uintptr_t)io->foot_positions_base & 15u) != 0) {  // ... and the twelve foot coordinates with three 128-bit loads
     rg_set_error("rg_mpc_build_solve: foot_positions_base must be 16-byte aligned");
+    return RG_ERR_BAD_ARG;
+  }
+  if (((uintptr_t)foothold_plan & 15u) != 0) {   // ... and each row of a foothold plan likewise
+    rg_set_error("rg_mpc_build_solve_footholds: foothold_plan must be 16-byte aligned");
     return RG_ERR_BAD_ARG;
   }
   const rg_mpc_env_model* m = nullptr;
@@ -351,7 +366,7 @@ extern "C" int rg_mpc_build_solve_schedule(const void* workspace, int n_env, con
   rc = rg_mpc_workspace_info(workspace, &info);
   if (rc != RG_OK) return rc;
   return rg_launch_mpc((const RgMpcDev*)workspace, info.horizon, n_env, *io, info.two_kernel && info.queue_capacity >= n_env,
-                       (cudaStream_t)stream, 0, m, contact_schedule);
+                       (cudaStream_t)stream, 0, m, contact_schedule, foothold_plan);
 }
 
 extern "C" int rg_mpc_build_solve(const void* workspace, int n_env, const float* com_velocity_body,

@@ -104,8 +104,10 @@ struct rg_controller_state;
 // model: a per-env model with at least one non-NULL array, or NULL (the model-free kernels).
 // plan: a [N,h,4] contact schedule (rg_mpc_build_solve_schedule) or NULL; non-NULL launches the schedule kernels, with
 // `model` or, when it is NULL, the workspace's body and ground.
+// feet: a [N,h,12] foothold plan (rg_mpc_build_solve_footholds) or NULL; non-NULL (with a plan) launches the foothold
+// kernels.
 int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained = 0,
-                  const rg_mpc_env_model* model = nullptr, const uint8_t* plan = nullptr);
+                  const rg_mpc_env_model* model = nullptr, const uint8_t* plan = nullptr, const float* feet = nullptr);
 // NULL, or a model whose three pointers are all NULL -> NULL; RG_ERR_BAD_ARG for an array that is not 8-byte aligned
 int rg_check_env_model(const rg_mpc_env_model* model, const char* what, const rg_mpc_env_model** out);
 

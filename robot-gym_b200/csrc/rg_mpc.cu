@@ -1376,11 +1376,15 @@ __device__ __forceinline__ int stance_count(const unsigned w) {
 // PLAN = true : the stance of block (t, leg) comes from byte `leg` of row t of the env's contact schedule `plan`
 //               ([N,h,4], rg_mpc_build_solve_schedule) instead of one contact word held over the horizon; the com
 //               height is taken over the stance feet of row 0, or of the first row that has one (DESIGN.md 3.15).
-template <int H, bool LEAN, bool ENV_MODEL, bool PLAN = false>
+// FEET = true (with PLAN): the lever arm of block (t, leg) is foot `leg` of row t of the env's foothold plan `feet`
+//               ([N,h,12], rg_mpc_build_solve_footholds) instead of the current foot at every step, and the com height
+//               is taken over the stance feet of the same row r* the schedule names (DESIGN.md 3.16).
+template <int H, bool LEAN, bool ENV_MODEL, bool PLAN = false, bool FEET = false>
 __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch,
                                           const int env, const bool skip_cold,
                                           const rg_mpc_io& io, const rg_mpc_env_model& model,
-                                          const uint8_t* __restrict__ plan = nullptr) {
+                                          const uint8_t* __restrict__ plan = nullptr,
+                                          const float* __restrict__ feet = nullptr) {
   using C = Cfg<H>;
   const float* __restrict__ g_com_vel = io.com_velocity_body;
   const float* __restrict__ g_rpy = io.base_rpy;
@@ -1471,13 +1475,16 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
   // PLAN: every thread reads the env's h row words (one address across the CTA: broadcasts) for the schedule-wide
   // quantities -- the number of stance blocks and the first non-empty row -- and its own block's row word
   unsigned contact_word = 0u, row_word = 0u;
-  int plan_blocks = 0;
+  int plan_blocks = 0, r_star = 0;   // FEET: r_star = the row contact_word comes from
   if constexpr (PLAN) {
     const unsigned* __restrict__ rows = reinterpret_cast<const unsigned*>(plan + 4 * (size_t)H * env);
 #pragma unroll
     for (int k = 0; k < H; ++k) {
       const unsigned w = rows[k];
-      if (contact_word == 0u) contact_word = w;
+      if (contact_word == 0u) {
+        contact_word = w;
+        if constexpr (FEET) r_star = k;
+      }
       plan_blocks += stance_count(w);
     }
     if (is_blk) row_word = rows[t_blk];
@@ -1490,10 +1497,24 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
   float in_roll = 0.f, in_pitch = 0.f, in_yaw = 0.f, in_com_h = 0.f;
   float in_feet[12] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   float in_w[3] = {0.f, 0.f, 0.f}, in_v[3] = {0.f, 0.f, 0.f}, in_cmd[3] = {0.f, 0.f, 0.f};
+  // FEET: every block thread loads its own foot of its own row, consumed by itself alone (per-block constants below);
+  // the entries of swing blocks are loaded but never used
+  float blk_foot[3] = {0.f, 0.f, 0.f};
+  if constexpr (FEET) {
+    if (is_blk) {
+      const float* __restrict__ bf = feet + 12 * ((size_t)H * env + t_blk) + 3 * leg;
+      blk_foot[0] = bf[0]; blk_foot[1] = bf[1]; blk_foot[2] = bf[2];
+    }
+  }
   if (tid < 32) {
     in_roll = g_rpy[3 * (size_t)env + 0]; in_pitch = g_rpy[3 * (size_t)env + 1]; in_yaw = g_rpy[3 * (size_t)env + 2];
-    const float4* __restrict__ f4 = reinterpret_cast<const float4*>(g_feet + 12 * (size_t)env);
-    const float4 fa = f4[0], fb = f4[1], fc = f4[2];
+    // FEET: the feet of row 0 of the plan, issued with the other loads; reloaded from row r* when the schedule's first
+    // stance row is a later one (their only use is the com height)
+    const float4* __restrict__ f4 = reinterpret_cast<const float4*>(FEET ? feet + 12 * (size_t)H * env : g_feet + 12 * (size_t)env);
+    float4 fa = f4[0], fb = f4[1], fc = f4[2];
+    if constexpr (FEET) {
+      if (r_star != 0) { fa = f4[3 * r_star]; fb = f4[3 * r_star + 1]; fc = f4[3 * r_star + 2]; }
+    }
     in_feet[0] = fa.x; in_feet[1] = fa.y; in_feet[2] = fa.z; in_feet[3] = fa.w;
     in_feet[4] = fb.x; in_feet[5] = fb.y; in_feet[6] = fb.z; in_feet[7] = fb.w;
     in_feet[8] = fc.x; in_feet[9] = fc.y; in_feet[10] = fc.z; in_feet[11] = fc.w;
@@ -1608,7 +1629,9 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       if (stance_leg[l]) zsum += fw[l][2];
     }
     com_z = g_com_height ? (double)in_com_h : fabs(zsum / n_stance);
-    if (tid < 4) {
+    // FEET: thread 0 publishes rf and I_w^-1 (18 doubles, in the storage of sm.bang) for the block threads, which form
+    // their own lever-arm products after the barrier below
+    if (tid < (FEET ? 1 : 4)) {
       const double rb[9] = {cy * cp, cy * sp * sr - sy * cr, cy * sp * cr + sy * sr,
                             sy * cp, sy * sp * sr + cy * cr, sy * sp * cr - cy * sr,
                             -sp, cp * sr, cp * cr};
@@ -1641,20 +1664,26 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
           for (int c = 0; c < 3; ++c) v += tmp[3 * a + c] * rb[3 * b + c];
           iw[3 * a + b] = v;
         }
-      // own leg's lever arm by selects: a run-time index into fw[][] would put it (and in_feet[]) into a local-memory frame
-      const double rx = tid == 0 ? fw[0][0] : (tid == 1 ? fw[1][0] : (tid == 2 ? fw[2][0] : fw[3][0]));
-      const double ry = tid == 0 ? fw[0][1] : (tid == 1 ? fw[1][1] : (tid == 2 ? fw[2][1] : fw[3][1]));
-      const double rz = tid == 0 ? fw[0][2] : (tid == 1 ? fw[1][2] : (tid == 2 ? fw[2][2] : fw[3][2]));
-      const double sk[9] = {0.0, -rz, ry, rz, 0.0, -rx, -ry, rx, 0.0};
+      if constexpr (FEET) {
+        double* __restrict__ pub = &sm.bang[0][0];
 #pragma unroll
-      for (int a = 0; a < 3; ++a)
+        for (int i = 0; i < 9; ++i) { pub[i] = rf[i]; pub[9 + i] = iw[i]; }
+      } else {
+        // own leg's lever arm by selects: a run-time index into fw[][] would put it (and in_feet[]) into a local-memory frame
+        const double rx = tid == 0 ? fw[0][0] : (tid == 1 ? fw[1][0] : (tid == 2 ? fw[2][0] : fw[3][0]));
+        const double ry = tid == 0 ? fw[0][1] : (tid == 1 ? fw[1][1] : (tid == 2 ? fw[2][1] : fw[3][1]));
+        const double rz = tid == 0 ? fw[0][2] : (tid == 1 ? fw[1][2] : (tid == 2 ? fw[2][2] : fw[3][2]));
+        const double sk[9] = {0.0, -rz, ry, rz, 0.0, -rx, -ry, rx, 0.0};
 #pragma unroll
-        for (int b = 0; b < 3; ++b) {
-          double v = 0.0;
+        for (int a = 0; a < 3; ++a)
 #pragma unroll
-          for (int c = 0; c < 3; ++c) v += iw[3 * a + c] * sk[3 * c + b];
-          sm.bang[tid][3 * a + b] = v;
-        }
+          for (int b = 0; b < 3; ++b) {
+            double v = 0.0;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) v += iw[3 * a + c] * sk[3 * c + b];
+            sm.bang[tid][3 * a + b] = v;
+          }
+      }
     }
   }
   __syncthreads();
@@ -1742,8 +1771,34 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 #endif
   // ---------------------------------------------------------------- per-block constants
   Blk blk;
+  if constexpr (FEET) {
+    // I_w^-1 [r]x from this block's own foot, in the expressions of the per-leg products of the setup (a plan whose rows
+    // all equal the current feet gives the same bits)
 #pragma unroll
-  for (int i = 0; i < 9; ++i) blk.ba[i] = active_blk ? sm.bang[leg][i] : 0.0;
+    for (int i = 0; i < 9; ++i) blk.ba[i] = 0.0;
+    if (active_blk) {
+      const double* __restrict__ rf = &sm.bang[0][0];
+      const double* __restrict__ iw = rf + 9;
+      const double px = blk_foot[0], py = blk_foot[1], pz = blk_foot[2];
+      double fw[3];
+#pragma unroll
+      for (int r = 0; r < 3; ++r) fw[r] = rf[3 * r] * px + rf[3 * r + 1] * py + rf[3 * r + 2] * pz;
+      const double rx = fw[0], ry = fw[1], rz = fw[2];
+      const double sk[9] = {0.0, -rz, ry, rz, 0.0, -rx, -ry, rx, 0.0};
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) {
+          double v = 0.0;
+#pragma unroll
+          for (int c = 0; c < 3; ++c) v += iw[3 * a + c] * sk[3 * c + b];
+          blk.ba[3 * a + b] = v;
+        }
+    }
+  } else {
+#pragma unroll
+    for (int i = 0; i < 9; ++i) blk.ba[i] = active_blk ? sm.bang[leg][i] : 0.0;
+  }
   blk.inv_mass = inv_mass;
   blk.two_alpha = two_alpha;
   blk.t = t_blk;
@@ -2379,10 +2434,11 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 }
 
 // Grid of the lean kernel and of the single-kernel path: one CTA per env (blockIdx.x = env).
-template <int H, bool LEAN, bool ENV_MODEL, bool PLAN = false>
+template <int H, bool LEAN, bool ENV_MODEL, bool PLAN = false, bool FEET = false>
 __device__ __forceinline__ void solve_grid(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env,
                                            const rg_mpc_io& io, const rg_mpc_env_model& model,
-                                           const uint8_t* __restrict__ plan = nullptr) {
+                                           const uint8_t* __restrict__ plan = nullptr,
+                                           const float* __restrict__ feet = nullptr) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
   const int env = blockIdx.x;
@@ -2391,17 +2447,18 @@ __device__ __forceinline__ void solve_grid(const RgMpcDev* __restrict__ ws, RgMp
   RG_GRID_WAIT();                // launched programmatically behind the step prologue in rg_control_step; a no-op otherwise
 #endif
   if (env >= n_env) return;
-  solve_env<H, LEAN, ENV_MODEL, PLAN>(sm, ws, scratch, env, false, io, model, plan);
+  solve_env<H, LEAN, ENV_MODEL, PLAN, FEET>(sm, ws, scratch, env, false, io, model, plan, feet);
 }
 
 // Second kernel of the two-kernel solve: the complete solver on the envs the lean kernel queued.  Persistent CTAs
 // stride over the list (it is empty for trot / walk batches: the launch then costs a few microseconds); the cold
 // start is skipped -- the lean kernel has just spent its budget on exactly those rounds.  The last CTA to finish
 // re-arms the queue counters for the next solve.
-template <int H, bool ENV_MODEL, bool PLAN = false>
+template <int H, bool ENV_MODEL, bool PLAN = false, bool FEET = false>
 __device__ __forceinline__ void fallback_grid(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env,
                                               const rg_mpc_io& io, const rg_mpc_env_model& model,
-                                              const uint8_t* __restrict__ plan = nullptr) {
+                                              const uint8_t* __restrict__ plan = nullptr,
+                                              const float* __restrict__ feet = nullptr) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
 #if RG_PDL
@@ -2412,7 +2469,7 @@ __device__ __forceinline__ void fallback_grid(const RgMpcDev* __restrict__ ws, R
   for (int q = blockIdx.x; q < count; q += gridDim.x) {
     const int env = scratch->queue[q];
     if (env >= 0 && env < n_env)
-      solve_env<H, false, ENV_MODEL, PLAN>(sm, ws, scratch, env, true, io, model, plan);
+      solve_env<H, false, ENV_MODEL, PLAN, FEET>(sm, ws, scratch, env, true, io, model, plan, feet);
     __syncthreads();   // shared memory is reused by the next env of this CTA
   }
   if (threadIdx.x == 0) {
@@ -2470,6 +2527,21 @@ mpc_fallback_plan_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restri
   fallback_grid<H, true, true>(ws, scratch, n_env, io, model, plan);
 }
 
+// Foothold-plan twins (rg_mpc_build_solve_footholds): with the schedule and the per-env model, as the schedule twins.
+template <int H, bool LEAN>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_solve_feet_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
+                      const rg_mpc_env_model model, const uint8_t* __restrict__ plan, const float* __restrict__ feet) {
+  solve_grid<H, LEAN, true, true, true>(ws, scratch, n_env, io, model, plan, feet);
+}
+
+template <int H>
+__global__ void __launch_bounds__(Cfg<H>::NT, Cfg<H>::MIN_BLOCKS)
+mpc_fallback_feet_kernel(const RgMpcDev* __restrict__ ws, RgMpcScratch* __restrict__ scratch, int n_env, const rg_mpc_io io,
+                         const rg_mpc_env_model model, const uint8_t* __restrict__ plan, const float* __restrict__ feet) {
+  fallback_grid<H, true, true, true>(ws, scratch, n_env, io, model, plan, feet);
+}
+
 // Dynamic shared memory above 48 KB (h = 20) and the carveout are per-device function attributes: set them once
 // per (kernel, device), under a lock -- a process may drive several GPUs from several threads.
 int configure_kernel(const void* kernel, size_t smem, int min_blocks, const char* what) {
@@ -2516,20 +2588,26 @@ int sm_count() {
 template <bool B, class A, class C>
 constexpr auto pick(A a, C c) { if constexpr (B) return c; else return a; }
 
-template <int H, bool ENV_MODEL, bool PLAN = false>
+template <int H, bool ENV_MODEL, bool PLAN = false, bool FEET = false>
 int launch_kernels(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
-                   const rg_mpc_env_model& model, const uint8_t* plan = nullptr) {
+                   const rg_mpc_env_model& model, const uint8_t* plan = nullptr, const float* feet = nullptr) {
   static_assert(!PLAN || ENV_MODEL, "the schedule kernels are instantiated with the per-env model only");
-  const auto lean_kernel = pick<PLAN>(pick<ENV_MODEL>(mpc_solve_kernel<H, true>, mpc_solve_model_kernel<H, true>),
-                                      mpc_solve_plan_kernel<H, true>);
-  const auto full_kernel = pick<PLAN>(pick<ENV_MODEL>(mpc_solve_kernel<H, false>, mpc_solve_model_kernel<H, false>),
-                                      mpc_solve_plan_kernel<H, false>);
-  const auto fallback_kernel = pick<PLAN>(pick<ENV_MODEL>(mpc_fallback_kernel<H>, mpc_fallback_model_kernel<H>),
-                                          mpc_fallback_plan_kernel<H>);
+  static_assert(!FEET || PLAN, "the foothold kernels are instantiated with the schedule only");
+  const auto lean_kernel = pick<FEET>(pick<PLAN>(pick<ENV_MODEL>(mpc_solve_kernel<H, true>, mpc_solve_model_kernel<H, true>),
+                                                 mpc_solve_plan_kernel<H, true>),
+                                      mpc_solve_feet_kernel<H, true>);
+  const auto full_kernel = pick<FEET>(pick<PLAN>(pick<ENV_MODEL>(mpc_solve_kernel<H, false>, mpc_solve_model_kernel<H, false>),
+                                                 mpc_solve_plan_kernel<H, false>),
+                                      mpc_solve_feet_kernel<H, false>);
+  const auto fallback_kernel = pick<FEET>(pick<PLAN>(pick<ENV_MODEL>(mpc_fallback_kernel<H>, mpc_fallback_model_kernel<H>),
+                                                     mpc_fallback_plan_kernel<H>),
+                                          mpc_fallback_feet_kernel<H>);
   const size_t smem = sizeof(Smem<H>);
   RgMpcScratch* scratch = (RgMpcScratch*)((char*)ws + RG_MPC_SCRATCH_OFFSET);
   auto launch = [&](auto kernel, int grid, bool programmatic) {
-    if constexpr (PLAN)
+    if constexpr (FEET)
+      return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io, model, plan, feet);
+    else if constexpr (PLAN)
       return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io, model, plan);
     else if constexpr (ENV_MODEL)
       return rg_launch(kernel, dim3((unsigned)grid), dim3((unsigned)Cfg<H>::NT), smem, stream, programmatic, ws, scratch, n_env, io, model);
@@ -2564,10 +2642,14 @@ int launch_kernels(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_k
   return rc;
 }
 
-// model: NULL selects the model-free kernels; plan: non-NULL selects the schedule kernels (NULL model = the workspace's)
+// model: NULL selects the model-free kernels; plan: non-NULL selects the schedule kernels (NULL model = the workspace's);
+// feet (only with a plan): non-NULL selects the foothold kernels
 template <int H>
 int launch_h(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
-             const rg_mpc_env_model* model, const uint8_t* plan) {
+             const rg_mpc_env_model* model, const uint8_t* plan, const float* feet) {
+  if (plan && feet)
+    return launch_kernels<H, true, true, true>(ws, n_env, io, two_kernel, stream, chained,
+                                               model ? *model : rg_mpc_env_model{nullptr, nullptr, nullptr}, plan, feet);
   if (plan)
     return launch_kernels<H, true, true>(ws, n_env, io, two_kernel, stream, chained,
                                          model ? *model : rg_mpc_env_model{nullptr, nullptr, nullptr}, plan);
@@ -2672,11 +2754,11 @@ extern "C" int rg_debug_riccati_solve(int horizon, const double* k1, const doubl
 }
 
 int rg_launch_mpc(const RgMpcDev* ws, int horizon, int n_env, const rg_mpc_io& io, int two_kernel, cudaStream_t stream, int chained,
-                  const rg_mpc_env_model* model, const uint8_t* plan) {
+                  const rg_mpc_env_model* model, const uint8_t* plan, const float* feet) {
   switch (horizon) {
-    case 5: return launch_h<5>(ws, n_env, io, two_kernel, stream, chained, model, plan);
-    case 10: return launch_h<10>(ws, n_env, io, two_kernel, stream, chained, model, plan);
-    case 20: return launch_h<20>(ws, n_env, io, two_kernel, stream, chained, model, plan);
+    case 5: return launch_h<5>(ws, n_env, io, two_kernel, stream, chained, model, plan, feet);
+    case 10: return launch_h<10>(ws, n_env, io, two_kernel, stream, chained, model, plan, feet);
+    case 20: return launch_h<20>(ws, n_env, io, two_kernel, stream, chained, model, plan, feet);
     default:
       rg_set_error("unsupported horizon %d (kernels are built for 5, 10, 20)", horizon);
       return RG_ERR_UNSUPPORTED;

@@ -325,6 +325,62 @@ __device__ __forceinline__ double gen_parabola(double phase, double start, doubl
   return coef_a * phase * phase + coef_b * phase + start;
 }
 
+// The Raibert foothold of one leg (RaibertSwingLegController.get_action's end point): the swing trajectory's target and
+// the touchdown point of the foothold plan (rg_control_step_footholds).
+template <class Gait>
+__device__ __forceinline__ void raibert_end(const RgRobotDev& R, int leg, const Gait& gait, const double* v_body,
+                                            double yaw_dot, const float* cmd, double* end) {
+  const double hx = R.hip_positions[leg][0], hy = R.hip_positions[leg][1];
+  const double tw[3] = {-hy, hx, 0.0};
+  const double cv[3] = {v_body[0], v_body[1], 0.0};
+  const double ds[3] = {(double)cmd[0], (double)cmd[1], 0.0};
+  const double dtw = (double)cmd[2];
+  const double hgt[3] = {0.0, 0.0, R.desired_height - R.foot_clearance};
+  const double hip[3] = {hx, hy, 0.0};
+  for (int a = 0; a < 3; ++a) {
+    const double hv = cv[a] + yaw_dot * tw[a];
+    const double thv = ds[a] + dtw * tw[a];
+    end[a] = (hv * gait.stance() / 2.0 - R.swing_kp[a] * (thv - hv)) - hgt[a] + hip[a];
+  }
+}
+
+// Rows 1 .. h-1 of one leg's contact schedule (as plan_leg) and rows 0 .. h-1 of its footholds, in one pass over the
+// horizon (rg_control_step_footholds).  col[0] (the step's own contact flag) is written by the caller.  A planted foot
+// stays where it is while the body walks over it at the commanded velocity; a touchdown inside the horizon (swing at
+// k - 1, stance at k) plants it at the Raibert foothold.  Each product and difference is rounded separately; the yaw
+// rate is not integrated (the QP's model holds the yaw).  A gait row that is not valid holds the current foot.
+template <class Gait>
+__device__ __forceinline__ void plan_leg_feet(const RgRobotDev& R, int leg, const Gait& g, bool row_ok, double t, int h,
+                                              double dt, const float* foot, const double* v_body, double yaw_dot,
+                                              const float* cmd, uint8_t* __restrict__ col, float* __restrict__ fcol) {
+  const double v[2] = {(double)cmd[0], (double)cmd[1]};
+  double end[3];
+  raibert_end(R, leg, g, v_body, yaw_dot, cmd, end);
+  double anchor[3] = {(double)foot[0], (double)foot[1], (double)foot[2]};
+  int k_a = 0;
+  bool prev = col[0] != 0;
+  for (int k = 0; k < h; ++k) {
+    bool cur = prev;
+    if (k >= 1) {
+      cur = row_ok ? (gait_desired(g, __dadd_rn(t, __dmul_rn((double)k, dt))) == RG_LEG_STANCE) : true;
+      col[4 * k] = cur ? 1 : 0;
+      if (cur && !prev) {   // touchdown (never for an invalid row: all of its rows are stance)
+        anchor[0] = end[0]; anchor[1] = end[1]; anchor[2] = end[2];
+        k_a = k;
+      }
+    }
+    if (row_ok) {
+      const double back = __dmul_rn((double)(k - k_a), dt);
+      fcol[12 * k + 0] = (float)__dsub_rn(anchor[0], __dmul_rn(back, v[0]));
+      fcol[12 * k + 1] = (float)__dsub_rn(anchor[1], __dmul_rn(back, v[1]));
+      fcol[12 * k + 2] = (float)anchor[2];   // v_z = 0
+    } else {
+      fcol[12 * k + 0] = foot[0]; fcol[12 * k + 1] = foot[1]; fcol[12 * k + 2] = foot[2];
+    }
+    prev = cur;
+  }
+}
+
 // RaibertSwingLegController.update (latch) + get_action up to the IK call, for one leg.
 // Returns true if a swing target was produced (leg_state not in {STANCE, EARLY_CONTACT}).
 template <class Gait>
@@ -337,19 +393,8 @@ __device__ __forceinline__ bool swing_leg(const RgRobotDev& R, int leg, const Ga
   }
   last_state = desired;
   if (state == RG_LEG_STANCE || state == RG_LEG_EARLY_CONTACT) return false;
-  const double hx = R.hip_positions[leg][0], hy = R.hip_positions[leg][1];
-  const double tw[3] = {-hy, hx, 0.0};
-  const double cv[3] = {v_body[0], v_body[1], 0.0};
-  const double ds[3] = {(double)cmd[0], (double)cmd[1], 0.0};
-  const double dtw = (double)cmd[2];
-  const double hgt[3] = {0.0, 0.0, R.desired_height - R.foot_clearance};
-  const double hip[3] = {hx, hy, 0.0};
   double end[3];
-  for (int a = 0; a < 3; ++a) {
-    const double hv = cv[a] + yaw_dot * tw[a];
-    const double thv = ds[a] + dtw * tw[a];
-    end[a] = (hv * gait.stance() / 2.0 - R.swing_kp[a] * (thv - hv)) - hgt[a] + hip[a];
-  }
+  raibert_end(R, leg, gait, v_body, yaw_dot, cmd, end);
   // _gen_swing_foot_trajectory
   double phase;
   if (nphase <= 0.5) phase = 0.8 * sin(nphase * 3.14159265358979323846);
@@ -509,10 +554,11 @@ __global__ void pack_kernel(const RgRobotDev* __restrict__ R, int n_env, const i
 // unused one, moves ptxas's register assignment: DESIGN.md §3.12), so they compile to the code they had before the
 // per-env gait existed (DESIGN.md §3.14).
 // PLAN = true (Gait = EnvGait): the prologue also writes the env's contact schedule `plan` ([N,h,4], rg_control_step_plan).
-template <class Gait, bool PLAN = false>
+// FEET = true (with PLAN): ... and its foothold plan `feet` ([N,h,12], rg_control_step_footholds).
+template <class Gait, bool PLAN = false, bool FEET = false>
 __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__ R, int n_env, const rg_controller_state& s,
                                                   const rg_gait_env_params& gp, uint8_t* __restrict__ plan = nullptr,
-                                                  int h = 0, double dt = 0.0) {
+                                                  int h = 0, double dt = 0.0, float* __restrict__ feet = nullptr) {
   RG_GRID_LAUNCH_DEPENDENTS();   // the solve kernel is launched programmatically behind this grid (rg_control_step)
   const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int env = (int)(idx >> 2), leg = (int)(idx & 3);
@@ -559,7 +605,11 @@ __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__
   if constexpr (PLAN) {
     uint8_t* col = plan + 4 * (size_t)h * env + leg;
     col[0] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
-    plan_leg(g, row_ok, t, h, dt, col);
+    if constexpr (FEET)
+      plan_leg_feet(*R, leg, g, row_ok, t, h, dt, s.foot_positions_base + 3 * idx, vbr, yaw_dot, s.command + 3 * (size_t)env,
+                    col, feet + 12 * (size_t)h * env + 3 * leg);
+    else
+      plan_leg(g, row_ok, t, h, dt, col);
   }
   int32_t ls = s.last_leg_state[idx];
   double tg[3];
@@ -582,10 +632,10 @@ __device__ __forceinline__ void step_prologue_leg(const RgRobotDev* __restrict__
 // The same prologue with one thread per env (the four legs unrolled): fewer, fatter threads -- the faster mapping for
 // large batches, where the kernel is bound by its FP64 instruction count and per-leg lanes diverge (swing legs run the IK,
 // stance legs idle).  Bit-identical results: both call the same per-leg / per-axis routines.
-template <class Gait, bool PLAN = false>
+template <class Gait, bool PLAN = false, bool FEET = false>
 __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__ R, int n_env, const rg_controller_state& s,
                                                   const rg_gait_env_params& gp, uint8_t* __restrict__ plan = nullptr,
-                                                  int h = 0, double dt = 0.0) {
+                                                  int h = 0, double dt = 0.0, float* __restrict__ feet = nullptr) {
   RG_GRID_LAUNCH_DEPENDENTS();   // the solve kernel is launched programmatically behind this grid (rg_control_step)
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= n_env) return;
@@ -620,6 +670,12 @@ __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__
     s.normalized_phase[idx] = np;
     s.mpc_contact_state[idx] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
     if constexpr (PLAN) row0 |= (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1u << (8 * leg) : 0u;
+    if constexpr (FEET) {   // the leg's schedule column and footholds in one pass (byte stores instead of row words)
+      uint8_t* col = plan + 4 * (size_t)h * env + leg;
+      col[0] = (d == RG_LEG_STANCE || d == RG_LEG_EARLY_CONTACT) ? 1 : 0;
+      plan_leg_feet(*R, leg, g, valid, t, h, dt, s.foot_positions_base + 3 * idx, vbr, yaw_dot, s.command + 3 * (size_t)env,
+                    col, feet + 12 * (size_t)h * env + 3 * leg);
+    }
     int32_t ls = s.last_leg_state[idx];
     double tg[3];
     const bool has = swing_leg(*R, leg, g, d, st, np, s.foot_positions_base + 3 * idx, vbr, yaw_dot,
@@ -637,7 +693,7 @@ __device__ __forceinline__ void step_prologue_env(const RgRobotDev* __restrict__
       s.swing_joint_valid[idx] = 1;
     }
   }
-  if constexpr (PLAN) {   // one 4-byte store per row: the row's four leg bytes assembled in a register
+  if constexpr (PLAN && !FEET) {   // one 4-byte store per row: the row's four leg bytes assembled in a register
     unsigned* rows = reinterpret_cast<unsigned*>(plan + 4 * (size_t)h * env);
     rows[0] = row0;
     for (int k = 1; k < h; ++k) {
@@ -682,6 +738,19 @@ __global__ void step_prologue_plan_kernel(const RgRobotDev* __restrict__ R, int 
 __global__ void step_prologue_env_plan_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
                                               rg_gait_env_params gp, uint8_t* __restrict__ plan, int h, double dt) {
   step_prologue_env<EnvGait, true>(R, n_env, s, gp, plan, h, dt);
+}
+
+// Foothold-plan twins (rg_control_step_footholds): the schedule twins that also write the foothold plan.
+__global__ void step_prologue_feet_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
+                                          rg_gait_env_params gp, uint8_t* __restrict__ plan, float* __restrict__ feet,
+                                          int h, double dt) {
+  step_prologue_leg<EnvGait, true, true>(R, n_env, s, gp, plan, h, dt, feet);
+}
+
+__global__ void step_prologue_env_feet_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s,
+                                              rg_gait_env_params gp, uint8_t* __restrict__ plan, float* __restrict__ feet,
+                                              int h, double dt) {
+  step_prologue_env<EnvGait, true, true>(R, n_env, s, gp, plan, h, dt, feet);
 }
 
 __global__ void step_epilogue_kernel(const RgRobotDev* __restrict__ R, int n_env, rg_controller_state s) {
@@ -1016,6 +1085,12 @@ extern "C" int rg_control_step_env(const void* mpc_ws, const void* robot_ws, int
 extern "C" int rg_control_step_plan(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                     const rg_mpc_env_model* model, const rg_gait_env_params* gait, uint8_t* plan,
                                     void* stream) {
+  return rg_control_step_footholds(mpc_ws, robot_ws, n_env, s, model, gait, plan, nullptr, stream);
+}
+
+extern "C" int rg_control_step_footholds(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
+                                         const rg_mpc_env_model* model, const rg_gait_env_params* gait, uint8_t* plan,
+                                         float* feet, void* stream) {
   if (n_env == 0) return RG_OK;   // empty batch: nothing to validate, nothing to launch
   RG_REQUIRE(mpc_ws && robot_ws && s && n_env >= 0, "rg_control_step");
   RG_REQUIRE(s->time_since_reset && s->foot_contacts && s->base_velocity_world && s->base_orientation_xyzw && s->base_rpy &&
@@ -1037,6 +1112,14 @@ extern "C" int rg_control_step_plan(const void* mpc_ws, const void* robot_ws, in
     rg_set_error("rg_control_step_plan: contact_schedule_out must be 4-byte aligned");
     return RG_ERR_BAD_ARG;
   }
+  if (feet && !plan) {
+    rg_set_error("rg_control_step_footholds: a foothold plan needs contact_schedule_out");
+    return RG_ERR_BAD_ARG;
+  }
+  if ((uintptr_t)feet & 15u) {
+    rg_set_error("rg_control_step_footholds: foothold_plan_out must be 16-byte aligned");
+    return RG_ERR_BAD_ARG;
+  }
   cudaStream_t st = (cudaStream_t)stream;
   const RgRobotDev* R = (const RgRobotDev*)robot_ws;
   RgMpcHostInfo info;
@@ -1044,7 +1127,11 @@ extern "C" int rg_control_step_plan(const void* mpc_ws, const void* robot_ws, in
     rc = rg_mpc_workspace_info(mpc_ws, &info);
     if (rc != RG_OK) return rc;
     const rg_gait_env_params gp = g ? *g : rg_gait_env_params{nullptr, nullptr, nullptr, nullptr};
-    if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS)
+    if (feet && n_env <= RG_PROLOGUE_LEG_MAX_ENVS)
+      step_prologue_feet_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, feet, info.horizon, info.dt);
+    else if (feet)
+      step_prologue_env_feet_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, feet, info.horizon, info.dt);
+    else if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS)
       step_prologue_plan_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, info.horizon, info.dt);
     else
       step_prologue_env_plan_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, info.horizon, info.dt);
@@ -1077,7 +1164,7 @@ extern "C" int rg_control_step_plan(const void* mpc_ws, const void* robot_ws, in
   io.zero_yaw = 1;
   // prologue -> solve kernel(s) -> epilogue are chained by programmatic dependent launches: each grid becomes resident
   // while its predecessor drains and waits (griddepcontrol.wait) for it to complete, so the launch latencies overlap
-  rc = rg_launch_mpc((const RgMpcDev*)mpc_ws, info.horizon, n_env, io, info.two_kernel && info.queue_capacity >= n_env, st, 1, m, plan);
+  rc = rg_launch_mpc((const RgMpcDev*)mpc_ws, info.horizon, n_env, io, info.two_kernel && info.queue_capacity >= n_env, st, 1, m, plan, feet);
   if (rc != RG_OK) return rc;
   rc = rg_check_cuda(rg_launch(step_epilogue_kernel, dim3((unsigned)grid_for(4 * n_env, 256)), dim3(256), 0, st, true,
                                (const RgRobotDev*)robot_ws, n_env, *s), "step_epilogue_kernel launch");
@@ -1114,12 +1201,19 @@ extern "C" int rg_control_step_graph_create_env(const void* mpc_ws, const void* 
 extern "C" int rg_control_step_graph_create_plan(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s,
                                                  const rg_mpc_env_model* model, const rg_gait_env_params* gait, uint8_t* plan,
                                                  void* stream, void** graph_out) {
+  return rg_control_step_graph_create_footholds(mpc_ws, robot_ws, n_env, s, model, gait, plan, nullptr, stream, graph_out);
+}
+
+extern "C" int rg_control_step_graph_create_footholds(const void* mpc_ws, const void* robot_ws, int n_env,
+                                                      const rg_controller_state* s, const rg_mpc_env_model* model,
+                                                      const rg_gait_env_params* gait, uint8_t* plan, float* feet,
+                                                      void* stream, void** graph_out) {
   RG_REQUIRE(mpc_ws && robot_ws && s && graph_out && n_env > 0, "rg_control_step_graph_create");
   *graph_out = nullptr;
   // one eager step on the caller's stream first: kernel attributes get configured outside the capture, and argument
   // errors surface here with their own message.  The controller state advances by this step -- the caller accounts for it
   // by creating the graph INSTEAD of a step, not before one (see rg_cuda.h).
-  int rc = rg_control_step_plan(mpc_ws, robot_ws, n_env, s, model, gait, plan, stream);
+  int rc = rg_control_step_footholds(mpc_ws, robot_ws, n_env, s, model, gait, plan, feet, stream);
   if (rc == RG_OK) rc = rg_check_cuda(cudaStreamSynchronize((cudaStream_t)stream), "graph warm-up step");
   if (rc != RG_OK) return rc;
   cudaStream_t cap = nullptr;
@@ -1129,7 +1223,7 @@ extern "C" int rg_control_step_graph_create_plan(const void* mpc_ws, const void*
   RgStepGraph* g = new RgStepGraph{nullptr, nullptr, 0};
   cudaError_t e = cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal);
   if (e == cudaSuccess) {
-    rc = rg_control_step_plan(mpc_ws, robot_ws, n_env, s, model, gait, plan, cap);
+    rc = rg_control_step_footholds(mpc_ws, robot_ws, n_env, s, model, gait, plan, feet, cap);
     e = cudaStreamEndCapture(cap, &g->graph);
     if (rc != RG_OK) e = cudaErrorUnknown;
   }

@@ -65,7 +65,7 @@ class BatchedMPCController(Controller):
     GRAPH_MAX_ENVS = 2048          # below this a control step is launch-bound: replay it as one CUDA graph
 
     def __init__(self, robot, get_time_since_reset, horizon=10, mpc_overrides=None, squeeze_single=True,
-                 warm_start=True, use_graph=None, contact_plan=False):
+                 warm_start=True, use_graph=None, contact_plan=False, foothold_plan=False):
         """``robot``: batched state provider with the getter names of robot.py (see
         ``SyntheticRobotBatch``); ``get_time_since_reset``: callable returning a float or an
         ``[N]`` float64 tensor (Simulation.GetTimeSinceReset, core/simulation.py:141-142).
@@ -73,7 +73,13 @@ class BatchedMPCController(Controller):
         earlier (``rg_mpc_build_solve_warm``); the optimum is unique, so the forces do not depend on it.
         ``contact_plan``: plan the stance QP over each env's gait schedule -- the desired stance of every leg at every
         horizon step (``rg_control_step_plan``) -- instead of holding the current contact row over the horizon.  The
-        schedule the step solved against is ``mpc_contact_schedule`` ([N, horizon, 4] uint8, row 0 = ``mpc_contact_state``)."""
+        schedule the step solved against is ``mpc_contact_schedule`` ([N, horizon, 4] uint8, row 0 = ``mpc_contact_state``).
+        ``foothold_plan`` (needs ``contact_plan``): take the QP's lever arms at every horizon step from the predicted
+        footholds (``rg_control_step_footholds``): a planted foot moves back at the commanded velocity, and a leg that
+        touches down inside the horizon lands at its Raibert foothold.  The footholds the step solved against are
+        ``mpc_foothold_plan`` ([N, horizon, 4, 3] float32, in the frame of the feet's base positions)."""
+        if foothold_plan and not contact_plan:
+            raise ValueError("foothold_plan=True needs contact_plan=True (the footholds follow the contact schedule)")
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedMPCController needs a CUDA device (no CPU fallback)")
         rg.load()
@@ -141,6 +147,7 @@ class BatchedMPCController(Controller):
         self.solve_info = z((n, 4), i32)
         self.mpc_active_set = rg.new_active_set(n, self.horizon, dev) if warm_start else None
         self.mpc_contact_schedule = z((n, self.horizon, 4), u8) if contact_plan else None
+        self.mpc_foothold_plan = z((n, self.horizon, 4, 3), f32) if foothold_plan else None
         self.action = z((n, 60), f32)
         self.reset_time = z((n,), f64)
         self.time_since_reset = z((n,), f64)
@@ -338,7 +345,12 @@ class BatchedMPCController(Controller):
                 if self._graph is None:
                     # creating the graph executes this step eagerly (and synchronises once)
                     handle = ctypes.c_void_p()
-                    if self.mpc_contact_schedule is not None:
+                    if self.mpc_foothold_plan is not None:
+                        rg.check(lib.rg_control_step_graph_create_footholds(
+                            self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
+                            self._env_model_ref(), self._env_gait_ref(), self._schedule_ptr(), self._footholds_ptr(),
+                            rg.current_stream_ptr(), ctypes.byref(handle)))
+                    elif self.mpc_contact_schedule is not None:
                         rg.check(lib.rg_control_step_graph_create_plan(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
                                                                        ctypes.byref(self._state), self._env_model_ref(),
                                                                        self._env_gait_ref(), self._schedule_ptr(),
@@ -358,7 +370,11 @@ class BatchedMPCController(Controller):
         return self.action
 
     def _eager_step(self, lib):
-        if self.mpc_contact_schedule is not None:
+        if self.mpc_foothold_plan is not None:
+            rg.check(lib.rg_control_step_footholds(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs,
+                                                   ctypes.byref(self._state), self._env_model_ref(), self._env_gait_ref(),
+                                                   self._schedule_ptr(), self._footholds_ptr(), rg.current_stream_ptr()))
+        elif self.mpc_contact_schedule is not None:
             rg.check(lib.rg_control_step_plan(self._mpc_ws.ptr, self._robot_ws.ptr, self.num_envs, ctypes.byref(self._state),
                                               self._env_model_ref(), self._env_gait_ref(), self._schedule_ptr(),
                                               rg.current_stream_ptr()))
@@ -371,6 +387,10 @@ class BatchedMPCController(Controller):
 
     def _schedule_ptr(self):
         return rg._ptr(self.mpc_contact_schedule, torch.uint8, (self.horizon, 4), n=self.num_envs, device=self.device, align=4)
+
+    def _footholds_ptr(self):
+        return rg._ptr(self.mpc_foothold_plan, torch.float32, (self.horizon, 4, 3), n=self.num_envs, device=self.device,
+                       align=16)
 
     def _env_model_ref(self):
         return None if self._env_model is None else ctypes.byref(self._env_model)

@@ -34,6 +34,7 @@ EXPORTED_SYMBOLS = (
     "rg_force_to_torque", "rg_pack_hybrid_action", "rg_control_step", "rg_control_step_graph_create", "rg_control_step_graph_launch", "rg_control_step_graph_destroy",
     "rg_control_step_model", "rg_control_step_graph_create_model", "rg_control_step_env", "rg_control_step_graph_create_env",
     "rg_mpc_build_solve_schedule", "rg_control_step_plan", "rg_control_step_graph_create_plan",
+    "rg_mpc_build_solve_footholds", "rg_control_step_footholds", "rg_control_step_graph_create_footholds",
     "rg_hybrid_motor_torque", "rg_hybrid_motor_torque_ex",
     "rg_measure_fma_peak", "rg_launch_count", "rg_last_error", "rg_version",
 )
@@ -173,6 +174,13 @@ def load(build_if_missing: bool = False):
                                          POINTER(GaitEnvParams), c_void_p, c_void_p]
     lib.rg_control_step_graph_create_plan.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
                                                       POINTER(GaitEnvParams), c_void_p, c_void_p, POINTER(c_void_p)]
+    lib.rg_mpc_build_solve_footholds.argtypes = [c_void_p, c_int, POINTER(MpcIo), POINTER(MpcEnvModel), c_void_p, c_void_p,
+                                                 c_void_p]
+    lib.rg_control_step_footholds.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState), POINTER(MpcEnvModel),
+                                              POINTER(GaitEnvParams), c_void_p, c_void_p, c_void_p]
+    lib.rg_control_step_graph_create_footholds.argtypes = [c_void_p, c_void_p, c_int, POINTER(ControllerState),
+                                                           POINTER(MpcEnvModel), POINTER(GaitEnvParams), c_void_p, c_void_p,
+                                                           c_void_p, POINTER(c_void_p)]
     lib.rg_hybrid_motor_torque.argtypes = [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.rg_hybrid_motor_torque_ex.argtypes = [c_void_p, c_int] + [c_void_p] * 6 + [c_void_p]
     lib.rg_measure_fma_peak.argtypes = [c_int, c_int, POINTER(c_double)]
@@ -299,7 +307,8 @@ def calibrate_ik(params: RobotParams, reference_motor_angles) -> None:
 def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate, foot_contact_state,
                     foot_positions_base, command, com_height=None, contact_forces=None,
                     horizon_forces=None, solve_info=None, want_horizon=False, want_info=True, active_set=None,
-                    zero_yaw=False, horizon_forces_f64=None, env_model=None, contact_schedule=None):
+                    zero_yaw=False, horizon_forces_f64=None, env_model=None, contact_schedule=None,
+                    foothold_plan=None):
     """``rg_mpc_build_solve`` (``rg_mpc_build_solve_warm`` when ``active_set`` -- an ``[N, 4*horizon]`` int16 tensor
     initialised to -1, see ``new_active_set`` -- is given) on the current stream.  ``base_rpy`` is used as given:
     pass a yaw-aligned attitude (yaw = 0) to reproduce TorqueStanceLegController (the controller's fused step
@@ -309,8 +318,13 @@ def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate
     ``friction_coeffs`` [N,4] float64 CUDA tensors, any of them None (= the workspace's value); an env whose row fails
     the workspace checks gets zero forces and RG_STATUS_BAD_MODEL.  ``contact_schedule``: the planned stance of every
     leg at every horizon step, an ``[N,h,4]`` uint8 or bool CUDA tensor (nonzero = stance; ``rg_mpc_build_solve_schedule``);
-    ``foot_contact_state`` is then not read and may be None.  Returns (contact_forces, horizon_forces, solve_info)."""
+    ``foot_contact_state`` is then not read and may be None.  ``foothold_plan``: the position of every foot at every
+    horizon step, an ``[N,h,12]`` or ``[N,h,4,3]`` float32 CUDA tensor in the frame of ``foot_positions_base``, used as
+    the QP's per-step lever arms (``rg_mpc_build_solve_footholds``); it needs ``contact_schedule``, and
+    ``foot_positions_base`` is then not read and may be None.  Returns (contact_forces, horizon_forces, solve_info)."""
     import torch
+    if foothold_plan is not None and contact_schedule is None:
+        raise ValueError("mpc_build_solve: foothold_plan needs contact_schedule")
     n = base_rpy.shape[0]
     dev = base_rpy.device
     if ws.buffer.device != dev:
@@ -327,7 +341,8 @@ def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate
             P(com_velocity_body, torch.float32, (3,)), P(base_rpy, torch.float32, (3,)),
             P(base_rpy_rate, torch.float32, (3,)),
             P(foot_contact_state, torch.uint8, (4,), align=4, allow_none=contact_schedule is not None),
-            P(foot_positions_base.view(n, 12), torch.float32, (12,), align=16), P(command, torch.float32, (3,)),
+            P(None if foot_positions_base is None else foot_positions_base.view(n, 12), torch.float32, (12,), align=16,
+              allow_none=foothold_plan is not None), P(command, torch.float32, (3,)),
             P(com_height, torch.float32, (), allow_none=True),
             P(contact_forces, torch.float32, (12,)), hf,
             P(solve_info, torch.int32, (4,), allow_none=True))
@@ -337,13 +352,22 @@ def mpc_build_solve(ws: MpcWorkspace, com_velocity_body, base_rpy, base_rpy_rate
         if isinstance(contact_schedule, torch.Tensor) and contact_schedule.dtype == torch.bool:
             contact_schedule = contact_schedule.view(torch.uint8)
         schedule = P(contact_schedule, torch.uint8, (ws.horizon, 4), align=4)
+    feet = None
+    if foothold_plan is not None:
+        if isinstance(foothold_plan, torch.Tensor) and tuple(foothold_plan.shape[1:]) == (ws.horizon, 4, 3):
+            foothold_plan = foothold_plan.view(foothold_plan.shape[0], ws.horizon, 12)
+        feet = P(foothold_plan, torch.float32, (ws.horizon, 12), align=16)
     with torch.cuda.device(dev):
         if zero_yaw or horizon_forces_f64 is not None or model is not None or schedule is not None:
             io = MpcIo(*[a if a is None or isinstance(a, int) else a.value for a in args[2:]],
                        None if active_set is None else P(active_set, torch.int16, (4 * ws.horizon,)).value,
                        None if horizon_forces_f64 is None else P(horizon_forces_f64.view(n, ws.horizon * 12), torch.float64, (ws.horizon * 12,)).value,
                        1 if zero_yaw else 0, 0)
-            if schedule is not None:
+            if feet is not None:
+                check(load().rg_mpc_build_solve_footholds(ws.ptr, n, ctypes.byref(io),
+                                                          None if model is None else ctypes.byref(model), schedule, feet,
+                                                          current_stream_ptr()))
+            elif schedule is not None:
                 check(load().rg_mpc_build_solve_schedule(ws.ptr, n, ctypes.byref(io),
                                                          None if model is None else ctypes.byref(model), schedule,
                                                          current_stream_ptr()))
