@@ -68,88 +68,40 @@ namespace {
 
 constexpr unsigned kFull = 0xffffffffu;
 
+// Linear algebra behind the Newton / active-set systems:  horizons >= kRiccatiMinH factorise Psi by a backward
+// Riccati sweep over the horizon (O(h) work and storage: riccati_factor / riccati_solve), shorter ones by the dense
+// packed Cholesky (O(h^3), but 60 rows keep 64 threads busy and the panel routine is faster up to h = 10; measured
+// in profiles/r02_riccati_vs_cholesky.md).
+constexpr int kRiccatiMinH = 20;
+
 template <int H>
 struct Cfg {
   static constexpr int N6 = 6 * H;
   static constexpr int NB = 4 * H;
-#ifndef RG_RICCATI_MIN_H
-#define RG_RICCATI_MIN_H 20
-#endif
+  static constexpr bool RICCATI = H >= kRiccatiMinH;
   // Threads per CTA.  Dense path: one per row of Psi (6h) for the Cholesky.  Riccati path: the sweeps run in one warp,
   // so only the 4h (step, leg) block threads are needed -- the 6h "rows" of K-products are looped over (h = 20: 96
   // threads instead of 128, i.e. 5 resident CTAs per SM at 128 registers instead of 4).
-  static constexpr bool RICCATI_ = H >= RG_RICCATI_MIN_H;
-  static constexpr int NT = RICCATI_ ? ((NB + 31) / 32) * 32 : ((N6 + 31) / 32) * 32;
+  static constexpr int NT = RICCATI ? ((NB + 31) / 32) * 32 : ((N6 + 31) / 32) * 32;
   static constexpr int NW = NT / 32;
-  // Psi rows are stored with an even number of slots each (row i holds i+1 entries) so that every row
-  // starts 16-byte aligned and the hot loops can use 128-bit shared-memory loads: see prow().
-#ifdef RG_PADDED_ROWS
-  static constexpr int NPSI = (N6 % 2 == 0) ? 2 * (N6 / 2) * (N6 / 2 + 1) : 2 * (N6 / 2 + 1) * (N6 / 2 + 1);
-#else
   static constexpr int NPSI = N6 * (N6 + 1) / 2 + 64;   // slack: the pipelined loads of the factor routines over-read (values unused)
-#endif
   static constexpr int NA = 3 * H;
   static constexpr int NKA = NA * (NA + 1) / 2;
   static constexpr int RPL = (N6 + 31) / 32;   // Psi rows per lane in the triangular sweeps
-  // resident CTAs per SM the register allocation is sized for (shared memory allows 9 / 2 at h = 10 / 20)
-// Cholesky panel width at h = 10: 4 (hand-pipelined cholesky_rows) or 6 (cholesky_rows_w, one panel per time
-// block).  6 measured between +2 % and -25 % at h = 10 depending on the build, -12 % at h = 5, -33 % at h = 20:
-// kept as an A/B option only.
-#ifndef RG_CHOL_W_H10
-#define RG_CHOL_W_H10 4
-#endif
-// resident CTAs per SM at h = 10 (launch bound and shared-memory carveout).  8 until the instruction-count pass of round 2
-// had loaded the shared-memory pipe to 60 % of its wavefront peak; since then 7 is faster (+2.5 % at 65536 envs, +3.5 %
-// at 4096, where 4096 / (148 x 7) is almost a whole number of waves); 6: -6 %, 9: -4 %.
-#ifndef RG_MIN_BLOCKS_H10
-#define RG_MIN_BLOCKS_H10 7
-#endif
-// the two heavy routines: one out-of-line copy each (default) or inlined at their call sites (A/B)
-#ifndef RG_HEAVY_INLINE
-#define RG_HEAVY_INLINE __noinline__
-#endif
-#ifndef RG_MIN_BLOCKS_H5
-#define RG_MIN_BLOCKS_H5 24
-#endif
-// Linear algebra behind the Newton / active-set systems:  horizons >= RG_RICCATI_MIN_H factorise Psi by a backward
-// Riccati sweep over the horizon (O(h) work and storage: riccati_factor / riccati_solve), shorter ones by the dense
-// packed Cholesky (O(h^3), but 60 rows keep 64 threads busy and the panel routine is faster up to h = 10; measured
-// in profiles/r02_riccati_vs_cholesky.md).
-#ifndef RG_RICCATI_MIN_H
-#define RG_RICCATI_MIN_H 20
-#endif
-#ifndef RG_MIN_BLOCKS_H20
-#define RG_MIN_BLOCKS_H20 5
-#endif
-  static constexpr bool RICCATI = H >= RG_RICCATI_MIN_H;
-  // active-set basis of a block in named registers (no local-memory frame: DRAM traffic = algorithmic bytes) or in small
-  // local arrays indexed by the run-time row count.  With the basis kept live across the heavy phases the registers won
-  // only at h = 10 (profiles/r02_basis_storage.md); since it is rebuilt for the multiplier test (RG_REBUILD_BASIS) they
-  // win everywhere: h = 5 27.2 -> 28.8 M, h = 20 5.72 -> 5.85 M solves/s at 65536 envs.  The array scheme stays as an A/B option.
-#ifndef RG_BASIS_IN_REGS_H10
-#define RG_BASIS_IN_REGS_H10 1
-#endif
-#ifndef RG_BASIS_IN_REGS_H5
-#define RG_BASIS_IN_REGS_H5 1
-#endif
-#ifndef RG_BASIS_IN_REGS_H20
-#define RG_BASIS_IN_REGS_H20 1
-#endif
-  static constexpr bool BASIS_IN_REGS = H == 10 ? RG_BASIS_IN_REGS_H10 : (H < 10 ? RG_BASIS_IN_REGS_H5 : RG_BASIS_IN_REGS_H20);
   // the gradient at the particular solution is evaluated as "pass -1" of the solve / refine loop (one inlined copy of
   // apply_p instead of two: less code on the round's path; +1.5 % at h = 10, -3 % at h = 5 where the kernel spills)
-#ifndef RG_GRAD_IN_PASS_LOOP_H10
-#define RG_GRAD_IN_PASS_LOOP_H10 1
-#endif
-  static constexpr bool GRAD_IN_PASS_LOOP = (H == 10) && RG_GRAD_IN_PASS_LOOP_H10;
-  static constexpr int CHOL_W = (H == 10) ? RG_CHOL_W_H10 : 4;
-  static constexpr int MIN_BLOCKS = H <= 5 ? RG_MIN_BLOCKS_H5 : (H <= 10 ? RG_MIN_BLOCKS_H10 : (RICCATI ? RG_MIN_BLOCKS_H20 : 2));
+  static constexpr bool GRAD_IN_PASS_LOOP = H == 10;
+  // resident CTAs per SM the register allocation is sized for (launch bound and shared-memory carveout; shared memory
+  // allows 9 / 2 at h = 10 / 20).  h = 10: 8 until the instruction-count pass of round 2 had loaded the shared-memory pipe
+  // to 60 % of its wavefront peak; since then 7 is faster (+2.5 % at 65536 envs, +3.5 % at 4096, where 4096 / (148 x 7)
+  // is almost a whole number of waves); 6: -6 %, 9: -4 %.
+  static constexpr int MIN_BLOCKS = H <= 5 ? 24 : (H <= 10 ? 7 : 5);
 };
 
 template <int H, bool RIC = Cfg<H>::RICCATI>
 struct Smem {
   // dense path: Psi and its Cholesky factor
-  __align__(16) double psi[RIC ? 2 : Cfg<H>::NPSI];   // lower triangle, row-major, rows padded to even length (prow)
+  __align__(16) double psi[RIC ? 2 : Cfg<H>::NPSI];   // lower triangle, row-major, packed (prow)
   double kinv_ang[RIC ? 1 : Cfg<H>::NKA];    // K^-1 angular block, packed, index a = 3 j + c
   __align__(16) double rdiag[RIC ? 1 : Cfg<H>::N6];
   // Riccati path (see riccati_factor): per stage P_{t+1} Gam (12 x 6), J_t, N_t (6 x 6), and the sweep's scratch
@@ -165,7 +117,7 @@ struct Smem {
   double gt[H * 6];                // g~ : gradient in acceleration space
   __align__(16) double avec[H * 6];   // W u, right-hand sides and Woodbury solutions
   double kvec[H * 6];              // K (W u)
-  __align__(16) double blk44[36];  // updated diagonal block of the current Cholesky panel (4x4 or 6x6)
+  __align__(16) double blk44[36];  // updated 4x4 diagonal block of the current Cholesky panel (36: the tuned smem layout)
   double bang[4][9];               // A_leg = I_world^-1 [r_leg]x
   double k2ang[9];
   double k1[6];
@@ -179,94 +131,38 @@ struct Smem {
 __device__ __forceinline__ int tri(int i, int k) { return i * (i + 1) / 2 + k; }
 
 // offset of row i of the lower-triangular Psi storage.
-#ifdef RG_PADDED_ROWS
-// rows padded to even length (16-byte aligned rows, 128-bit loads): sum_{r<i} 2 ceil((r+1)/2)
-__device__ __forceinline__ int prow(int i) {
-  const int p = i >> 1;
-  return (i & 1) ? 2 * (p + 1) * (p + 1) : 2 * p * (p + 1);
-}
-__device__ __forceinline__ double2 ld2(const double* p) { return *reinterpret_cast<const double2*>(p); }
-#else
 // packed triangle: T(i) mod 16 is a permutation over 16 consecutive rows, so the per-column 64-bit
 // accesses of a half-warp (same column, consecutive rows) are bank-conflict free
 __device__ __forceinline__ int prow(int i) { return i * (i + 1) / 2; }
 __device__ __forceinline__ double2 ld2(const double* p) { return make_double2(p[0], p[1]); }
-#endif
 // 128-bit load of two consecutive doubles; the caller guarantees 16-byte alignment
 __device__ __forceinline__ double2 ld2v(const double* p) { return *reinterpret_cast<const double2*>(p); }
 
 __device__ __forceinline__ double c1f(int h, int j, int k) { return (double)(h - (j > k ? j : k)); }
 
-// After the first solve of an active-set round the refinement pass is skipped when the projected
-// gradient is already below this (relative to the gradient scale): the error it leaves in the
-// weakly curved directions is <= tol / (2 alpha).
-#ifndef RG_IPM_LAM0
-#define RG_IPM_LAM0 0.01
-#endif
 // Interior-point start (used only when the cold start gives up; A/B in tools/ab_gaits.py):
-//   mu0 = RG_IPM_LAM0 * max(|q|, RG_IPM_RD_SCALE * |P u0 + q|)   centred start s lam = mu0
-//   u0  = safe point + RG_IPM_WARM * (largest strictly feasible step towards the last active-set iterate)
-#ifndef RG_IPM_RD_SCALE
-#define RG_IPM_RD_SCALE 1.0
-#endif
-#ifndef RG_ADD_ONE_PER_BLOCK
-#define RG_ADD_ONE_PER_BLOCK 1
-#endif
-// cold start: give up when the number of moving rows stops shrinking.  OFF since rows enter one per block per
-// round: the count is then small and not monotone, and the rule sent solvable problems to the interior point.
-#ifndef RG_COLD_NO_DECREASE_RULE
-#define RG_COLD_NO_DECREASE_RULE 0
-#endif
-#ifndef RG_IPM_TAU_LATE
-#define RG_IPM_TAU_LATE 0.99
-#endif
-#ifndef RG_IPM_SLOW_ITERS
-#define RG_IPM_SLOW_ITERS 5
-#endif
-// Cholesky update loop: 128-bit broadcast loads of the panel rows (see cholesky_rows)
-#ifndef RG_CHOL_LDS128
-#define RG_CHOL_LDS128 1
-#endif
-// unroll factor of that loop (2 or 4): a trip moves five pointers and rotates the lagged operands, ~10 of 38 instructions at 2
-#ifndef RG_CHOL_UNROLL
-#define RG_CHOL_UNROLL 4
-#endif
-// cold start: fz >= fz_min is guessed active in the last RG_COLD_GUESS_LAST steps of the horizon (0 = empty set)
-#ifndef RG_COLD_GUESS_LAST
-#define RG_COLD_GUESS_LAST 1
-#endif
-// ... and in the last RG_COLD_GUESS_LAST_4 steps when all four legs stand: the redundant legs are unloaded earlier
+//   mu0 = kIpmLam0 * max(|q|, |P u0 + q|)   centred start s lam = mu0
+//   u0  = safe point + kIpmWarm * (largest strictly feasible step towards the last active-set iterate)
+constexpr double kIpmLam0 = 0.01;
+constexpr double kIpmWarm = 0.99;
+// interior point: iterations without halving the best residual before a close iterate is handed to the rounds
+constexpr int kIpmSlowIters = 5;
+// cold start: fz >= fz_min is guessed active in the last kColdGuessLast steps of the horizon
+constexpr int kColdGuessLast = 1;
+// ... and in the last kColdGuessLast4 steps when all four legs stand: the redundant legs are unloaded earlier
 // (fz_min is active at step h-2 on 78 % of the legs of four-stance trot states against 50 % with two stance legs,
 // and a four-stance problem never verifies from the one-step guess alone: tools/experiments/guess_stats.py)
-#ifndef RG_COLD_GUESS_LAST_4
-#define RG_COLD_GUESS_LAST_4 2
-#endif
-// cold start: rounds granted beyond cold_start_rounds while at most this many rows still move
-#ifndef RG_COLD_EXTEND_ROUNDS
-#define RG_COLD_EXTEND_ROUNDS 0
-#endif
-#ifndef RG_COLD_EXTEND_NCHG
-#define RG_COLD_EXTEND_NCHG 4.0
-#endif
-#ifndef RG_IPM_WARM
-#define RG_IPM_WARM 0.99
-#endif
+constexpr int kColdGuessLast4 = 2;
+// cold start: its last round hands over when more than this many rows still move
+constexpr double kColdLastRoundNchg = 4.0;
 // multiplier tolerance (relative to the gradient scale) below which a STICKY row -- one that was dropped and came back --
 // is still held: it stops the in / out cycling of weakly active rows, at the price of a point that may sit up to
 // tol / (2 alpha) away from the optimum along a weakly curved direction
-#ifndef RG_STICKY_TOL
-#define RG_STICKY_TOL 1e-9
-#endif
-// programmatic dependent launch of the fallback kernel behind the lean kernel (launch_h)
-#ifndef RG_PDL
-#define RG_PDL 1
-#endif
-#ifndef RG_REBUILD_BASIS
-#define RG_REBUILD_BASIS 1
-#endif
-#ifndef RG_SKIP_REFINE_TOL
-#define RG_SKIP_REFINE_TOL 1e-10
-#endif
+constexpr double kStickyTol = 1e-9;
+// After the first solve of an active-set round the refinement pass is skipped when the projected
+// gradient is already below this (relative to the gradient scale): the error it leaves in the
+// weakly curved directions is <= tol / (2 alpha).
+constexpr double kSkipRefineTol = 1e-10;
 
 // ---- block-wide reductions (all threads call; result valid in all threads) -------------------
 // WHAT: bit 0 = the sum, bit 1 = the maximum, bit 2 = the minimum is wanted (the others are left untouched)
@@ -308,14 +204,10 @@ __device__ __forceinline__ double quad_sum(double v) {   // sum over the 4 legs 
 // y (1 + e/2 + 3 e^2/8), e = 1 - d y^2  (error 5 e^3 / 16 < 2^-60): 6 instructions on the pivot chain instead of the 12
 // of rsqrt() with its range checks.  No special cases: d <= 0 gives NaN / inf, which the caller tests for once per panel.
 __device__ __forceinline__ double rsqrt_pivot(double d) {
-#ifdef RG_LIBM_RSQRT
-  return rsqrt(d);
-#else
   double y;
   asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(d));
   const double e = fma(-(d * y), y, 1.0);
   return fma(y * e, fma(0.375, e, 0.5), y);
-#endif
 }
 
 // ---- in-place Cholesky of the packed SPD matrix: one thread per row, panels of 4 columns --------
@@ -333,7 +225,7 @@ __device__ __forceinline__ double rsqrt_pivot(double d) {
 // j_begin (a multiple of 4): columns before it already hold the factor and are kept -- a matrix that
 // changed only in rows/columns >= j_begin has the same leading factor columns (left-looking order).
 template <int H, class SM>
-__device__ RG_HEAVY_INLINE void cholesky_rows(SM& sm, int j_begin) {
+__device__ __noinline__ void cholesky_rows(SM& sm, int j_begin) {
   constexpr int N6 = Cfg<H>::N6;
   const int i = threadIdx.x;
   const bool row_ok = i < N6;
@@ -356,7 +248,7 @@ __device__ RG_HEAVY_INLINE void cholesky_rows(SM& sm, int j_begin) {
 #pragma unroll
       for (int c = 0; c < 4; ++c) acc[c] = (c < w && j0 + c <= i) ? row_i[j0 + c] : 0.0;
       const int ng = j0 >> 1;                          // pairs of columns already factored (j0 % 4 == 0)
-      if (w == 4 && RG_CHOL_LDS128) {
+      if (w == 4) {
         // 128-bit broadcast loads of the panel rows.  T(r) = r(r+1)/2 is even for r = 0, 3 (mod 4) and odd for
         // r = 1, 2 (mod 4): rows j0 and j0+3 are 16-byte aligned at even k, rows j0+1 and j0+2 at odd k.  The
         // latter two are read as the pairs (2g+1, 2g+2) and consumed with a one-element lag.  All loads of step
@@ -366,11 +258,8 @@ __device__ RG_HEAVY_INLINE void cholesky_rows(SM& sm, int j_begin) {
         double2 b0 = ld2v(p0), b3 = ld2v(p3);
         double b1x = p1[0], b2x = p2[0];
         double2 q1 = ld2v(p1 + 1), q2 = ld2v(p2 + 1);
-#if RG_CHOL_UNROLL == 4
+        // unrolled 4 times: a trip moves five pointers and rotates the lagged operands, ~10 of 38 instructions at 2
 #pragma unroll 4
-#else
-#pragma unroll 2
-#endif
         for (int g = 0; g < ng; ++g) {
           const double2 an = ld2(r2 + 2 * g + 2);
           const double2 c0 = ld2v(p0 + 2 * g + 2), c3 = ld2v(p3 + 2 * g + 2);
@@ -472,89 +361,6 @@ __device__ RG_HEAVY_INLINE void cholesky_rows(SM& sm, int j_begin) {
   if (i == 0 && !(sm.rdiag[N6 - 2] * sm.rdiag[N6 - 1] < 1e300)) sm.flag = 1;
 }
 
-// Generic W-wide panel variant of cholesky_rows (compiler-scheduled update loop, right-looking factorisation of the
-// W x W diagonal block in registers).  RG_CHOL_W = 6 matches the 6 x 6 time blocks of Psi: 10 panels instead of 15
-// at h = 10, and a partial refactorisation can restart at ANY time block (6 t_begin is always a panel boundary).
-template <int H, int W, class SM>
-__device__ RG_HEAVY_INLINE void cholesky_rows_w(SM& sm, int j_begin) {
-  constexpr int N6 = Cfg<H>::N6;
-  static_assert(N6 % W == 0 && W * W <= 36, "panel width must divide 6h and fit the side buffer");
-  const int i = threadIdx.x;
-  const bool row_ok = i < N6;
-  double* row_i = sm.psi + prow(row_ok ? i : 0);
-  if (i == 0) sm.flag = 0;   // published by the first barrier below
-#pragma unroll 1
-  for (int j0 = j_begin; j0 < N6; j0 += W) {
-    double acc[W];
-    const bool in_play = row_ok && i >= j0;
-    if (in_play) {
-      const double* p[W];
-#pragma unroll
-      for (int c = 0; c < W; ++c) {
-        p[c] = sm.psi + prow(j0 + c);
-        acc[c] = (j0 + c <= i) ? row_i[j0 + c] : 0.0;
-      }
-#pragma unroll 2
-      for (int k = 0; k < j0; k += 2) {
-        const double2 a = ld2(row_i + k);
-#pragma unroll
-        for (int c = 0; c < W; ++c) {
-          const double2 b = ld2(p[c] + k);
-          acc[c] = fma(-a.x, b.x, acc[c]);
-          acc[c] = fma(-a.y, b.y, acc[c]);
-        }
-      }
-      if (i < j0 + W) {
-#pragma unroll
-        for (int c = 0; c < W; ++c) if (j0 + c <= i) sm.blk44[W * (i - j0) + c] = acc[c];
-      }
-    }
-    __syncthreads();
-    if (in_play) {
-      double a[W][W];
-#pragma unroll
-      for (int r = 0; r < W; ++r)
-#pragma unroll
-        for (int c = 0; c <= r; ++c) a[r][c] = sm.blk44[W * r + c];
-      double rd[W];
-      bool bad = false;
-      const bool panel_row = i < j0 + W;
-#pragma unroll
-      for (int c = 0; c < W; ++c) {
-        double d = a[c][c];
-        if (!(d > 0.0)) { bad = true; d = 1e-300; }
-        rd[c] = rsqrt(d);
-#pragma unroll
-        for (int r = c + 1; r < W; ++r) a[r][c] *= rd[c];
-#pragma unroll
-        for (int r = c + 1; r < W; ++r)
-#pragma unroll
-          for (int cc = c + 1; cc <= r; ++cc) a[r][cc] = fma(-a[r][c], a[cc][c], a[r][cc]);
-        // the row below the block: x L_JJ^T = acc, eagerly (column c of the block is final here)
-        acc[c] *= rd[c];
-#pragma unroll
-        for (int r = c + 1; r < W; ++r) acc[r] = fma(-acc[c], a[r][c], acc[r]);
-      }
-      if (panel_row) {
-        const int r = i - j0;
-#pragma unroll
-        for (int rr = 0; rr < W; ++rr) {
-          if (rr == r) {
-#pragma unroll
-            for (int c = 0; c < rr; ++c) row_i[j0 + c] = a[rr][c];
-            sm.rdiag[i] = rd[rr];
-          }
-        }
-        if (bad && r == 0) sm.flag = 1;
-      } else {
-#pragma unroll
-        for (int c = 0; c < W; ++c) row_i[j0 + c] = acc[c];
-      }
-    }
-    __syncthreads();
-  }
-}
-
 // ---- Psi x = b with the factor, b/x in sm.avec; executed by one warp ---------------------------
 // Each lane owns RPL CONSECUTIVE rows (30 lanes x 1, 2 or 4 rows).  One step eliminates the RPL pivots
 // of one lane: a lane-local RPL x RPL triangular solve with the own diagonal reciprocals held in
@@ -568,7 +374,7 @@ __device__ RG_HEAVY_INLINE void cholesky_rows_w(SM& sm, int j_begin) {
 // T(i) mod 16 is a permutation over the even and over the odd rows of 16 consecutive lanes, so the
 // per-column loads stay bank-conflict free with this ownership too.
 template <int H, class SM>
-__device__ RG_HEAVY_INLINE void tri_solve_warp0(SM& sm) {
+__device__ __noinline__ void tri_solve_warp0(SM& sm) {
   constexpr int N6 = Cfg<H>::N6;
   constexpr int RPL = Cfg<H>::RPL;
   constexpr int NL = N6 / RPL;
@@ -766,7 +572,7 @@ __device__ __forceinline__ double pick_sym3(const double* m, int r, int c) {
 }
 
 template <int H, class SM>
-__device__ RG_HEAVY_INLINE void riccati_factor(SM& sm) {
+__device__ __noinline__ void riccati_factor(SM& sm) {
   const int lane = threadIdx.x & 31;   // one warp runs this routine (sm.solver_warp)
   // Lane roles (indices of lanes without the role are clamped to 0: every lane computes, only role lanes store --
   // predicated stores instead of divergent branches around each step)
@@ -953,7 +759,7 @@ __device__ RG_HEAVY_INLINE void riccati_factor(SM& sm) {
 // The 12-vectors p and x live in lanes 0..11 (pi part in lanes 0..5, sigma part in lanes 6..11), the 6-vectors in
 // lanes 0..5; everything moves by warp shuffles: no barrier and no shared-memory round trip on the chain.
 template <int H, class SM>
-__device__ RG_HEAVY_INLINE void riccati_solve(SM& sm) {
+__device__ __noinline__ void riccati_solve(SM& sm) {
   const int lane = threadIdx.x & 31;   // one warp runs this routine (sm.solver_warp)
   const int k12 = lane < 12 ? lane : 0, c6 = lane < 6 ? lane : 0;
   // The 6- and 12-vectors a stage hands from one product to the next go through shared memory (one predicated store,
@@ -1183,8 +989,7 @@ __device__ __forceinline__ void factor_psi(Smem<H>& sm, const RgMpcDev* __restri
     psi_build_rows<H>(sm, ws, t_begin);
     __syncthreads();
     RG_TOC(10);
-    if constexpr (Cfg<H>::CHOL_W == 4) cholesky_rows<H>(sm, 6 * t_begin);
-    else cholesky_rows_w<H, Cfg<H>::CHOL_W>(sm, 6 * t_begin);
+    cholesky_rows<H>(sm, 6 * t_begin);
   }
   RG_TOC(11);
 }
@@ -1584,9 +1389,6 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
     asm volatile("mov.u32 %0, %%warpid;" : "=r"(slot));
     const unsigned group = slot / C::NW;
     sm.solver_warp = C::NW >= 4 ? (int)(group % C::NW) : (C::NW == 2 ? (int)((group >> 1) & 1u) : 0);
-#ifdef RG_SOLVER_WARP0
-    sm.solver_warp = 0;
-#endif
   }
 
   RG_TOC(40);
@@ -1840,7 +1642,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 #pragma unroll
     for (int r = 0; r < 10; ++r) {
       if (!active_blk) s[r] = 1.0;
-      lam[r] = active_blk ? RG_IPM_LAM0 * qscale / s[r] : 1.0;   // inactive threads carry harmless 1/1 pairs
+      lam[r] = active_blk ? kIpmLam0 * qscale / s[r] : 1.0;   // inactive threads carry harmless 1/1 pairs
     }
   }
   const double m_total = PLAN ? 10.0 * plan_blocks : 10.0 * H * n_stance;
@@ -1868,7 +1670,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
   const double cold_max_viol = (double)ws->cold_start_max_violations;
   // Weakly active rows (multiplier ~ 0 at the optimum: strict complementarity fails) flip for ever between "dropped
   // because its multiplier is -1e-10" and "violated by 1e-9 without it".  A row that was dropped and came back is
-  // sticky: it then only leaves for a multiplier that is wrong by more than RG_STICKY_TOL (1e-9) of the gradient scale.
+  // sticky: it then only leaves for a multiplier that is wrong by more than kStickyTol (1e-9) of the gradient scale.
   unsigned dropped_rows = 0u, sticky_rows = 0u;
 #pragma unroll 1
   for (int attempt = (cold_rounds > 0 && !skip_cold) ? -1 : 0; attempt < (LEAN ? 0 : 3) && !done; ++attempt) {
@@ -1887,7 +1689,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
         for (int d = 0; d < 3; ++d) rd0 = fmax(rd0, fabs(pu0[d] + q[d]));
       }
       block_reduce<C::NW, 2>(dsum, rd0, dmn, sm.red);
-      const double mu0 = RG_IPM_LAM0 * fmax(qscale, RG_IPM_RD_SCALE * rd0);
+      const double mu0 = kIpmLam0 * fmax(qscale, rd0);
 #pragma unroll
       for (int r = 0; r < 10; ++r) lam[r] = active_blk ? mu0 / s[r] : 1.0;
     }
@@ -1916,7 +1718,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       const double res = fmax(rdmax, mu_c) / qscale;
       RG_TRACE(4 * trace_n + 0, res); RG_TRACE(4 * trace_n + 1, mu_c); RG_TRACE(4 * trace_n + 2, (double)iters); RG_TRACE(4 * trace_n + 3, tol);
       ++trace_n;
-      // slow lane: the best residual has not halved for RG_IPM_SLOW_ITERS iterations although the iterate is
+      // slow lane: the best residual has not halved for kIpmSlowIters iterations although the iterate is
       // already close (mu oscillating around 1e-5 on a few pace / bound problems, 40 iterations to the cap):
       // hand over to the active-set rounds, which verify from such a point in a round or two
       slow = (res < 0.5 * best_res) ? 0 : slow + 1;
@@ -1926,7 +1728,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
         for (int d = 0; d < 3; ++d) u_best[d] = u[d];
       }
       if (res < tol) { converged = true; break; }
-      if (slow >= RG_IPM_SLOW_ITERS && res < 1e-3 && max_polish > 0) { handed_over = true; slow = 0; break; }
+      if (slow >= kIpmSlowIters && res < 1e-3 && max_polish > 0) { handed_over = true; slow = 0; break; }
       stall = (res > 0.9 * prev_res && res < 1e-7) ? stall + 1 : 0;   // only near the numerical floor
       prev_res = res;
       // dead: budget spent, stalled at the numerical floor, NaN, or diverging (deep iterates lose the
@@ -2015,7 +1817,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       // fraction to the boundary: 0.99 throughout.  (0.999 once the residuals are small saved nothing measurable
       // and made two bound-gait problems in 1.5 M oscillate at mu ~ 1e-4; steps closer to 1 collapse the slacks
       // while the dual residual is still finite and de-centre the iterate.)
-      const double tau = res < 1e-3 ? RG_IPM_TAU_LATE : 0.99;
+      const double tau = 0.99;
       const double step = tmax > tau ? tau / tmax : 1.0;
       if (active_blk) {
 #pragma unroll
@@ -2050,111 +1852,45 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
       // warm start: the verified active set of this block from the previous solve of the same env
       // (consecutive control steps see almost the same problem); wrong guesses are repaired by the rounds
       act = active_blk ? warm_act : 0u;
-    } else if (RG_COLD_GUESS_LAST && active_blk && t_blk >= H - (n_step == 4 ? RG_COLD_GUESS_LAST_4 : RG_COLD_GUESS_LAST)) {
+    } else if (active_blk && t_blk >= H - (n_step == 4 ? kColdGuessLast4 : kColdGuessLast)) {
       // a force in the last step(s) of the horizon barely moves any tracked state, so the regulariser
       // drives it to zero: fz >= fz_min is active there in practically every problem (bit 9)
       act = 1u << 9;
     }
     bool polished = false, fact_valid = false;   // the factor in shared memory is the interior point's, if any
     unsigned act_fact = 0;
-    double prev_nchg = 1e300;
+    double prev_nchg = 1e300;   // unused, but deleting it moves ptxas's register assignment in the h = 20 lean model kernel
     double up[3] = {0.0, 0.0, 0.0};
     // 3, 6, 12 rounds: later attempts start from a sharper guess; a dead interior point gets the full budget
-    const int round_budget = cold ? cold_rounds + RG_COLD_EXTEND_ROUNDS : (ipm_dead || handed_over) ? (max_polish << 2) : (max_polish << attempt);
+    const int round_budget = cold ? cold_rounds : (ipm_dead || handed_over) ? (max_polish << 2) : (max_polish << attempt);
 #pragma unroll 1
     for (int round = 0; round < round_budget; ++round) {
       ++polish_rounds;
       // --- per block: orthonormal basis of the active normals (<= 3), null-space basis Z, u0.
-      // Two storage schemes, chosen per horizon by measurement (profiles/r02_basis_storage.md): named registers
-      // (Cfg::BASIS_IN_REGS: no local-memory frame, DRAM traffic = the algorithmic bytes) or small local arrays indexed
-      // by the run-time row count (fewer live registers across the heavy phases, but a 480-byte frame per thread).
+      // The basis sits in named registers (no local-memory frame: DRAM traffic = the algorithmic bytes) and only while
+      // it is used here: the multiplier test rebuilds it.  Against small local arrays indexed by the run-time row count:
+      // h = 5 27.2 -> 28.8 M, h = 20 5.72 -> 5.85 M solves/s at 65536 envs (profiles/r02_basis_storage.md).
       int na;
       double u0[3], mproj[6];
-#if !RG_REBUILD_BASIS
-      BlockBasis B;                                                        // register scheme
-#endif
-      double e[3][3], rr[3][3];                                            // array scheme: a_i = sum_k rr[k][i] e_k
-      int rows[3] = {-1, -1, -1};
-      if constexpr (C::BASIS_IN_REGS) {
-        {
-#if RG_REBUILD_BASIS
-          BlockBasis B;
-#endif
-          build_basis(act, active_blk, mu, hv_up, lo_b, B);
-          na = B.na;
-          // particular solution u0 = sum_k c_k e_k with a_i . u0 = b_i  (forward substitution with rr^T; unused slots have
-          // zero basis vectors and unit diagonal, so they contribute nothing)
-          const double cp0 = na > 0 ? B.bt0 * B.ir00 : 0.0;
-          const double cp1 = na > 1 ? (B.bt1 - B.r01 * cp0) * B.ir11 : 0.0;
-          const double cp2 = na > 2 ? (B.bt2 - B.r02 * cp0 - B.r12 * cp1) * B.ir22 : 0.0;
+      {
+        BlockBasis B;
+        build_basis(act, active_blk, mu, hv_up, lo_b, B);
+        na = B.na;
+        // particular solution u0 = sum_k c_k e_k with a_i . u0 = b_i  (forward substitution with rr^T; unused slots have
+        // zero basis vectors and unit diagonal, so they contribute nothing)
+        const double cp0 = na > 0 ? B.bt0 * B.ir00 : 0.0;
+        const double cp1 = na > 1 ? (B.bt1 - B.r01 * cp0) * B.ir11 : 0.0;
+        const double cp2 = na > 2 ? (B.bt2 - B.r02 * cp0 - B.r12 * cp1) * B.ir22 : 0.0;
 #pragma unroll
-          for (int d = 0; d < 3; ++d) u0[d] = cp0 * B.e0[d] + cp1 * B.e1[d] + cp2 * B.e2[d];
-          // projector onto the free directions  M = I - sum_k e_k e_k^T, packed (xx,yy,zz,xz,yz,xy),
-          // scaled by 1 / (2 alpha): this is the "E^-1" of the equality-constrained Newton system
-          mproj[0] = 1.0 - (B.e0[0] * B.e0[0] + B.e1[0] * B.e1[0] + B.e2[0] * B.e2[0]);
-          mproj[1] = 1.0 - (B.e0[1] * B.e0[1] + B.e1[1] * B.e1[1] + B.e2[1] * B.e2[1]);
-          mproj[2] = 1.0 - (B.e0[2] * B.e0[2] + B.e1[2] * B.e1[2] + B.e2[2] * B.e2[2]);
-          mproj[3] = -(B.e0[0] * B.e0[2] + B.e1[0] * B.e1[2] + B.e2[0] * B.e2[2]);
-          mproj[4] = -(B.e0[1] * B.e0[2] + B.e1[1] * B.e1[2] + B.e2[1] * B.e2[2]);
-          mproj[5] = -(B.e0[0] * B.e0[1] + B.e1[0] * B.e1[1] + B.e2[0] * B.e2[1]);
-        }
-
-      } else {
-#pragma unroll
-        for (int i = 0; i < 3; ++i)
-#pragma unroll
-          for (int k = 0; k < 3; ++k) { e[i][k] = 0.0; rr[i][k] = 0.0; }
-        double bt[3] = {0, 0, 0};
-        na = 0;
-        if (active_blk) {
-#pragma unroll 1
-          for (int r = 0; r < 10; ++r) {
-            if (!((act >> r) & 1u) || na >= 3) continue;
-            const int rw = r < 5 ? r : r - 5;
-            double a[3] = {rw == 0 ? -1.0 : rw == 1 ? 1.0 : 0.0, rw == 2 ? -1.0 : rw == 3 ? 1.0 : 0.0,
-                           rw < 4 ? mu[rw] : 1.0};
-            const double target = r < 5 ? hv_up[rw] : lo_b[rw];
-            double coef[3] = {0, 0, 0};
-            for (int k = 0; k < na; ++k) {
-              coef[k] = a[0] * e[k][0] + a[1] * e[k][1] + a[2] * e[k][2];
-              a[0] -= coef[k] * e[k][0]; a[1] -= coef[k] * e[k][1]; a[2] -= coef[k] * e[k][2];
-            }
-            const double nrm = sqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]);
-            if (nrm < 1e-9) { act &= ~(1u << r); continue; }   // dependent normal: drop
-            const double inrm = 1.0 / nrm;
-            e[na][0] = a[0] * inrm; e[na][1] = a[1] * inrm; e[na][2] = a[2] * inrm;
-            for (int k = 0; k < na; ++k) rr[k][na] = coef[k];
-            rr[na][na] = nrm;
-            bt[na] = target;
-            rows[na] = r;
-            ++na;
-          }
-          // rows beyond the third independent one cannot be held: drop them from the guess
-#pragma unroll 1
-          for (int r = 0; r < 10; ++r) {
-            if (((act >> r) & 1u) && r != rows[0] && r != rows[1] && r != rows[2]) act &= ~(1u << r);
-          }
-        }
-        // particular solution u0 = sum_k c_k e_k with a_i . u0 = b_i
-        double cpar[3] = {0, 0, 0};
-#pragma unroll 1
-        for (int i = 0; i < na; ++i) {
-          double v = bt[i];
-          for (int k = 0; k < i; ++k) v -= rr[k][i] * cpar[k];
-          cpar[i] = v / rr[i][i];
-        }
-        u0[0] = u0[1] = u0[2] = 0.0;
-#pragma unroll 1
-        for (int k = 0; k < na; ++k) { u0[0] += cpar[k] * e[k][0]; u0[1] += cpar[k] * e[k][1]; u0[2] += cpar[k] * e[k][2]; }
+        for (int d = 0; d < 3; ++d) u0[d] = cp0 * B.e0[d] + cp1 * B.e1[d] + cp2 * B.e2[d];
         // projector onto the free directions  M = I - sum_k e_k e_k^T, packed (xx,yy,zz,xz,yz,xy),
         // scaled by 1 / (2 alpha): this is the "E^-1" of the equality-constrained Newton system
-        mproj[0] = mproj[1] = mproj[2] = 1.0; mproj[3] = mproj[4] = mproj[5] = 0.0;
-#pragma unroll 1
-        for (int k = 0; k < na; ++k) {
-          mproj[0] -= e[k][0] * e[k][0]; mproj[1] -= e[k][1] * e[k][1]; mproj[2] -= e[k][2] * e[k][2];
-          mproj[3] -= e[k][0] * e[k][2]; mproj[4] -= e[k][1] * e[k][2]; mproj[5] -= e[k][0] * e[k][1];
-        }
-
+        mproj[0] = 1.0 - (B.e0[0] * B.e0[0] + B.e1[0] * B.e1[0] + B.e2[0] * B.e2[0]);
+        mproj[1] = 1.0 - (B.e0[1] * B.e0[1] + B.e1[1] * B.e1[1] + B.e2[1] * B.e2[1]);
+        mproj[2] = 1.0 - (B.e0[2] * B.e0[2] + B.e1[2] * B.e1[2] + B.e2[2] * B.e2[2]);
+        mproj[3] = -(B.e0[0] * B.e0[2] + B.e1[0] * B.e1[2] + B.e2[0] * B.e2[2]);
+        mproj[4] = -(B.e0[1] * B.e0[2] + B.e1[1] * B.e1[2] + B.e2[1] * B.e2[2]);
+        mproj[5] = -(B.e0[0] * B.e0[1] + B.e1[0] * B.e1[1] + B.e2[0] * B.e2[1]);
       }
       if (na == 3 || !active_blk) { mproj[0] = mproj[1] = mproj[2] = mproj[3] = mproj[4] = mproj[5] = 0.0; }
       const double inv2a = 1.0 / two_alpha;
@@ -2170,7 +1906,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
         if (active_blk && act != act_fact) tmin = (double)t_blk;
         if (!fact_valid) tmin = 0.0;
         block_reduce<C::NW, 4>(dsum, dmx, tmin, sm.red);
-        t_fac = tmin < (double)H ? (C::RICCATI ? 0 : (C::CHOL_W == 4 ? (((int)tmin) & ~1) : (int)tmin)) : -1;
+        t_fac = tmin < (double)H ? (C::RICCATI ? 0 : (((int)tmin) & ~1)) : -1;   // cholesky_rows restarts on a 4-column panel
       }
       RG_TIC();
       if (t_fac >= 0) factor_psi<H>(sm, ws, blk, mproj, t_fac);
@@ -2238,66 +1974,37 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 #pragma unroll
           for (int r = 0; r < 10; ++r) {
             const double slack = r < 5 ? hv_up[r] - c5[r] : c5[r - 5] - lo_b[r - 5];
-            if (!((act >> r) & 1u) && slack < worst) {
-              if (RG_ADD_ONE_PER_BLOCK) { worst = slack; rworst = r; }
-              else act_new |= 1u << r;
-            }
+            if (!((act >> r) & 1u) && slack < worst) { worst = slack; rworst = r; }
           }
           if (rworst >= 0) {
             act_new |= 1u << rworst;
             if ((dropped_rows >> rworst) & 1u) sticky_rows |= 1u << rworst;
           }
           int rmin = -1;
-          if constexpr (C::BASIS_IN_REGS) {
-#if RG_REBUILD_BASIS
-            // the basis is rebuilt from the bit mask (a few dozen instructions) instead of being kept live across the
-            // factorisation and the sweeps: 21 doubles fewer in flight over the heavy calls
-            BlockBasis B;
-            { unsigned act_again = act; build_basis(act_again, active_blk, mu, hv_up, lo_b, B); }
-#endif
-            // multipliers: sum_i y_i a_i = -gr on span(e)  ->  back substitution with the upper triangular rr
-            const int row0 = B.row0, row1 = B.row1, row2 = B.row2;
-            const double g0 = -(gr[0] * B.e0[0] + gr[1] * B.e0[1] + gr[2] * B.e0[2]);
-            const double g1 = -(gr[0] * B.e1[0] + gr[1] * B.e1[1] + gr[2] * B.e1[2]);
-            const double g2 = -(gr[0] * B.e2[0] + gr[1] * B.e2[1] + gr[2] * B.e2[2]);
-            const double y2 = g2 * B.ir22;
-            const double y1 = (g1 - B.r12 * y2) * B.ir11;
-            const double y0 = (g0 - B.r01 * y1 - B.r02 * y2) * B.ir00;
-            double ymin = 1e300;
+          // the basis is rebuilt from the bit mask (a few dozen instructions) instead of being kept live across the
+          // factorisation and the sweeps: 21 doubles fewer in flight over the heavy calls
+          BlockBasis B;
+          { unsigned act_again = act; build_basis(act_again, active_blk, mu, hv_up, lo_b, B); }
+          // multipliers: sum_i y_i a_i = -gr on span(e)  ->  back substitution with the upper triangular rr
+          const int row0 = B.row0, row1 = B.row1, row2 = B.row2;
+          const double g0 = -(gr[0] * B.e0[0] + gr[1] * B.e0[1] + gr[2] * B.e0[2]);
+          const double g1 = -(gr[0] * B.e1[0] + gr[1] * B.e1[1] + gr[2] * B.e1[2]);
+          const double g2 = -(gr[0] * B.e2[0] + gr[1] * B.e2[1] + gr[2] * B.e2[2]);
+          const double y2 = g2 * B.ir22;
+          const double y1 = (g1 - B.r12 * y2) * B.ir11;
+          const double y0 = (g0 - B.r01 * y1 - B.r02 * y2) * B.ir00;
+          double ymin = 1e300;
 #pragma unroll
-            for (int i = 0; i < 3; ++i) {
-              const int row = i == 0 ? row0 : (i == 1 ? row1 : row2);
-              const double yi = i == 0 ? y0 : (i == 1 ? y1 : y2);
-              if (i < na) {
-                // upper-bound rows need y >= 0, lower-bound rows y <= 0
-                const double ysgn = row < 5 ? yi : -yi;
-                const double drop_tol = ((sticky_rows >> row) & 1u) ? RG_STICKY_TOL : 1e-10;
-                if (ysgn < -drop_tol * qscale) { act_new &= ~(1u << row); dropped_rows |= 1u << row; }
-                if (ysgn < ymin) { ymin = ysgn; rmin = row; }
-              }
-            }
-
-          } else {
-            // multipliers: sum_i y_i a_i = -gr on span(e)
-            double y[3] = {0, 0, 0};
-#pragma unroll 1
-            for (int i = na - 1; i >= 0; --i) {
-              double v = -(gr[0] * e[i][0] + gr[1] * e[i][1] + gr[2] * e[i][2]);
-              for (int k = i + 1; k < na; ++k) v -= rr[i][k] * y[k];
-              y[i] = v / rr[i][i];
-            }
-            double ymin = 1e300;
-            int imin = -1;
-#pragma unroll 1
-            for (int i = 0; i < na; ++i) {
+          for (int i = 0; i < 3; ++i) {
+            const int row = i == 0 ? row0 : (i == 1 ? row1 : row2);
+            const double yi = i == 0 ? y0 : (i == 1 ? y1 : y2);
+            if (i < na) {
               // upper-bound rows need y >= 0, lower-bound rows y <= 0
-              const double ysgn = rows[i] < 5 ? y[i] : -y[i];
-              const double drop_tol = ((sticky_rows >> rows[i]) & 1u) ? RG_STICKY_TOL : 1e-10;
-              if (ysgn < -drop_tol * qscale) { act_new &= ~(1u << rows[i]); dropped_rows |= 1u << rows[i]; }
-              if (ysgn < ymin) { ymin = ysgn; imin = i; }
+              const double ysgn = row < 5 ? yi : -yi;
+              const double drop_tol = ((sticky_rows >> row) & 1u) ? kStickyTol : 1e-10;
+              if (ysgn < -drop_tol * qscale) { act_new &= ~(1u << row); dropped_rows |= 1u << row; }
+              if (ysgn < ymin) { ymin = ysgn; rmin = row; }
             }
-
-            rmin = imin >= 0 ? rows[imin] : -1;
           }
           // a block that already holds three rows is a vertex: a violated fourth row can only come in if one
           // leaves, and the basis builder keeps the first three in bit order -- without this swap the newcomer
@@ -2319,7 +2026,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
         RG_TOC(24);
         const bool trusted = pgm <= 1e-9 * qscale || pass == 2;
         if (nchg > 0.0) { if (trusted) break; else continue; }
-        if (pgm <= (pass == 0 ? RG_SKIP_REFINE_TOL : pass == 1 ? 1e-10 : 1e-7) * qscale) { accept = true; break; }
+        if (pgm <= (pass == 0 ? kSkipRefineTol : pass == 1 ? 1e-10 : 1e-7) * qscale) { accept = true; break; }
       }
 #if defined(RG_DEBUG_TRACE) && !defined(RG_DEBUG_TIMELINE_ONLY)
       {
@@ -2331,10 +2038,8 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
 #endif
       if (accept) { polished = true; break; }
       // the cold start hands over to the interior point when the unconstrained minimiser violates too
-      // many friction-cone rows (fz-bound rows settle in a round or two, cone rows make it cycle), or when the number of rows that move stops shrinking (the iteration is cycling)
-      // (past the nominal budget only an almost-settled iteration -- <= RG_COLD_EXTEND_NCHG rows still moving -- goes on)
-      if (cold && ((round == 0 && ncone > cold_max_viol) || (RG_COLD_NO_DECREASE_RULE && round >= 1 && nchg >= prev_nchg && nchg > 2.0) ||
-                   (round + 1 >= cold_rounds && nchg > RG_COLD_EXTEND_NCHG))) break;
+      // many friction-cone rows (fz-bound rows settle in a round or two, cone rows make it cycle)
+      if (cold && ((round == 0 && ncone > cold_max_viol) || (round + 1 >= cold_rounds && nchg > kColdLastRoundNchg))) break;
       prev_nchg = nchg;
       act = act_new;
     }
@@ -2366,7 +2071,7 @@ __device__ __forceinline__ void solve_env(Smem<H>& sm, const RgMpcDev* __restric
         if (!(thmax == thmax)) thmax = 0.0;
       }
       block_reduce<C::NW, 4>(dsum, dmx, thmax, sm.red);
-      const double theta = RG_IPM_WARM * thmax;
+      const double theta = kIpmWarm * thmax;
       if constexpr (!LEAN) {
         if (active_blk && theta > 0.0) {
 #pragma unroll
@@ -2442,10 +2147,8 @@ __device__ __forceinline__ void solve_grid(const RgMpcDev* __restrict__ ws, RgMp
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
   const int env = blockIdx.x;
-#if RG_PDL
   RG_GRID_LAUNCH_DEPENDENTS();   // see launch_kernels: the fallback grid (lean) or the step epilogue (complete kernel) may be scheduled behind us
   RG_GRID_WAIT();                // launched programmatically behind the step prologue in rg_control_step; a no-op otherwise
-#endif
   if (env >= n_env) return;
   solve_env<H, LEAN, ENV_MODEL, PLAN, FEET>(sm, ws, scratch, env, false, io, model, plan, feet);
 }
@@ -2461,10 +2164,8 @@ __device__ __forceinline__ void fallback_grid(const RgMpcDev* __restrict__ ws, R
                                               const float* __restrict__ feet = nullptr) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem<H>& sm = *reinterpret_cast<Smem<H>*>(smem_raw);
-#if RG_PDL
   RG_GRID_LAUNCH_DEPENDENTS();   // the step epilogue may be scheduled behind this grid
   RG_GRID_WAIT();                // launched programmatically: the lean grid must have completed
-#endif
   const int count = min(scratch->queue_tail, min(scratch->capacity, n_env));
   for (int q = blockIdx.x; q < count; q += gridDim.x) {
     const int env = scratch->queue[q];
@@ -2557,13 +2258,9 @@ int configure_kernel(const void* kernel, size_t smem, int min_blocks, const char
   if (e != cudaSuccess) return rg_check_cuda(e, what);
   // the default carveout leaves room for only ~5 CTAs: ask for what MIN_BLOCKS resident CTAs need and no
   // more, so that the rest of the 228 KB stays L1 (local-memory traffic and the parameter block live there)
-#ifndef RG_CARVEOUT_PCT
   const int need_kb = (int)((min_blocks * (smem + 1024) + 1023) / 1024);
   int carveout = (need_kb * 100 + 227) / 228 + 1;
   if (carveout > 100) carveout = 100;
-#else
-  const int carveout = RG_CARVEOUT_PCT;
-#endif
   e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
   if (e != cudaSuccess) return rg_check_cuda(e, what);
   if (dev < 64) mask |= 1ull << dev;
@@ -2624,20 +2321,20 @@ int launch_kernels(const RgMpcDev* ws, int n_env, const rg_mpc_io& io, int two_k
     if (rc != RG_OK) return rc;
     rc = configure_kernel((const void*)fallback_kernel, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_fallback_kernel)");
     if (rc != RG_OK) return rc;
-    rc = rg_check_cuda(launch(lean_kernel, n_env, RG_PDL && chained), "mpc_solve_kernel (lean) launch");
+    rc = rg_check_cuda(launch(lean_kernel, n_env, chained), "mpc_solve_kernel (lean) launch");
     rg_count_launch();
     if (rc != RG_OK) return rc;
     const int grid = n_env < slots ? n_env : slots;       // as many CTAs as fit at once: an empty queue costs one wave of exits
     // Programmatic dependent launch: every lean CTA signals at its start, so once the last one HAS STARTED the fallback
     // grid may take the slots the draining lean grid leaves free; its CTAs block in griddepcontrol.wait until the lean
     // grid has completed (queue visible).  The launch latency of the second kernel hides behind the first one's tail.
-    rc = rg_check_cuda(launch(fallback_kernel, grid, RG_PDL != 0), "mpc_fallback_kernel launch");
+    rc = rg_check_cuda(launch(fallback_kernel, grid, true), "mpc_fallback_kernel launch");
     rg_count_launch();
     return rc;
   }
   rc = configure_kernel((const void*)full_kernel, smem, Cfg<H>::MIN_BLOCKS, "cudaFuncSetAttribute(mpc_solve_kernel)");
   if (rc != RG_OK) return rc;
-  rc = rg_check_cuda(launch(full_kernel, n_env, RG_PDL && chained), "mpc_solve_kernel launch");
+  rc = rg_check_cuda(launch(full_kernel, n_env, chained), "mpc_solve_kernel launch");
   rg_count_launch();
   return rc;
 }
@@ -2674,8 +2371,7 @@ __global__ void __launch_bounds__(Cfg<H>::NT) chol_selftest_kernel(const double*
     for (int k = 0; k <= tid; ++k) sm.psi[prow(tid) + k] = a_dense[tid * N6 + k];
   }
   __syncthreads();
-  if constexpr (Cfg<H>::CHOL_W == 4) cholesky_rows<H>(sm, 0);
-  else cholesky_rows_w<H, Cfg<H>::CHOL_W>(sm, 0);
+  cholesky_rows<H>(sm, 0);
   if (tid < N6) sm.avec[tid] = rhs[tid];   // after the factorisation: avec / kvec are its scratch
   __syncthreads();
   if (tid < 32) tri_solve_warp0<H>(sm);

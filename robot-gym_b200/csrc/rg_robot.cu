@@ -1048,9 +1048,7 @@ extern "C" int rg_hybrid_motor_torque_ex(const void* ws, int n_env, const float*
 // Batches up to this many envs run the per-(env, leg) prologue (a quarter of the dependent chain per thread), larger ones
 // the per-env one.  Measured on the B200 (tools/gpu/lat_step.py, warm-started control step): per leg -8 us at 1 ... 1024
 // envs (88 -> 80 us with the Python call), -9 us at 4096, -6 us at 16384, +13 us at 65536.
-#ifndef RG_PROLOGUE_LEG_MAX_ENVS
-#define RG_PROLOGUE_LEG_MAX_ENVS 32768
-#endif
+constexpr int kPrologueLegMaxEnvs = 32768;
 
 extern "C" int rg_control_step(const void* mpc_ws, const void* robot_ws, int n_env, const rg_controller_state* s, void* stream) {
   return rg_control_step_model(mpc_ws, robot_ws, n_env, s, nullptr, stream);
@@ -1127,15 +1125,15 @@ extern "C" int rg_control_step_footholds(const void* mpc_ws, const void* robot_w
     rc = rg_mpc_workspace_info(mpc_ws, &info);
     if (rc != RG_OK) return rc;
     const rg_gait_env_params gp = g ? *g : rg_gait_env_params{nullptr, nullptr, nullptr, nullptr};
-    if (feet && n_env <= RG_PROLOGUE_LEG_MAX_ENVS)
+    if (feet && n_env <= kPrologueLegMaxEnvs)
       step_prologue_feet_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, feet, info.horizon, info.dt);
     else if (feet)
       step_prologue_env_feet_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, feet, info.horizon, info.dt);
-    else if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS)
+    else if (n_env <= kPrologueLegMaxEnvs)
       step_prologue_plan_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, info.horizon, info.dt);
     else
       step_prologue_env_plan_kernel<<<grid_for(n_env, 128), 128, 0, st>>>(R, n_env, *s, gp, plan, info.horizon, info.dt);
-  } else if (n_env <= RG_PROLOGUE_LEG_MAX_ENVS) {
+  } else if (n_env <= kPrologueLegMaxEnvs) {
     if (g) step_prologue_gait_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s, *g);
     else step_prologue_kernel<<<grid_for(4 * n_env, 128), 128, 0, st>>>(R, n_env, *s);
   } else {

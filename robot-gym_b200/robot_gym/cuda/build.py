@@ -33,7 +33,7 @@ def _extra_flags():
     # RG_DEBUG_TRACE=1: per-phase cycle counters of one env (intrusive); =2: only the per-CTA start / end stamps
     mode = os.environ.get("RG_DEBUG_TRACE")
     flags = ("-DRG_DEBUG_TRACE",) if mode == "1" else (("-DRG_DEBUG_TRACE", "-DRG_DEBUG_TIMELINE_ONLY") if mode == "2" else ())
-    if os.environ.get("RG_EXTRA_NVCC_FLAGS"):          # tuning experiments, e.g. -DRG_MIN_BLOCKS_H10=7
+    if os.environ.get("RG_EXTRA_NVCC_FLAGS"):          # experiments and checks, e.g. -DRG_DEBUG_POISON_SMEM=0xa5
         flags += tuple(os.environ["RG_EXTRA_NVCC_FLAGS"].split())
     return flags
 

@@ -414,7 +414,7 @@ def test_estimator_windows_bit_exact_standalone_and_fused(rg_lib, cuda_device, w
     oracle MovingWindowFilter (same IEEE operations in the same order, including the drop-oldest branch once the
     deque is full), the world-frame average is the float32 of the oracle's, the body frame within 5e-7 relative,
     count and head follow the deque.  Then the fused rg_control_step over the same velocities, at a batch on each side
-    of RG_PROLOGUE_LEG_MAX_ENVS (32768: per-(env, leg) and per-env prologue kernels), gives bitwise the same sums."""
+    of kPrologueLegMaxEnvs (32768: per-(env, leg) and per-env prologue kernels), gives bitwise the same sums."""
     dev = cuda_device
     n, W = 64, window
     steps = 3 * W + 5
